@@ -2,6 +2,7 @@
 """Benchmark of the pre + post + track hot path (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--schedule 0..6] [--no-graph] [--no-cpu]
+                    [--dump-outputs DIR]
 
 Workload at every N: each GPU serves 32 streams of 1080p BGR frames with a synthetic decoded
 YOLOv8 head [32, 84, 8400] (config 3 of BASELINE.json, the one the metric is quoted on); with
@@ -12,11 +13,13 @@ the caller's stream, decode -> NMS -> tracker on the library's second stream, fo
 call).  The detector forward is outside the measured path (north_star): the head tensors stand in
 for its output.
 
-`value`   : frames/s with frames and heads already resident in HBM (CUDA events around the K steps,
-            max over ranks).  The tick is replayed from a CUDA graph per input set; every 10th step is
-            launched eagerly with an event pair around the letterbox launch (the live kernel timing of
-            `roofline`).  Four rotating input sets keep every step's reads out of the 126 MB L2.
-`roofline`: the letterbox kernel's algorithmic bytes / that event-timed duration vs the measured HBM peak.
+`value`   : frames/s with frames and heads already resident in HBM (CUDA events around exactly K timed
+            steps, max over ranks).  The tick is replayed from a CUDA graph per input set.  Four rotating
+            input sets keep every step's reads out of the 126 MB L2.
+`--dump-outputs DIR`: after the K timed steps, rank 0 writes what the last of them handed its caller
+            (letterbox tensor as a fixed seeded sample, detection and track tables) as DIR/<name>.npy in
+            float32 / float64.  Inputs depend only on the arguments, so two builds compare output for output.
+`roofline`: the letterbox kernel's algorithmic bytes / its event-timed duration vs the measured HBM peak.
 `e2e`     : the same tick through the public API (HotPathEngine.submit / collect, two ticks in flight)
             with HOST buffers: pinned frames and heads are copied to the device and the result tables
             are read back inside the timed region.
@@ -227,9 +230,32 @@ def run_reference(args) -> None:
 # --------------------------------------------------------------------------------------------
 # GPU arm
 # --------------------------------------------------------------------------------------------
-WINDOWS = 15          # the K-step timed window is repeated this many times; the median window is the headline
+WINDOWS = 15          # K-step windows of the N > 1 strong-scaling variant; its median window is reported
 KERNEL_SAMPLES = 24   # eager ticks with per-kernel CUDA-event pairs (b200va_set_profiling), whatever --steps is
 HEAD_BYTES_PER_FRAME = C * A * 4
+DUMP_NET_SAMPLES = 1 << 21  # letterbox elements --dump-outputs writes (of 32 x 3 x 640 x 640)
+
+
+def dump_outputs(out_dir: str, net, dets: dict, tracks: dict) -> None:
+    """The arrays one tick hands its caller, as float32 / float64 .npy files: the letterbox tensor as a fixed
+    seeded sample of its elements (with their flat indices), every field of the detection and track tables.
+    Table rows past a stream's `count` hold nothing a caller may read and are written as 0."""
+    import torch
+
+    os.makedirs(out_dir, exist_ok=True)
+    flat = net.reshape(-1)
+    idx = np.sort(np.random.default_rng(0).choice(flat.numel(), DUMP_NET_SAMPLES, replace=False))
+    arrays = {"letterbox_sample": flat[torch.from_numpy(idx).to(flat.device)].cpu().numpy(),
+              "letterbox_sample_index": idx.astype(np.float64)}
+    for prefix, table in (("dets", dets), ("tracks", tracks)):
+        host = {k: v.cpu().numpy() for k, v in table.items() if not k.startswith("_")}
+        for name, v in host.items():
+            v = v.astype(np.float32 if v.dtype == np.float32 else np.float64)
+            if v.ndim > 1:  # [streams, rows(, width)]
+                v[np.arange(v.shape[1])[None, :] >= host["count"][:, None]] = 0
+            arrays[f"{prefix}_{name}"] = v
+    for name, v in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), v)
 
 
 def _capture(torch, h, plans):
@@ -403,7 +429,8 @@ def run_gpu(args) -> None:
     def windows(fn, n_windows, frames_per_step=STREAMS):
         """`n_windows` timed windows of EXACTLY K steps each, every one bracketed by barrier + synchronize on both
         sides and timed with CUDA events on the launching stream.  Per window the job time is the max over ranks;
-        the reported time is the median window.  Returns (median ms, stats)."""
+        returns (median window ms, stats).  The headline calls it with one window, so its timed region is exactly K
+        steps; the informational variants after it take the median of several windows."""
         for k in range(warm):
             fn(k)
         per = []
@@ -431,9 +458,11 @@ def run_gpu(args) -> None:
     clocks = ClockSampler(local, period_s=0.010)
     launches0 = h.launch_count
     clocks.start()
-    ms, win_stats = windows(run_step, WINDOWS)
+    ms, win_stats = windows(run_step, 1)
     clocks.stop()
-    launches_per_step = kernels_per_graph if graphs is not None else (h.launch_count - launches0) / ((WINDOWS * K) + warm)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, nets[(K - 1) % N_SETS], dets, tracks)
+    launches_per_step = kernels_per_graph if graphs is not None else (h.launch_count - launches0) / (K + warm)
     value = world * STREAMS * K / (ms * 1e-3)
     n_tracks = int(tracks["count"].sum().item())
     h.poll_status()
@@ -686,8 +715,8 @@ def run_gpu(args) -> None:
                 "warmup": warm, "ms_per_step": round(ms / K, 5), "higher_is_better": True,
                 "scaling": "weak", "vs_baseline": None, "dtype": "u8/f32", "data": "synthetic",
                 "config": workload_config(world),
-                "timing": dict(win_stats, how="CUDA events around each K-step window, barrier + synchronize on both sides, "
-                                              "max over ranks per window, median over the windows"),
+                "timing": dict(win_stats, how="CUDA events around the K timed steps, barrier + synchronize on both sides, "
+                                              "max over ranks"),
                 "parity_checked": parity is not None, "parity": parity,
                 "roofline": roofline, "roofline_kernels": roofline_kernels,
                 "tick_hbm": {"algorithmic_bytes_per_tick": tick_bytes,
@@ -746,7 +775,10 @@ def main() -> None:
     ap.add_argument("--no-cpu", action="store_true", help="skip the single-core CPU sample")
     ap.add_argument("--no-configs", action="store_true", help="skip the `configs` block (BASELINE.json configs 1, 2, 4, 5)")
     ap.add_argument("--no-parity", action="store_true", help="skip the oracle comparison of two ticks before the timed region")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU path; it does not apply to --impl reference")
     if args.impl == "reference":
         run_reference(args)
     else:

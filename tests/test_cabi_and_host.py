@@ -166,20 +166,115 @@ def test_sharded_id_aggregation_two_ranks_gloo(tmp_path):
     assert all(r["next"] == counter for r in res)
 
 
-def test_registration_shim_wires_the_reference_factory():
-    """INTEGRATION.md §3(a): with the reference importable (build container only), `backend: b200`
-    validates, create_detector dispatches to B200Detector and `tracker.type: b200_iou` selects
-    B200IouTracker.  Without a GPU construction must fail loudly (no silent CPU path)."""
-    ref = "/root/" + "reference/src"
-    if not os.path.isdir(ref):
-        pytest.skip("reference tree not present")
-    sys.path.insert(0, ref)
-    try:
-        import realtime_analytics.config as rcfg
-        import realtime_analytics.detector as rdet
-        import realtime_analytics.pipeline as rpipe
-    except Exception as exc:  # pragma: no cover
-        pytest.skip(f"reference not importable: {exc}")
+def _stand_in_reference():
+    """The three reference modules the shim patches, reduced to what it touches: the backend whitelist of
+    ``DetectorConfig.validate`` (config.py:155-157), ``load_config``, ``create_detector`` (detector.py:54-96) and the names
+    ``pipeline.py`` imports or owns (:33, :452, the pipeline and its stream workers)."""
+    import dataclasses
+    import types
+
+    import yaml
+
+    from realtime_video_analytics_32streams_b200 import types as T
+
+    cfg, det, pipe = (types.ModuleType(f"realtime_analytics.{m}") for m in ("config", "detector", "pipeline"))
+
+    class ConfigError(ValueError):
+        pass
+
+    @dataclasses.dataclass
+    class DetectorConfig:
+        model_path: str = "yolov8n.pt"
+        backend: str = "ultralytics"
+        model_type: str = "yolov8"
+        confidence_threshold: float = 0.5
+        iou_threshold: float = 0.45
+        input_size: list = None
+        half: bool = False
+
+        def validate(self):
+            valid_backends = {"ultralytics", "tensorrt", "onnx", "onnxruntime", "openvino", "rknn", "rk3588"}
+            if self.backend.lower() not in valid_backends:
+                raise ConfigError(f"Unsupported detector backend: {self.backend}")
+
+    @dataclasses.dataclass
+    class TrackerConfig:
+        type: str = "iou"
+        max_age: int = 30
+        max_iou_distance: float = 0.7
+        min_hits: int = 3
+
+    def load_config(path):
+        with open(path) as fh:
+            raw = yaml.safe_load(fh)
+        full = types.SimpleNamespace(detector=DetectorConfig(**raw["detector"]), tracker=TrackerConfig(**raw["tracker"]),
+                                     streams=[T.StreamConfig(**s) for s in raw["streams"]])
+        full.detector.validate()
+        return full
+
+    cfg.ConfigError, cfg.DetectorConfig, cfg.TrackerConfig, cfg.load_config = ConfigError, DetectorConfig, TrackerConfig, load_config
+
+    def create_detector(config):
+        if config.backend.lower() not in ("ultralytics", "tensorrt", "onnx", "onnxruntime", "openvino", "rknn", "rk3588"):
+            raise ValueError(f"Unsupported backend: {config.backend}")
+        return types.SimpleNamespace(config=config)
+
+    det.create_detector = create_detector
+
+    class IouTracker:
+        def __init__(self, config):
+            self.config = config
+
+    class AnalyticsPipeline:
+        def __init__(self, config):
+            self.config = config
+
+        async def wait_closed(self):
+            pass
+
+    class StreamWorker:
+        def __init__(self, context):
+            self.ctx = context
+
+        async def run(self):
+            pass
+
+        async def _process_packet(self, packet):
+            pass
+
+    def apply_roi(frame, polygons):
+        return frame
+
+    def downsample(frame, ratio):
+        return frame
+
+    class MotionFilter:
+        pass
+
+    for f in (apply_roi, downsample, MotionFilter):
+        f.__module__ = "realtime_analytics.filters"
+    pipe.create_detector, pipe.IouTracker, pipe.AnalyticsPipeline, pipe.StreamWorker = (create_detector, IouTracker,
+                                                                                        AnalyticsPipeline, StreamWorker)
+    pipe.apply_roi, pipe.downsample, pipe.MotionFilter = apply_roi, downsample, MotionFilter
+    pkg = types.ModuleType("realtime_analytics")
+    pkg.config, pkg.detector, pkg.pipeline = cfg, det, pipe
+    return {"realtime_analytics": pkg, cfg.__name__: cfg, det.__name__: det, pipe.__name__: pipe}
+
+
+def test_registration_shim_wires_the_reference_factory(monkeypatch):
+    """INTEGRATION.md §3(a): after registration `backend: b200` validates, create_detector dispatches to B200Detector and
+    `tracker.type: b200_iou` selects B200IouTracker; unregistering puts back everything it replaced.  Without a GPU
+    construction must fail loudly (no silent CPU path).  Runs against the reference itself when B200VA_REFERENCE_SRC
+    names its src/ directory, else against a stand-in of the modules the shim patches."""
+    ref = os.environ.get("B200VA_REFERENCE_SRC", "")
+    if os.path.isdir(ref):
+        monkeypatch.syspath_prepend(ref)
+    else:
+        for name, module in _stand_in_reference().items():
+            monkeypatch.setitem(sys.modules, name, module)
+    import realtime_analytics.config as rcfg
+    import realtime_analytics.detector as rdet
+    import realtime_analytics.pipeline as rpipe
     import torch
 
     from realtime_video_analytics_32streams_b200 import register_with_reference

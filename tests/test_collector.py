@@ -1,15 +1,12 @@
 """The in-pipeline tick collector (SURVEY.md §8f-1, collector.py).
 
-CPU part (runs in the build container, where the reference tree is importable): the REAL reference
-``StreamWorker`` objects (pipeline.py:88-262), patched by ``collector.install``, share one tick per frame period and
-produce, per stream, exactly the side effects the unpatched workers produce one frame at a time --
-``metrics.update_counters``, ``kafka.send_tracks`` (track ids, boxes, hits), ``health.update_success`` /
-``update_error`` and the adaptive-FPS fields.  The engine behind the collector is an oracle-backed stand-in there
-(no GPU); the GPU part runs the same collector over the real ``HotPathEngine``.
+CPU part: workers patched with the collector's ``_process_packet`` share one tick per frame period and reproduce, per
+stream, what the reference's own ``StreamWorker`` objects (pipeline.py:88-262) did one frame at a time, as stored in
+tests/golden/pipeline.npz -- processed or skipped, the published track table (ids, boxes, hits), the counters, the
+health calls and the adaptive-FPS fields.  The engine behind the collector is an oracle-backed stand-in there (no
+GPU); the GPU part runs the same collector over the real ``HotPathEngine``.
 """
 import asyncio
-import os
-import sys
 import types
 
 import numpy as np
@@ -18,7 +15,8 @@ import pytest
 import golden_util as G
 from oracle import hotpath as O
 from realtime_video_analytics_32streams_b200 import synth
-from realtime_video_analytics_32streams_b200.collector import TickCollector, install, make_process_packet
+from realtime_video_analytics_32streams_b200.collector import TickCollector, make_process_packet
+from realtime_video_analytics_32streams_b200.types import StreamConfig
 
 H, W, IN_HW = 108, 192, (64, 64)
 CONF, IOU = 0.35, 0.5
@@ -100,122 +98,69 @@ class OracleEngine:
         return out
 
 
-def _same_calls(got, want):
-    assert len(got) == len(want), (len(got), len(want))
-    for g, w in zip(got, want):
-        assert g[0] == w[0] and g[1] == w[1], (g[:2], w[:2])
-        if g[0] == "metrics":
-            assert g == w, (g, w)
-        elif g[0] == "kafka":
-            assert g[2] == w[2] and g[4] == w[4]
-            for k in w[3]:
-                assert np.array_equal(g[3][k], w[3][k]), (g[1], g[2], k)
-
-
-def test_collector_drives_the_real_reference_workers_like_their_own_per_frame_path():
-    ref = "/root/" + "reference/src"
-    if not os.path.isdir(ref):
-        pytest.skip("reference tree not present")
-    sys.path.insert(0, ref)
-    sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden"))
-    try:
-        import realtime_analytics.config as rcfg
-        import realtime_analytics.pipeline as rpipe
-        from realtime_analytics.detector import _TensorRTBaseDetector
-        from realtime_analytics.tracker import IouTracker
-        from realtime_analytics.video_stream import FramePacket
-    except Exception as exc:  # pragma: no cover
-        pytest.skip(f"reference not importable: {exc}")
-
-    class StubDetector(_TensorRTBaseDetector):  # the reference's numpy pre / post with the forward replaced by a lookup
-        def __init__(self, config, input_hw):
-            super().__init__(config, input_hw)
-            self.head = None
-
-        def _infer(self, tensor):
-            return self.head
-
-    det_cfg = rcfg.DetectorConfig(backend="tensorrt", confidence_threshold=CONF, iou_threshold=IOU)
-    trk_cfg = rcfg.TrackerConfig(max_age=3, max_iou_distance=0.5, min_hits=1)
-    streams = [rcfg.StreamConfig(url="x", **_stream_kwargs(i)) for i in range(N_STREAMS)]
-    scenes = [_scene(i) for i in range(N_STREAMS)]
-    frames = [[scenes[i].frame(t) for i in range(N_STREAMS)] for t in range(N_FRAMES)]
-
-    def make_workers(tracker, detector, rec, log):
-        ws = []
-        for s in streams:
-            ctx = rpipe.StreamWorkerContext(stream=s, detector=detector, tracker=tracker, kafka=rec, metrics=rec,
-                                            health=Health(log, s.name))
-            w = rpipe.StreamWorker(ctx)
-            w._maybe_save_snapshot = lambda *a, **k: None
-            ws.append(w)
-        return ws
-
-    # (A) the unmodified reference, one frame at a time, streams in order
-    rec_a, log_a = Recorder(), []
-    det_a = StubDetector(det_cfg, IN_HW)
-    workers_a = make_workers(IouTracker(trk_cfg), det_a, rec_a, log_a)
-    state_a = []
-
-    async def drive_a():
-        for t in range(N_FRAMES):
-            for i, w in enumerate(workers_a):
-                det_a.head = _head(i, t)
-                await w._process_packet(FramePacket(streams[i], frames[t][i], t, 0.0))
-            state_a.append([(w._process_every, w._idle_frames, w._frame_index) for w in workers_a])
-
-    asyncio.run(drive_a())
-    assert any(c[0] == "kafka" for c in rec_a.calls) and any(c[0] == "metrics" and c[3] == 0 for c in rec_a.calls)
-
-    # (B) the same workers patched: every frame period is ONE engine tick
-    saved = {k: getattr(rpipe.StreamWorker, k) for k in ("_process_packet", "run", "__init__")}
-    saved_p = {k: getattr(rpipe.AnalyticsPipeline, k) for k in ("__init__", "wait_closed")}
-    engines = []
-
-    def engine_factory(strs, detector, cfg):
-        e = OracleEngine(strs, CONF, IOU, (3, 0.5, 1), _head)
-        engines.append(e)
-        return e
-
-    try:
-        install(rpipe, engine_factory, max_wait_s=5.0)
-        install(rpipe, engine_factory)  # idempotent
-        cfg = rcfg.PipelineConfig(streams=streams, detector=det_cfg, tracker=trk_cfg, kafka=rcfg.KafkaSinkConfig(enabled=False))
-        pipe = rpipe.AnalyticsPipeline(cfg)
-        rec_b, log_b = Recorder(), []
-        det_b = types.SimpleNamespace(config=det_cfg)
-        workers_b = make_workers(pipe.tracker, det_b, rec_b, log_b)
-        state_b = []
-
-        async def drive_b():
-            for t in range(N_FRAMES):
-                await asyncio.gather(*[w._process_packet(FramePacket(streams[i], frames[t][i], t, 0.0))
-                                       for i, w in enumerate(workers_b)])
-                state_b.append([(w._process_every, w._idle_frames, w._frame_index) for w in workers_b])
-            for col in pipe._b200va["collectors"].values():
-                assert col.ticks == N_FRAMES and col.frames == N_FRAMES * N_STREAMS
-                await col.close()
-
-        asyncio.run(drive_b())
-    finally:
-        for k, v in saved.items():
-            setattr(rpipe.StreamWorker, k, v)
-        for k, v in saved_p.items():
-            setattr(rpipe.AnalyticsPipeline, k, v)
-        rpipe.StreamWorker._b200va_batched = False
-    assert len(engines) == 1 and [s.name for s in engines[0].streams] == [s.name for s in streams]
-    assert all(all(b) for b in engines[0].batches) and len(engines[0].batches) == N_FRAMES
-    # same side effects per stream, in the same order (calls of different streams interleave differently: the batched
-    # workers resume after the tick, so compare stream by stream)
-    for s in streams:
-        _same_calls([c for c in rec_b.calls if c[1] == s.name], [c for c in rec_a.calls if c[1] == s.name])
-        assert [c for c in log_b if c[1] == s.name] == [c for c in log_a if c[1] == s.name]
-    assert state_b == state_a
-
-
 class _Packet:
     def __init__(self, stream, frame, frame_id):
         self.stream, self.frame, self.frame_id = stream, frame, frame_id
+
+
+def test_collector_workers_reproduce_the_reference_workers_per_frame_trace():
+    """Workers patched with the collector's ``_process_packet``, both streams sharing one tick per frame period, against
+    what the reference's own ``StreamWorker._process_packet`` did one frame at a time on the same inputs
+    (tests/golden/pipeline.npz, tests/golden/make_golden.py): per frame whether it was processed, the adaptive-FPS
+    fields and the stream's track table, which is what the worker publishes."""
+    z = G.load("pipeline")
+    h, w, ih, iw = z["pipe_cfg"].tolist()
+    polys = [[tuple(p) for p in z["pipe_polys"].tolist()]]
+    scenes = [synth.MotionScene(61, h, w, rect=30, speed=11), synth.MotionScene(62, h, w, static=True)]
+    burst = synth.MotionScene(63, h, w, rect=30, speed=11)
+    streams = [StreamConfig(name=f"cam{i}", roi_polygons=polys if i == 0 else None, motion_filter=True, motion_threshold=0.02,
+                            downsample_ratio=1.0 if i == 0 else 0.75, adaptive_fps=True, target_fps=25, min_target_fps=5,
+                            idle_frame_tolerance=3) for i in range(2)]
+
+    def head(i, t):
+        n_obj = 5 if ((i == 0 or 8 <= t <= 12) and t < 14) else 0
+        return synth.synth_head(7000 + 10 * t + i, 20, 256, n_obj, dup=2, input_hw=(ih, iw))[None]
+
+    def frame(i, t):
+        return (burst if (i == 1 and 8 <= t <= 12) else scenes[i]).frame(t)
+
+    assert (ih, iw) == IN_HW
+    eng = OracleEngine(streams, CONF, IOU, (3, 0.5, 1), head)
+    col = TickCollector(eng, max_wait_s=5.0)
+    rec, log = Recorder(), []
+    proc = make_process_packet(lambda wk: col)
+    workers = [types.SimpleNamespace(ctx=types.SimpleNamespace(metrics=rec, kafka=rec, health=Health(log, s.name)),
+                                     _frame_index=0, _maybe_save_snapshot=lambda *a, **k: None, _process_every=1,
+                                     _idle_frames=0) for s in streams]
+    n = int(z["pipe_n"][0])
+    n_frames = n // len(streams)
+
+    async def drive():
+        for t in range(n_frames):
+            n_calls = len(rec.calls)
+            await asyncio.gather(*[proc(wk, _Packet(s, frame(i, t), t)) for i, (s, wk) in enumerate(zip(streams, workers))])
+            calls = rec.calls[n_calls:]
+            for i, (s, wk) in enumerate(zip(streams, workers)):
+                k = t * len(streams) + i
+                zi, zt, processed, pe, idle = z[f"pipe_{k}_hdr"].tolist()
+                assert (zi, zt) == (i, t)
+                assert [G.sha(frame(i, t)), G.sha(head(i, t))] == z[f"pipe_{k}_sha"].tolist(), "synthetic generator drifted"
+                want = {kk: z[f"pipe_{k}_t{kk}"] for kk in ("id", "cls", "conf", "box", "age", "hits")}
+                sent = [c for c in calls if c[0] == "kafka" and c[1] == s.name]
+                metrics = [c for c in calls if c[0] == "metrics" and c[1] == s.name]
+                assert len(metrics) == 1 and metrics[0][2] == 1, (t, s.name)
+                assert len(sent) == int(processed), (t, s.name)
+                if processed:
+                    assert sent[0][2] == t and metrics[0][4] == len(want["id"])
+                    for kk, v in want.items():
+                        assert np.array_equal(sent[0][3][kk], v), (t, s.name, kk)
+                assert (wk._process_every, wk._idle_frames, wk._frame_index) == (pe, idle, t + 1), (t, s.name)
+        assert col.ticks == n_frames and col.frames == n
+        await col.close()
+
+    asyncio.run(drive())
+    assert all(all(b) for b in eng.batches)
+    assert log == [("health_ok", s.name) for _ in range(n_frames) for s in streams]
 
 
 def test_collector_partial_ticks_errors_and_retired_streams():
