@@ -276,9 +276,12 @@ B200VA_API int b200va_motion_preprocess(b200va_handle h, const uint8_t* const* f
  * meta       HOST [batch] letterbox geometry of each frame
  * conf_thr / iou_thr  the Python floats of DetectorConfig; rounded to float32 exactly where
  *            NumPy does (detector.py:312, :373)
- * classes    HOST int32 [n_classes] whitelist (detector.py:313-314) or NULL
+ * classes    HOST int32 [n_classes] whitelist (detector.py:313-314) or NULL; ids below 0 or at or above the
+ *            head's class count match nothing (np.isin); an id in [2048, class count) is refused with
+ *            B200VA_ERR_INVALID (the kernels hold the whitelist as a 2048-bit map)
  * out        kept detections in keep order (score descending), at most max_dets per frame
- * Equal scores are ordered higher-candidate-index first (stable argsort reversed). */
+ * Equal scores are ordered higher-candidate-index first (stable argsort reversed); -0.0 and +0.0 are
+ * equal scores, and each detection keeps the sign of its own score. */
 B200VA_API int b200va_postprocess(b200va_handle h, const float* head, int layout, int batch, int channels, int anchors,
                        const b200va_letterbox* meta, double conf_thr, double iou_thr, const int32_t* classes,
                        int n_classes, int score_mode, int nms_mode, double filter_conf_thr_f64, int use_filter,
@@ -389,7 +392,8 @@ B200VA_API int b200va_preprocess_geom(b200va_handle h, const uint8_t* const* fra
  * scores keep the lower anchor first (stable descending sort); the first max_det survivors are un-letterboxed
  * with gain = min(in_h/h, in_w/w), pad = round((in - size * gain) / 2 - 0.1), true division by float32(gain),
  * clamp to [0, w] x [0, h].  max_nms (30000) is never reached: candidates are bounded by max_candidates.
- * in_h / in_w: shape of the network input the head was computed from.  filter_*: as in b200va_postprocess. */
+ * in_h / in_w: shape of the network input the head was computed from.  filter_*, classes and signed zeros: as in
+ * b200va_postprocess. */
 B200VA_API int b200va_postprocess_ultralytics(b200va_handle h, const float* head, int layout, int batch, int channels,
                                               int anchors, const int* src_h, const int* src_w, int in_h, int in_w,
                                               double conf_thr, double iou_thr, const int32_t* classes, int n_classes,

@@ -167,8 +167,13 @@ def nms(boxes: np.ndarray, scores: np.ndarray, iou_threshold: float, cls: Option
     return keep
 
 
-def decode_candidates(pred: np.ndarray, conf_thr: float, classes: Optional[Sequence[int]], v8_native: bool = False):
+def decode_candidates(pred: np.ndarray, conf_thr: float, classes: Optional[Sequence[int]], v8_native: bool = False,
+                      layout: Optional[str] = None):
     """detector.py:278-317: layout fix-up, objectness x class score, argmax, filters.
+
+    ``layout`` (not a reference feature; the explicit ``layout`` argument of the C ABI): ``"cm"`` for a
+    [C, A] head, ``"am"`` for [A, C]; None applies the reference's rule (transpose when rows < columns),
+    which calls a head with A <= C anchor-major.
 
     Returns (xywh[N,4] f32, conf[N] f32, cls[N] int64, anchor_index[N]) or None for the
     "unexpected shape" early-out (:285-287).
@@ -179,8 +184,13 @@ def decode_candidates(pred: np.ndarray, conf_thr: float, classes: Optional[Seque
         if pred.shape[0] != 1:
             raise ValueError("cannot select an axis to squeeze out which has size not equal to one")
         pred = pred[0]
-    if pred.shape[0] != 0 and pred.shape[0] < pred.shape[1]:
+    if layout is None:
+        if pred.shape[0] != 0 and pred.shape[0] < pred.shape[1]:
+            pred = pred.T
+    elif layout == "cm":
         pred = pred.T
+    elif layout != "am":
+        raise ValueError(f"unknown layout {layout!r}")
     if pred.ndim != 2 or pred.shape[1] < 5:
         return None
     pred = pred.astype(F32, copy=False)
@@ -221,10 +231,11 @@ def scale_boxes(b: np.ndarray, meta: dict) -> np.ndarray:
 
 
 def postprocess(pred: np.ndarray, meta: dict, conf_thr: float, iou_thr: float,
-                classes: Optional[Sequence[int]] = None, v8_native: bool = False, class_aware: bool = False) -> List[Det]:
+                classes: Optional[Sequence[int]] = None, v8_native: bool = False, class_aware: bool = False,
+                layout: Optional[str] = None) -> List[Det]:
     """``_TensorRTBaseDetector._postprocess`` (detector.py:266-338); output in keep order.
-    ``v8_native`` / ``class_aware`` select the additive modes (both False = the reference)."""
-    cand = decode_candidates(pred, conf_thr, classes, v8_native)
+    ``v8_native`` / ``class_aware`` / ``layout`` select the additive modes (all default = the reference)."""
+    cand = decode_candidates(pred, conf_thr, classes, v8_native, layout)
     if cand is None:
         return []
     xywh, conf, cls, _ = cand

@@ -41,7 +41,7 @@ struct b200va_ctx {
   std::recursive_mutex mu;  // recursive: b200va_tick holds it while calling the per-step entry points
 
   // ---- post-process scratch (device), all [max_batch, max_candidates] ----
-  unsigned long long* cand_key = nullptr;  // (score bits << 32) | anchor index
+  unsigned long long* cand_key = nullptr;  // (score bits << 32) | anchor tie rule | slot (cand_key() in postprocess.cu)
   float4* cand_box = nullptr;              // xyxy, frame pixels
   int32_t* cand_cls = nullptr;
   int32_t* cand_count = nullptr;           // [max_batch]

@@ -27,9 +27,11 @@ struct PostFrame {
   float left, top, scale, xmax, ymax;
 };
 
+constexpr int kClassMaskIds = 2048;  // class ids the whitelist bitmap covers (the host refuses larger ids the head can produce)
+
 struct PostParams {
   PostFrame f[B200VA_LAUNCH_FRAMES];
-  uint32_t class_mask[64];  // whitelist bitmap over class ids (np.isin, detector.py:313-314)
+  uint32_t class_mask[kClassMaskIds / 32];  // whitelist bitmap over class ids (np.isin, detector.py:313-314)
   const float* head;
   unsigned long long* cand_key;
   float4* cand_box;
@@ -55,6 +57,22 @@ __device__ __forceinline__ float unorder_bits(uint32_t u) {
   uint32_t b = (u & 0x80000000u) ? (u ^ 0x80000000u) : ~u;
   return __uint_as_float(b);
 }
+
+// Candidate key, descending order = NMS order: [63:32] order_bits(score) | [31:14] anchor tie rule | [13] the score is
+// -0.0 | [12:0] candidate slot (max_candidates <= 8192).  -0.0 and +0.0 rank equal, as NumPy and torch compare them:
+// both take the key of +0.0 and bit 13 keeps the sign for the emitted confidence.  Bit 13 never decides an order
+// because the tie field above it is unique within a frame.
+constexpr unsigned long long kKeySlotMask = 0x1fffull;
+constexpr unsigned long long kKeyNegZero = 1ull << 13;
+__device__ __forceinline__ unsigned long long cand_key(float conf, uint32_t tie, int slot) {
+  const bool neg_zero = __float_as_uint(conf) == 0x80000000u;
+  return ((unsigned long long)order_bits(neg_zero ? 0.f : conf) << 32) | ((unsigned long long)tie << 14) |
+         (neg_zero ? kKeyNegZero : 0ull) | (unsigned long long)(uint32_t)slot;
+}
+__device__ __forceinline__ float key_conf(unsigned long long k) {
+  return (k & kKeyNegZero) ? -0.f : unorder_bits((uint32_t)(k >> 32));
+}
+__device__ __forceinline__ int key_slot(unsigned long long k) { return (int)(k & kKeySlotMask); }
 
 // ultralytics scale_boxes + clip_boxes (utils/ops.py): un-pad, true division by float32(gain), clamp to [0, w] x [0, h]
 // (torch CPU semantics; torch CUDA multiplies by the float32 reciprocal instead).
@@ -104,7 +122,7 @@ __device__ __forceinline__ float4 decode_box(float cx, float cy, float w, float 
 
 __device__ __forceinline__ bool class_allowed(const PostParams& p, int cls) {
   if (!p.use_mask) return true;
-  if (cls >= 2048) return false;
+  if (cls >= kClassMaskIds) return false;  // (never whitelisted: the host refuses such an id)
   return (p.class_mask[cls >> 5] >> (cls & 31)) & 1u;
 }
 
@@ -113,8 +131,7 @@ __device__ __forceinline__ void emit_candidate(const PostParams& p, int frame, i
   if (pos >= p.max_cand) return;  // overflow is flagged by k_sort_nms from the raw count
   const size_t o = (size_t)frame * p.max_cand + pos;
   const uint32_t tie = p.ultra ? (0x3ffffu - (uint32_t)anchor) : (uint32_t)anchor;  // descending sort: which anchor first on equal scores
-  p.cand_key[o] = ((unsigned long long)order_bits(conf) << 32) | ((unsigned long long)tie << 14) |
-                  (unsigned long long)(uint32_t)pos;
+  p.cand_key[o] = cand_key(conf, tie, pos);
   p.cand_box[o] = box;
   p.cand_cls[o] = cls;
 }
@@ -550,7 +567,8 @@ __global__ void __launch_bounds__(32 * (kRingWarps + 1)) k_decode_ring(const __g
       }
     }
     // resolve the class of the (rare) anchors that pass the confidence filter: first row of the winning group whose
-    // score equals the maximum; the rows come back from L2
+    // score equals the maximum; the rows come back from L2.  That row's score is the confidence: max.NaN.f32 makes
+    // +0.0 of a -0.0 / +0.0 pair, np.argmax sees them equal and reports the first
     int cls[4] = {0, 0, 0, 0};
     if (active) {
       const float* hd = p.head + (size_t)(frame0 + frame) * C * A + a_tile + 4 * g;
@@ -559,11 +577,14 @@ __global__ void __launch_bounds__(32 * (kRingWarps + 1)) k_decode_ring(const __g
       for (int k = 0; k < 4; ++k) {
         if (!(p.ultra ? best[k] > p.conf_thr : best[k] >= p.conf_thr)) continue;
         cls[k] = grp[k];
-        for (int j = 0; j < 4 && grp[k] + j < C - cls0; ++j)
-          if (__fmul_rn(__ldg(hd + (size_t)(cls0 + grp[k] + j) * A + k), oa[k]) == best[k]) {
+        for (int j = 0; j < 4 && grp[k] + j < C - cls0; ++j) {
+          const float s = __fmul_rn(__ldg(hd + (size_t)(cls0 + grp[k] + j) * A + k), oa[k]);
+          if (s == best[k]) {
             cls[k] = grp[k] + j;
+            best[k] = s;
             break;
           }
+        }
       }
     }
     emit_quad(p, frame, lane, a_tile + 4 * g, active, best, cls, 0u, cx, cy, bwid, bh);
@@ -819,7 +840,7 @@ __device__ __forceinline__ void nms_general_body(const NmsParams& p, const int f
   PHASE_STAMP(p.dbg, 18);
   // gather boxes and class ids of the sorted candidates into shared memory in one round of global loads
   for (int i = tid; i < n; i += NT) {
-    const size_t o = cbase + (keys[i] & 0x3fffull);
+    const size_t o = cbase + key_slot(keys[i]);
     float4 b = p.cand_box[o];
     const int cl = p.cand_cls[o];
     if (p.ultra && !p.ultra_agnostic) {  // boxes = x[:, :4] + x[:, 5:6] * max_wh, float32 (the rounding is part of the semantics)
@@ -1108,7 +1129,7 @@ __device__ __forceinline__ void nms_general_body(const NmsParams& p, const int f
   if (p.use_filter) {
     for (int i = tid; i < n; i += NT) {
       if ((keep_w[i >> 5] >> (i & 31)) & 1u) {
-        const float conf = unorder_bits((uint32_t)(keys[i] >> 32));
+        const float conf = key_conf(keys[i]);
         if (!((double)conf >= p.filter_thr)) atomicAnd(&keep_w[i >> 5], ~(1u << (i & 31)));
       }
     }
@@ -1135,10 +1156,10 @@ __device__ __forceinline__ void nms_general_body(const NmsParams& p, const int f
       if (pos < p.max_dets) {
         const size_t o = (size_t)frame * p.max_dets + pos;
         float4 b = box[i];
-        const int slot = (int)(keys[i] & 0x3fffull);
+        const int slot = key_slot(keys[i]);
         if (ultra) b = ultra_scale_box(small ? sm.ubox[slot] : p.cand_box[cbase + slot], p.f[frame]);  // the un-shifted box
         else if (b.x != b.x) b = small ? sm.ubox[slot] : p.cand_box[cbase + slot];  // (nan_box_view: emit the box as decoded)
-        const float cf = unorder_bits((uint32_t)(keys[i] >> 32));
+        const float cf = key_conf(keys[i]);
         const int cl = small ? sm.ucls[slot] : p.cand_cls[cbase + slot];  // the full int32 class id (scl[] holds 16 bits)
         reinterpret_cast<float4*>(p.out_box)[o] = b;
         p.out_conf[o] = cf;
@@ -1250,7 +1271,7 @@ __device__ __forceinline__ void nms_frame(const NmsParams& p, const int frame, u
     PHASE_STAMP(p.dbg, 18);
     if (tid < n) {
       const unsigned long long k = sm.sorted[tid];
-      const int slot = (int)(k & 0x3fffull);
+      const int slot = key_slot(k);
       float4 b = sm.ubox[slot];
       const int cl = sm.ucls[slot];
       if (ultra && !p.ultra_agnostic) {  // boxes = x[:, :4] + x[:, 5:6] * max_wh, float32 (the rounding is part of the semantics)
@@ -1391,8 +1412,8 @@ __device__ __forceinline__ void nms_frame(const NmsParams& p, const int frame, u
           acc_kept += __popcll(kept);
         }
         if (p.use_filter) {
-          m0 = m0 && (double)unorder_bits((uint32_t)(sm.keys[r0] >> 32)) >= p.filter_thr;
-          m1 = m1 && (double)unorder_bits((uint32_t)(sm.keys[r1] >> 32)) >= p.filter_thr;
+          m0 = m0 && (double)key_conf(sm.keys[r0]) >= p.filter_thr;
+          m1 = m1 && (double)key_conf(sm.keys[r1]) >= p.filter_thr;
         }
         const uint32_t w0 = __ballot_sync(0xffffffffu, m0), w1 = __ballot_sync(0xffffffffu, m1);
         if (tid == 0) {
@@ -1422,10 +1443,10 @@ __device__ __forceinline__ void nms_frame(const NmsParams& p, const int frame, u
       if (pos < p.max_dets) {
         const size_t o = (size_t)frame * p.max_dets + pos;
         float4 b = box[i];
-        const int slot = (int)(keys[i] & 0x3fffull);
+        const int slot = key_slot(keys[i]);
         if (ultra) b = ultra_scale_box(small ? sm.ubox[slot] : p.cand_box[cbase + slot], p.f[frame]);  // the un-shifted box
         else if (b.x != b.x) b = small ? sm.ubox[slot] : p.cand_box[cbase + slot];  // (nan_box_view: emit the box as decoded)
-        const float cf = unorder_bits((uint32_t)(keys[i] >> 32));
+        const float cf = key_conf(keys[i]);
         const int cl = small ? sm.ucls[slot] : p.cand_cls[cbase + slot];  // the full int32 class id (scl[] holds 16 bits)
         reinterpret_cast<float4*>(p.out_box)[o] = b;
         p.out_conf[o] = cf;
@@ -1870,11 +1891,11 @@ __device__ __forceinline__ void dense_resolve_frame(const NmsParams& p, const De
   // the score the keys are ordered by, so the boxes that pass are a prefix and their ranks do not move)
   auto emit = [&](const unsigned long long k, const int pos) {
     if (ultra && pos >= p.max_det_cap) return;
-    const float conf = unorder_bits((uint32_t)(k >> 32));
+    const float conf = key_conf(k);
     if (p.use_filter && !((double)conf >= p.filter_thr)) return;
     atomicAdd(&s_out, 1);
     if (pos >= p.max_dets) return;
-    const int slot = (int)(k & 0x3fffull);
+    const int slot = key_slot(k);
     const size_t o = (size_t)frame * p.max_dets + pos;
     float4 b = p.cand_box[cbase + slot];
     if (ultra) b = ultra_scale_box(b, p.f[frame]);
@@ -2185,6 +2206,12 @@ static int postprocess_impl(b200va_handle h, const float* head, int layout, int 
     return B200VA_OK;
   }
   REQUIRE(h, n_classes >= 0 && (n_classes == 0 || classes), "class whitelist is NULL");
+  // the whitelist is a bitmap over class ids 0..2047 in the kernel parameters; a larger id that the head can produce is
+  // refused rather than silently never matched (ids < 0 or >= the class count match nothing, as in np.isin)
+  const int n_cls_rows = channels - ((score_mode == B200VA_SCORE_REF_COMPAT && channels > 5) ? 5 : 4);
+  for (int k = 0; k < n_classes; ++k)
+    REQUIRE(h, classes[k] < kClassMaskIds || classes[k] >= n_cls_rows,
+            "class whitelist id %d: ids >= %d are not supported", classes[k], kClassMaskIds);
 
   for (int base = 0; base < batch; base += B200VA_LAUNCH_FRAMES) {
     const int n = batch - base < B200VA_LAUNCH_FRAMES ? batch - base : B200VA_LAUNCH_FRAMES;
@@ -2215,7 +2242,7 @@ static int postprocess_impl(b200va_handle h, const float* head, int layout, int 
     if (n_classes > 0) {  // an empty list means "no filter" (detector.py:313: `if self.config.classes`)
       p.use_mask = 1;
       for (int k = 0; k < n_classes; ++k)
-        if (classes[k] >= 0 && classes[k] < 2048) p.class_mask[classes[k] >> 5] |= 1u << (classes[k] & 31);
+        if (classes[k] >= 0 && classes[k] < kClassMaskIds) p.class_mask[classes[k] >> 5] |= 1u << (classes[k] & 31);
     }
     const bool defer = fuse && fuse->defer && base == 0 && n == batch;
     const int set = defer ? h->cand_set : 0;  // ordinary calls always use set 0 (decode and NMS in the same call)
