@@ -68,6 +68,15 @@ enum b200va_head_layout {
   B200VA_HEAD_ANCHOR_MAJOR = 1   /* [B, A, C]  e.g. YOLOv5 [B,25200,85]  */
 };
 
+/* OR-ed into `layout` (b200va_postprocess, b200va_postprocess_ultralytics, b200va_tick_args.layout): the head is
+ * IEEE binary16 in the same [B, C, A] / [B, A, C] layout, as a model exported for fp16 input returns it, and is
+ * read in place -- half the bytes of the float32 head, and no conversion pass before the call.  Every element is
+ * widened to float32 exactly where it is loaded (float16 -> float32 is exact, subnormals included) and all
+ * arithmetic after that is the float32 code: the results are bit-for-bit those of the same call on the head
+ * converted to float32.  An fp16 head never takes the TMA ring decode (B200VA_DECODE_IMPL=2 selects the register
+ * kernels for it).  Any other bit in `layout` is refused with B200VA_ERR_INVALID. */
+#define B200VA_HEAD_F16 0x200
+
 /* Scoring rule.  REF_COMPAT is what detector.py:294-307 computes for BOTH model types:
  * C>5: score_k = head[5+k] * head[4];  C==5: score_0 = head[4]. */
 enum b200va_score_mode {
@@ -272,7 +281,8 @@ B200VA_API int b200va_motion_preprocess(b200va_handle h, const uint8_t* const* f
  * filter_detections (detector.py:99-103, called at pipeline.py:182) when use_filter != 0:
  * kept boxes whose float64 confidence is below filter_conf_thr_f64 still suppress others but
  * are not emitted.
- * head       DEVICE float32, layout per `layout`; B frames, C channels, A anchors
+ * head       DEVICE float32 (float16 with B200VA_HEAD_F16 in `layout`), layout per `layout`; B frames, C channels,
+ *            A anchors
  * meta       HOST [batch] letterbox geometry of each frame
  * conf_thr / iou_thr  the Python floats of DetectorConfig; rounded to float32 exactly where
  *            NumPy does (detector.py:312, :373)
@@ -282,7 +292,7 @@ B200VA_API int b200va_motion_preprocess(b200va_handle h, const uint8_t* const* f
  * out        kept detections in keep order (score descending), at most max_dets per frame
  * Equal scores are ordered higher-candidate-index first (stable argsort reversed); -0.0 and +0.0 are
  * equal scores, and each detection keeps the sign of its own score. */
-B200VA_API int b200va_postprocess(b200va_handle h, const float* head, int layout, int batch, int channels, int anchors,
+B200VA_API int b200va_postprocess(b200va_handle h, const void* head, int layout, int batch, int channels, int anchors,
                        const b200va_letterbox* meta, double conf_thr, double iou_thr, const int32_t* classes,
                        int n_classes, int score_mode, int nms_mode, double filter_conf_thr_f64, int use_filter,
                        const b200va_dets* out, void* stream);
@@ -394,7 +404,7 @@ B200VA_API int b200va_preprocess_geom(b200va_handle h, const uint8_t* const* fra
  * clamp to [0, w] x [0, h].  max_nms (30000) is never reached: candidates are bounded by max_candidates.
  * in_h / in_w: shape of the network input the head was computed from.  filter_*, classes and signed zeros: as in
  * b200va_postprocess. */
-B200VA_API int b200va_postprocess_ultralytics(b200va_handle h, const float* head, int layout, int batch, int channels,
+B200VA_API int b200va_postprocess_ultralytics(b200va_handle h, const void* head, int layout, int batch, int channels,
                                               int anchors, const int* src_h, const int* src_w, int in_h, int in_w,
                                               double conf_thr, double iou_thr, const int32_t* classes, int n_classes,
                                               int agnostic, int max_det, double filter_conf_thr_f64, int use_filter,
@@ -442,7 +452,7 @@ typedef struct b200va_tick_args {
   int dst_h, dst_w, out_format;
   b200va_letterbox* meta_out;
   /* b200va_postprocess */
-  const float* head;
+  const void* head; /* float32, or float16 with B200VA_HEAD_F16 in `layout` */
   int layout, head_batch, channels, anchors;
   const b200va_letterbox* meta;
   double conf_thr, iou_thr;

@@ -19,6 +19,7 @@ OK, ERR_INVALID, ERR_CUDA, ERR_CAPACITY, ERR_STATE = 0, -1, -2, -3, -4
 OUT_F32_RGB_NCHW, OUT_F16_RGB_NCHW, OUT_U8_BGR_NCHW, OUT_U8_BGR_NHWC = 0, 1, 2, 3
 OUT_FLAG_PADS_VALID = 0x100  # OR into the format: the pad rows of `out` are still valid from an earlier call
 HEAD_CHANNEL_MAJOR, HEAD_ANCHOR_MAJOR = 0, 1
+HEAD_F16 = 0x200  # OR into the layout: the head is float16 (read in place, exactly as its float32 widening)
 SCORE_REF_COMPAT, SCORE_V8_NATIVE = 0, 1
 NMS_AGNOSTIC, NMS_CLASS_AWARE = 0, 1
 
@@ -583,17 +584,26 @@ class Handle:
     def _dets_struct(d) -> Dets:
         return Dets(d["bbox_xyxy"].data_ptr(), d["conf"].data_ptr(), d["cls"].data_ptr(), d["count"].data_ptr())
 
+    def _head_args(self, head, layout):
+        """(batch, layout | HEAD_F16 for a float16 head, channels, anchors) of a contiguous CUDA float32 / float16 head
+        [B, C, A] (channel major) or [B, A, C] (anchor major).  layout=None: detector.py:282-283 -- transpose when
+        shape[0] < shape[1]."""
+        t = self.torch
+        if not (head.is_cuda and head.dtype in (t.float32, t.float16) and head.dim() == 3 and head.is_contiguous()):
+            raise ValueError("head must be a contiguous CUDA float32 / float16 tensor [B, C, A] or [B, A, C]")
+        b, d1, d2 = head.shape
+        if layout is None:
+            layout = HEAD_CHANNEL_MAJOR if (d1 != 0 and d1 < d2) else HEAD_ANCHOR_MAJOR
+        layout &= ~HEAD_F16
+        channels, anchors = (d1, d2) if layout == HEAD_CHANNEL_MAJOR else (d2, d1)
+        return b, layout | (HEAD_F16 if head.dtype == t.float16 else 0), channels, anchors
+
     def postprocess(self, head, metas, conf_thr: float, iou_thr: float, classes=None, layout=None,
                     filter_conf: Optional[float] = None, out=None, score_mode: int = SCORE_REF_COMPAT,
                     nms_mode: int = NMS_AGNOSTIC):
-        """Decode + filter + NMS for ``head`` [B,C,A] (channel major) or [B,A,C] (anchor major)."""
-        t = self.torch
-        if not (head.is_cuda and head.dtype == t.float32 and head.dim() == 3 and head.is_contiguous()):
-            raise ValueError("head must be a contiguous CUDA float32 tensor [B, C, A] or [B, A, C]")
-        b, d1, d2 = head.shape
-        if layout is None:  # detector.py:282-283: transpose when shape[0] < shape[1]
-            layout = HEAD_CHANNEL_MAJOR if (d1 != 0 and d1 < d2) else HEAD_ANCHOR_MAJOR
-        channels, anchors = (d1, d2) if layout == HEAD_CHANNEL_MAJOR else (d2, d1)
+        """Decode + filter + NMS for ``head`` [B,C,A] (channel major) or [B,A,C] (anchor major), float32 or float16
+        (read in place: the same results as ``head.float()``)."""
+        b, layout, channels, anchors = self._head_args(head, layout)
         if out is None:
             out = self.alloc_dets(b)
         marr = metas if isinstance(metas, C.Array) else (Letterbox * max(b, 1))(*metas)
@@ -631,13 +641,7 @@ class Handle:
                                 filter_conf: Optional[float] = None, out=None):
         """``ops.non_max_suppression`` + ``ops.scale_boxes`` for ``head`` [B, 4 + nc, A] (or [B, A, 4 + nc]).
         ``frame_hw``: (h, w) of every original frame; ``in_hw``: the network-input shape the head came from."""
-        t = self.torch
-        if not (head.is_cuda and head.dtype == t.float32 and head.dim() == 3 and head.is_contiguous()):
-            raise ValueError("head must be a contiguous CUDA float32 tensor [B, C, A] or [B, A, C]")
-        b, d1, d2 = head.shape
-        if layout is None:
-            layout = HEAD_CHANNEL_MAJOR if (d1 != 0 and d1 < d2) else HEAD_ANCHOR_MAJOR
-        channels, anchors = (d1, d2) if layout == HEAD_CHANNEL_MAJOR else (d2, d1)
+        b, layout, channels, anchors = self._head_args(head, layout)
         if out is None:
             out = self.alloc_dets(b)
         cls_arr = (C.c_int32 * len(classes))(*[int(c) for c in classes]) if classes else None
@@ -730,12 +734,7 @@ class Handle:
             a.net_out, a.dst_h, a.dst_w, a.out_format, a.meta_out = net_out.data_ptr(), dh, dw, fmt, fb.metas
             keep += [fb, net_out]
         if head is not None:
-            if not (head.is_cuda and head.dtype == t.float32 and head.dim() == 3 and head.is_contiguous()):
-                raise ValueError("head must be a contiguous CUDA float32 tensor [B, C, A] or [B, A, C]")
-            b, d1, d2 = head.shape
-            if layout is None:
-                layout = HEAD_CHANNEL_MAJOR if (d1 != 0 and d1 < d2) else HEAD_ANCHOR_MAJOR
-            channels, anchors = (d1, d2) if layout == HEAD_CHANNEL_MAJOR else (d2, d1)
+            b, layout, channels, anchors = self._head_args(head, layout)
             marr = metas if isinstance(metas, C.Array) else (Letterbox * max(b, 1))(*metas)
             cls_arr = (C.c_int32 * len(classes))(*[int(c) for c in classes]) if classes else None
             if dets is None:

@@ -5,7 +5,8 @@
 // All float32 arithmetic uses explicit round-to-nearest intrinsics in NumPy's operation order
 // (no FMA contraction, true division), so kept indices, scores and boxes are bit-identical.
 //
-//   k_decode_cm / k_decode_am   one pass over the head tensor (the only HBM-heavy step):
+//   k_decode_cm / k_decode_am   one pass over the head tensor (the only HBM-heavy step; k_decode16_* read a float16
+//       head in place with the same code):
 //       objectness x class score, first-max argmax, confidence / class filter, xywh -> xyxy,
 //       un-letterbox, clip; survivors are compacted per frame with warp ballots.
 //   k_sort_nms                  one CTA per frame: bitonic sort of (score, anchor) keys in shared
@@ -32,7 +33,7 @@ constexpr int kClassMaskIds = 2048;  // class ids the whitelist bitmap covers (t
 struct PostParams {
   PostFrame f[B200VA_LAUNCH_FRAMES];
   uint32_t class_mask[kClassMaskIds / 32];  // whitelist bitmap over class ids (np.isin, detector.py:313-314)
-  const float* head;
+  const void* head;  // float32, or float16 for the k_decode16_* kernels
   unsigned long long* cand_key;
   float4* cand_box;
   int32_t* cand_cls;
@@ -136,19 +137,71 @@ __device__ __forceinline__ void emit_candidate(const PostParams& p, int frame, i
   p.cand_cls[o] = cls;
 }
 
+// Head elements.  The head is float32, or IEEE binary16 (B200VA_HEAD_F16); the decode bodies below are templates
+// over that element type T, wrapped by one __global__ function per type.  HeadVec<T, N> is N consecutive elements
+// of one channel row fetched by ONE load and held as loaded -- packed halves for float16, so the rows a thread keeps
+// in flight cost N * sizeof(T) bytes of registers each -- and v[k] widens element k to float32 where it is used.
+// float16 -> float32 is exact (subnormals included: cvt.f32.f16 does not flush), so everything after the load is
+// the float32 code and an fp16 head decodes exactly like its float32 widening.
+__device__ __forceinline__ float half_bits_to_float(uint32_t bits) { return __half2float(__ushort_as_half((unsigned short)bits)); }
+
+template <typename T, int N>
+struct HeadVec;
+template <>
+struct HeadVec<float, 1> {
+  float q;
+  __device__ __forceinline__ void load(const float* s) { q = __ldg(s); }
+  __device__ __forceinline__ float operator[](int) const { return q; }
+};
+template <>
+struct HeadVec<float, 4> {  // 16-byte load: 4-anchor aligned row offset, 16-byte aligned base
+  float q[4];
+  __device__ __forceinline__ void load(const float* s) {
+    const float4 v = __ldg(reinterpret_cast<const float4*>(s));
+    q[0] = v.x, q[1] = v.y, q[2] = v.z, q[3] = v.w;
+  }
+  __device__ __forceinline__ float operator[](int k) const { return q[k]; }
+};
+template <>
+struct HeadVec<__half, 1> {
+  __half q;
+  __device__ __forceinline__ void load(const __half* s) { q = __ldg(s); }
+  __device__ __forceinline__ float operator[](int) const { return __half2float(q); }
+};
+template <>
+struct HeadVec<__half, 4> {  // 8-byte load
+  uint2 q;
+  __device__ __forceinline__ void load(const __half* s) { q = __ldg(reinterpret_cast<const uint2*>(s)); }
+  __device__ __forceinline__ float operator[](int k) const {
+    const uint32_t w = k < 2 ? q.x : q.y;
+    return half_bits_to_float((k & 1) ? w >> 16 : w & 0xffffu);
+  }
+};
+template <>
+struct HeadVec<__half, 8> {  // 16-byte load
+  uint4 q;
+  __device__ __forceinline__ void load(const __half* s) { q = __ldg(reinterpret_cast<const uint4*>(s)); }
+  __device__ __forceinline__ float operator[](int k) const {
+    const uint32_t w = k < 2 ? q.x : k < 4 ? q.y : k < 6 ? q.z : q.w;
+    return half_bits_to_float((k & 1) ? w >> 16 : w & 0xffffu);
+  }
+};
+__device__ __forceinline__ float head_at(const float* s) { return __ldg(s); }
+__device__ __forceinline__ float head_at(const __half* s) { return __half2float(__ldg(s)); }
+
 // channel-major head [B, C, A].  A thread owns VEC consecutive anchors (one 16-byte load per channel
-// row when VEC = 4) and walks the class rows in order; the next eight rows are already in flight
+// row when VEC * sizeof(T) = 16) and walks the class rows in order; the next eight rows are already in flight
 // while the current eight are scored (software double buffering), so ~16 independent 16-byte loads
 // per thread keep HBM busy.
-template <int VEC>
-__global__ void __launch_bounds__(64) k_decode_cm(const __grid_constant__ PostParams p, int frame0) {
+template <typename T, int VEC>
+__device__ __forceinline__ void decode_cm(const PostParams& p, int frame0) {
   griddep_launch_dependents();  // the NMS kernel may start its prologue now; its griddep_wait() still waits for this grid
   TIMELINE_BEGIN(p.dbg, 40);
   const int frame = blockIdx.y;
   if (p.skip && p.skip[frame0 + frame]) return;
   const int lane = threadIdx.x & 31;
   const int a0 = (blockIdx.x * blockDim.x + threadIdx.x) * VEC;
-  const float* __restrict__ hd = p.head + (size_t)(frame0 + frame) * p.C * p.A;
+  const T* __restrict__ hd = static_cast<const T*>(p.head) + (size_t)(frame0 + frame) * p.C * p.A;
   const int A = p.A, C = p.C;
   float best[VEC];
   int cls[VEC];
@@ -160,18 +213,14 @@ __global__ void __launch_bounds__(64) k_decode_cm(const __grid_constant__ PostPa
     best[k] = 0.f;
     cls[k] = 0;
   }
-  auto load = [&](int c, float (&v)[VEC]) {
-    if (VEC == 4) {
-      const float4 q = __ldg(reinterpret_cast<const float4*>(hd + (size_t)c * A + a0));
-      v[0] = q.x, v[1 % VEC] = q.y, v[2 % VEC] = q.z, v[3 % VEC] = q.w;
-    } else {
-      v[0] = __ldg(hd + (size_t)c * A + a0);
-    }
-  };
+  auto load = [&](int c, HeadVec<T, VEC>& v) { v.load(hd + (size_t)c * A + a0); };
   if (a0 < A) {
     float obj[VEC];
     if (p.use_obj) {
-      load(4, obj);
+      HeadVec<T, VEC> o;
+      load(4, o);
+#pragma unroll
+      for (int k = 0; k < VEC; ++k) obj[k] = o[k];
     } else {
 #pragma unroll
       for (int k = 0; k < VEC; ++k) obj[k] = 1.0f;  // x * 1.0f is exact: scores = pred[:, 4:]
@@ -179,9 +228,9 @@ __global__ void __launch_bounds__(64) k_decode_cm(const __grid_constant__ PostPa
     const int cls0 = p.cls0;
     {
       // REF_COMPAT: scores = class_probs * objectness for both model types (detector.py:294-305)
-      float first[VEC];
+      HeadVec<T, VEC> first;
       load(cls0, first);
-      float cur[8][VEC], nxt[8][VEC];
+      HeadVec<T, VEC> cur[8], nxt[8];
       int c = cls0 + 1;
       const bool have0 = c + 8 <= C;
       if (have0) {
@@ -213,13 +262,11 @@ __global__ void __launch_bounds__(64) k_decode_cm(const __grid_constant__ PostPa
         c += 8;
         if (more) {
 #pragma unroll
-          for (int u = 0; u < 8; ++u)
-#pragma unroll
-            for (int k = 0; k < VEC; ++k) cur[u][k] = nxt[u][k];
+          for (int u = 0; u < 8; ++u) cur[u] = nxt[u];
         }
       }
       for (; c < C; ++c) {
-        float v[VEC];
+        HeadVec<T, VEC> v;
         load(c, v);
 #pragma unroll
         for (int k = 0; k < VEC; ++k) {
@@ -255,7 +302,7 @@ __global__ void __launch_bounds__(64) k_decode_cm(const __grid_constant__ PostPa
   base = __shfl_sync(0xffffffffu, base, 31);
   int pos = base + incl - mine;
   if (pass) {
-    float cx[VEC], cy[VEC], w[VEC], h[VEC];
+    HeadVec<T, VEC> cx, cy, w, h;
     load(0, cx);
     load(1, cy);
     load(2, w);
@@ -269,6 +316,15 @@ __global__ void __launch_bounds__(64) k_decode_cm(const __grid_constant__ PostPa
   }
   TIMELINE_END(p.dbg, 40);
 }
+template <int VEC>
+__global__ void __launch_bounds__(64) k_decode_cm(const __grid_constant__ PostParams p, int frame0) {
+  decode_cm<float, VEC>(p, frame0);
+}
+// float16 head: VEC = 8 (16-byte loads; A % 8 == 0, 16-byte aligned base) or 1
+template <int VEC>
+__global__ void __launch_bounds__(64) k_decode16_cm(const __grid_constant__ PostParams p, int frame0) {
+  decode_cm<__half, VEC>(p, frame0);
+}
 
 // channel-major head, class rows split over the warps of a CTA -- the SMALL-BATCH variant.  k_decode_cm walks its
 // 80-odd rows in ~10 dependent rounds of loads; with a few frames per launch (4 streams per GPU when 32 streams are
@@ -277,8 +333,9 @@ __global__ void __launch_bounds__(64) k_decode_cm(const __grid_constant__ PostPa
 // (a warp still reads 512 contiguous bytes per row), the partial (best, class) pairs meet in shared memory and warp 0
 // merges them in class order -- `>` keeps the first maximum, exactly np.argmax -- then compacts and emits as before.
 // At 32 frames per launch the kernel is HBM-bound and this variant is slower (22 us against 20 us): the host picks.
-template <int kSplitParts, int kSplitRows>  // kSplitRows: rows one warp holds in flight (<= kSplitParts * kSplitRows class rows)
-__global__ void __launch_bounds__(32 * kSplitParts) k_decode_cm_split(const __grid_constant__ PostParams p, int frame0) {
+// The float16 variant keeps four anchors per lane (8-byte loads: A % 4 == 0, 8-byte aligned base).
+template <typename T, int kSplitParts, int kSplitRows>  // kSplitRows: rows one warp holds in flight (<= kSplitParts * kSplitRows class rows)
+__device__ __forceinline__ void decode_cm_split(const PostParams& p, int frame0) {
   griddep_launch_dependents();  // the NMS kernel may start its prologue now; its griddep_wait() still waits for this grid
   __shared__ float s_best[kSplitParts - 1][4][32];
   __shared__ int s_cls[kSplitParts - 1][4][32];
@@ -289,7 +346,7 @@ __global__ void __launch_bounds__(32 * kSplitParts) k_decode_cm_split(const __gr
   const int lane = threadIdx.x & 31, part = threadIdx.x >> 5;
   const int a0 = (blockIdx.x * 32 + lane) * 4;
   const int A = p.A, C = p.C, cls0 = p.cls0;
-  const float* __restrict__ hd = p.head + (size_t)(frame0 + frame) * C * A;
+  const T* __restrict__ hd = static_cast<const T*>(p.head) + (size_t)(frame0 + frame) * C * A;
   const int per = (C - cls0 + kSplitParts - 1) / kSplitParts;
   const int c_lo = cls0 + part * per, c_hi = min(C, c_lo + per);
   const bool in_range = a0 < A;
@@ -299,26 +356,31 @@ __global__ void __launch_bounds__(32 * kSplitParts) k_decode_cm_split(const __gr
   bool any = false;
   // the warp that emits (part 0) fetches the four box rows together with its class rows: one round of loads per launch
   // instead of a second, dependent one for the anchors that pass (a launch of a few frames is latency-bound)
-  float4 cx = make_float4(0.f, 0.f, 0.f, 0.f), cy = cx, w = cx, hh = cx;
+  HeadVec<T, 4> cx{}, cy{}, w{}, hh{};
   if (part == 0 && in_range) {
-    cx = __ldg(reinterpret_cast<const float4*>(hd + a0));
-    cy = __ldg(reinterpret_cast<const float4*>(hd + (size_t)A + a0));
-    w = __ldg(reinterpret_cast<const float4*>(hd + (size_t)2 * A + a0));
-    hh = __ldg(reinterpret_cast<const float4*>(hd + (size_t)3 * A + a0));
+    cx.load(hd + a0);
+    cy.load(hd + (size_t)A + a0);
+    w.load(hd + (size_t)2 * A + a0);
+    hh.load(hd + (size_t)3 * A + a0);
   }
   if (in_range && c_lo < c_hi) {
     any = true;
-    float4 obj = make_float4(1.f, 1.f, 1.f, 1.f);  // x * 1.0f is exact: scores = pred[:, 4:]
-    if (p.use_obj) obj = __ldg(reinterpret_cast<const float4*>(hd + (size_t)4 * A + a0));
-    float4 v[kSplitRows];
+    float obj[4] = {1.f, 1.f, 1.f, 1.f};  // x * 1.0f is exact: scores = pred[:, 4:]
+    if (p.use_obj) {
+      HeadVec<T, 4> o;
+      o.load(hd + (size_t)4 * A + a0);
+#pragma unroll
+      for (int k = 0; k < 4; ++k) obj[k] = o[k];
+    }
+    HeadVec<T, 4> v[kSplitRows];
 #pragma unroll
     for (int u = 0; u < kSplitRows; ++u)
-      if (c_lo + u < c_hi) v[u] = __ldg(reinterpret_cast<const float4*>(hd + (size_t)(c_lo + u) * A + a0));
+      if (c_lo + u < c_hi) v[u].load(hd + (size_t)(c_lo + u) * A + a0);
 #pragma unroll
     for (int u = 0; u < kSplitRows; ++u)
       if (c_lo + u < c_hi) {
-        const float sc[4] = {__fmul_rn(v[u].x, obj.x), __fmul_rn(v[u].y, obj.y), __fmul_rn(v[u].z, obj.z),
-                             __fmul_rn(v[u].w, obj.w)};
+        const float sc[4] = {__fmul_rn(v[u][0], obj[0]), __fmul_rn(v[u][1], obj[1]), __fmul_rn(v[u][2], obj[2]),
+                             __fmul_rn(v[u][3], obj[3])};
 #pragma unroll
         for (int k = 0; k < 4; ++k) {
           nan_seen |= (unsigned)(sc[k] != sc[k]) << k;
@@ -374,16 +436,20 @@ __global__ void __launch_bounds__(32 * kSplitParts) k_decode_cm_split(const __gr
   base = __shfl_sync(0xffffffffu, base, 31);
   int pos = base + incl - mine;
   if (pass) {
-    const float cxa[4] = {cx.x, cx.y, cx.z, cx.w}, cya[4] = {cy.x, cy.y, cy.z, cy.w};
-    const float wa[4] = {w.x, w.y, w.z, w.w}, ha[4] = {hh.x, hh.y, hh.z, hh.w};
 #pragma unroll
     for (int k = 0; k < 4; ++k)
       if (pass & (1u << k)) {
-        emit_candidate(p, frame, pos, a0 + k, best[k], cls[k],
-                       decode_box(cxa[k], cya[k], wa[k], ha[k], p.f[frame], p.ultra != 0));
+        emit_candidate(p, frame, pos, a0 + k, best[k], cls[k], decode_box(cx[k], cy[k], w[k], hh[k], p.f[frame], p.ultra != 0));
         ++pos;
       }
   }
+}
+template <int kSplitParts, int kSplitRows>
+__global__ void __launch_bounds__(32 * kSplitParts) k_decode_cm_split(const __grid_constant__ PostParams p, int frame0) {
+  decode_cm_split<float, kSplitParts, kSplitRows>(p, frame0);
+}
+__global__ void __launch_bounds__(256) k_decode16_cm_split(const __grid_constant__ PostParams p, int frame0) {
+  decode_cm_split<__half, 8, 12>(p, frame0);
 }
 
 // channel-major head, TMA-fed and persistent -- the LARGE-BATCH variant.  k_decode_cm is a one-wave kernel whose CTAs
@@ -571,7 +637,7 @@ __global__ void __launch_bounds__(32 * (kRingWarps + 1)) k_decode_ring(const __g
     // +0.0 of a -0.0 / +0.0 pair, np.argmax sees them equal and reports the first
     int cls[4] = {0, 0, 0, 0};
     if (active) {
-      const float* hd = p.head + (size_t)(frame0 + frame) * C * A + a_tile + 4 * g;
+      const float* hd = static_cast<const float*>(p.head) + (size_t)(frame0 + frame) * C * A + a_tile + 4 * g;
       const float oa[4] = {obj.x, obj.y, obj.z, obj.w};
 #pragma unroll
       for (int k = 0; k < 4; ++k) {
@@ -592,7 +658,8 @@ __global__ void __launch_bounds__(32 * (kRingWarps + 1)) k_decode_ring(const __g
 }
 
 // anchor-major head [B, A, C]: a warp owns one anchor and strides its lanes over the channels
-__global__ void __launch_bounds__(256) k_decode_am(const __grid_constant__ PostParams p, int frame0) {
+template <typename T>
+__device__ __forceinline__ void decode_am(const PostParams& p, int frame0) {
   griddep_launch_dependents();  // the NMS kernel may start its prologue now; its griddep_wait() still waits for this grid
   const int frame = blockIdx.y;
   if (p.skip && p.skip[frame0 + frame]) return;
@@ -600,14 +667,14 @@ __global__ void __launch_bounds__(256) k_decode_am(const __grid_constant__ PostP
   const int a = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
   if (a >= p.A) return;
   const int C = p.C;
-  const float* __restrict__ row = p.head + ((size_t)(frame0 + frame) * p.A + a) * C;
-  const float obj = p.use_obj ? __ldg(row + 4) : 1.0f;
+  const T* __restrict__ row = static_cast<const T*>(p.head) + ((size_t)(frame0 + frame) * p.A + a) * C;
+  const float obj = p.use_obj ? head_at(row + 4) : 1.0f;
   const int cls0 = p.cls0;
   float best = -INFINITY;
   int cls = 0x7fffffff;
   bool have = false, bad = false;
   for (int c = cls0 + lane; c < C; c += 32) {
-    const float s = __fmul_rn(__ldg(row + c), obj);
+    const float s = __fmul_rn(head_at(row + c), obj);
     bad |= (s != s);
     if (!have || s > best) {
       best = s;
@@ -632,10 +699,12 @@ __global__ void __launch_bounds__(256) k_decode_am(const __grid_constant__ PostP
     if ((p.ultra ? best > p.conf_thr : best >= p.conf_thr) && class_allowed(p, cls)) {
       const int pos = atomicAdd(p.cand_count + frame, 1);
       emit_candidate(p, frame, pos, a, best, cls,
-                     decode_box(__ldg(row), __ldg(row + 1), __ldg(row + 2), __ldg(row + 3), p.f[frame], p.ultra != 0));
+                     decode_box(head_at(row), head_at(row + 1), head_at(row + 2), head_at(row + 3), p.f[frame], p.ultra != 0));
     }
   }
 }
+__global__ void __launch_bounds__(256) k_decode_am(const __grid_constant__ PostParams p, int frame0) { decode_am<float>(p, frame0); }
+__global__ void __launch_bounds__(256) k_decode16_am(const __grid_constant__ PostParams p, int frame0) { decode_am<__half>(p, frame0); }
 
 // ---- sort + NMS + emit ----------------------------------------------------------------------
 
@@ -2096,6 +2165,10 @@ int postprocess_configure(b200va_ctx* h) {
     CUDA_TRY(h, prefer_max_shared(k_decode_cm_split<8, 12>));
     CUDA_TRY(h, prefer_max_shared(k_decode_am));
     CUDA_TRY(h, prefer_max_shared(k_decode_ring));
+    CUDA_TRY(h, prefer_max_shared(k_decode16_cm<8>));
+    CUDA_TRY(h, prefer_max_shared(k_decode16_cm<1>));
+    CUDA_TRY(h, prefer_max_shared(k_decode16_cm_split));
+    CUDA_TRY(h, prefer_max_shared(k_decode16_am));
     CUDA_TRY(h, prefer_max_shared(k_sort_nms<false>));
     CUDA_TRY(h, prefer_max_shared(k_sort_nms<true>));
     CUDA_TRY(h, prefer_max_shared(k_post_track<false>));
@@ -2179,7 +2252,7 @@ struct UltraOpts {  // b200va_postprocess_ultralytics
 };
 }  // namespace
 
-static int postprocess_impl(b200va_handle h, const float* head, int layout, int batch, int channels, int anchors,
+static int postprocess_impl(b200va_handle h, const void* head, int layout, int batch, int channels, int anchors,
                                   const b200va_letterbox* meta, double conf_thr, double iou_thr,
                                   const int32_t* classes, int n_classes, int score_mode, int nms_mode,
                                   double filter_conf_thr_f64, int use_filter, const b200va_dets* out, void* stream,
@@ -2194,7 +2267,10 @@ static int postprocess_impl(b200va_handle h, const float* head, int layout, int 
     REQUIRE(h, ultra->max_det >= 1, "max_det must be positive");
   }
   REQUIRE(h, batch >= 0 && batch <= h->cfg.max_batch, "batch %d outside [0, %d]", batch, h->cfg.max_batch);
-  REQUIRE(h, layout == B200VA_HEAD_CHANNEL_MAJOR || layout == B200VA_HEAD_ANCHOR_MAJOR, "unknown layout %d", layout);
+  const bool f16 = (layout & B200VA_HEAD_F16) != 0;
+  const int order = layout & ~B200VA_HEAD_F16;
+  REQUIRE(h, order == B200VA_HEAD_CHANNEL_MAJOR || order == B200VA_HEAD_ANCHOR_MAJOR, "unknown layout %d", layout);
+  layout = order;
   REQUIRE(h, score_mode == B200VA_SCORE_REF_COMPAT || score_mode == B200VA_SCORE_V8_NATIVE, "unknown score mode %d", score_mode);
   REQUIRE(h, nms_mode == B200VA_NMS_AGNOSTIC || nms_mode == B200VA_NMS_CLASS_AWARE, "unknown nms mode %d", nms_mode);
   REQUIRE(h, nms_mode == B200VA_NMS_AGNOSTIC || channels - 4 <= 65535, "class-aware NMS supports at most 65535 classes");
@@ -2264,7 +2340,24 @@ static int postprocess_impl(b200va_handle h, const float* head, int layout, int 
     p.skip = h->skip_dev;
     {
     PhaseScope phase(h, B200VA_PHASE_DECODE, st);
-    if (layout == B200VA_HEAD_CHANNEL_MAJOR) {
+    const int impl = h->tune.decode_impl;  // 0 auto, 1 registers (k_decode_cm), 2 ring, 3 split
+    if (f16) {
+      // the float16 kernels: the same selection with 16-byte loads of 8 anchors, the split variant with 8-byte loads of
+      // 4, and no ring (it buys nothing in float32 either, see below)
+      const uintptr_t addr = (uintptr_t)head;
+      const int n_cls_rows = channels - p.cls0;
+      const bool vec8 = anchors % 8 == 0 && addr % 16 == 0;
+      const bool split_ok = anchors % 4 == 0 && addr % 8 == 0 && n_cls_rows >= 16 && n_cls_rows <= 96;
+      if (layout == B200VA_HEAD_ANCHOR_MAJOR) {
+        k_decode16_am<<<dim3((anchors + 7) / 8, n), 256, 0, st>>>(p, base);
+      } else if (split_ok && (impl == 3 || (impl == 0 && n <= 8))) {
+        k_decode16_cm_split<<<dim3((anchors / 4 + 31) / 32, n), 256, 0, st>>>(p, base);
+      } else if (vec8) {
+        k_decode16_cm<8><<<dim3((anchors / 8 + 63) / 64, n), 64, 0, st>>>(p, base);
+      } else {
+        k_decode16_cm<1><<<dim3((anchors + 63) / 64, n), 64, 0, st>>>(p, base);
+      }
+    } else if (layout == B200VA_HEAD_CHANNEL_MAJOR) {
       // 16-byte loads need every channel row (A floats) and the tensor base 16-byte aligned
       // (a TMA-staged variant -- all C rows of a 128-anchor tile bulk-copied to shared memory -- measured
       // 24.6 us against 21.5 us for this register version on [32,84,8400]: the 512-byte row pieces at a
@@ -2272,7 +2365,6 @@ static int postprocess_impl(b200va_handle h, const float* head, int layout, int 
       const int n_cls_rows = channels - p.cls0;
       const bool vec4 = anchors % 4 == 0 && ((uintptr_t)head % 16 == 0);
       // few frames: latency-bound, split the class rows over 8 warps; many frames: HBM-bound, the TMA-fed persistent ring
-      const int impl = h->tune.decode_impl;  // 0 auto, 1 registers (k_decode_cm), 2 ring, 3 split
       const bool split_ok = vec4 && n_cls_rows >= 16 && n_cls_rows <= 96;
       // The ring kernel is opt-in (B200VA_DECODE_IMPL=2): measured on [32, 84, 8400] it is no faster than the register
       // kernel, and neither can be -- a pure 90 MB read of this tensor takes 19.4 us on a B200 whatever fetches it
@@ -2287,7 +2379,7 @@ static int postprocess_impl(b200va_handle h, const float* head, int layout, int 
         ring_plan(h, n, channels, anchors, p.cls0, &rc, &ring_ctas, &ring_smem);
         // the map spans the frames of this launch only (coordinate 2 = frame index inside the launch)
         ring_ok = ring_smem <= (size_t)kRingSmemMax &&
-                  head_tensor_map(head + (size_t)base * channels * anchors, n, channels, anchors, rc.bw, rc.rows, &tmap);
+                  head_tensor_map(static_cast<const float*>(head) + (size_t)base * channels * anchors, n, channels, anchors, rc.bw, rc.rows, &tmap);
       }
       if (split_ok && (impl == 3 || (impl == 0 && n <= 8))) {
         dim3 grid((anchors / 4 + 31) / 32, n);
@@ -2451,7 +2543,7 @@ static int postprocess_impl(b200va_handle h, const float* head, int layout, int 
   return B200VA_OK;
 }
 
-extern "C" int b200va_postprocess(b200va_handle h, const float* head, int layout, int batch, int channels, int anchors,
+extern "C" int b200va_postprocess(b200va_handle h, const void* head, int layout, int batch, int channels, int anchors,
                                   const b200va_letterbox* meta, double conf_thr, double iou_thr,
                                   const int32_t* classes, int n_classes, int score_mode, int nms_mode,
                                   double filter_conf_thr_f64, int use_filter, const b200va_dets* out, void* stream) {
@@ -2459,7 +2551,7 @@ extern "C" int b200va_postprocess(b200va_handle h, const float* head, int layout
                           nms_mode, filter_conf_thr_f64, use_filter, out, stream, nullptr);
 }
 
-extern "C" int b200va_postprocess_ultralytics(b200va_handle h, const float* head, int layout, int batch, int channels,
+extern "C" int b200va_postprocess_ultralytics(b200va_handle h, const void* head, int layout, int batch, int channels,
                                               int anchors, const int* src_h, const int* src_w, int in_h, int in_w,
                                               double conf_thr, double iou_thr, const int32_t* classes, int n_classes,
                                               int agnostic, int max_det, double filter_conf_thr_f64, int use_filter,

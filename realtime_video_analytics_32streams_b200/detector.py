@@ -81,15 +81,17 @@ class B200Detector:
         return self._infer_fn(tensor)
 
     def _as_head(self, predictions):
-        """Normalise whatever ``_infer`` returned to a contiguous CUDA float32 [B, d1, d2]."""
+        """Normalise whatever ``_infer`` returned to a contiguous CUDA [B, d1, d2]: float16 stays float16 (the decode
+        reads it in place, with the results of its float32 widening), every other dtype becomes float32."""
         t = self.h.torch
         if isinstance(predictions, (list, tuple)):
             predictions = predictions[0]  # detector.py:278-279
         if isinstance(predictions, np.ndarray):
-            predictions = t.from_numpy(np.ascontiguousarray(predictions, dtype=np.float32))
+            dtype = np.float16 if predictions.dtype == np.float16 else np.float32  # fp16 crosses PCIe at half the bytes
+            predictions = t.from_numpy(np.ascontiguousarray(predictions, dtype=dtype))
         if not predictions.is_cuda:
             predictions = predictions.to(self.h.device, non_blocking=True)
-        if predictions.dtype != t.float32:
+        if predictions.dtype not in (t.float32, t.float16):
             predictions = predictions.float()
         return predictions.contiguous()
 
