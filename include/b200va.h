@@ -236,6 +236,44 @@ B200VA_API int b200va_resize_linear_u8(b200va_handle h, const uint8_t* const* fr
                             const int64_t* src_pitch, int batch, const uint8_t* const* roi_masks,
                             uint8_t* const* dst, const int* dst_h, const int* dst_w, void* stream);
 
+/* ---- NV12 frames (what video decoders produce) ---------------------------------------------
+ * NVDEC / PyNvVideoCodec / DALI surfaces and FFmpeg's `-pix_fmt nv12` hold a frame as src_h rows of src_w luma bytes
+ * and a separate plane of src_h / 2 rows of src_w bytes, the interleaved Cb, Cr pair of each 2 x 2 pixel block.  Each
+ * plane has its own base and pitch (decoder surfaces keep the chroma plane at pitch * aligned_height).  The entry
+ * points below take such frames directly, with the colour conversion folded into the letterbox / resize taps (no
+ * conversion pass, no BGR frame in memory): every result is BYTE-IDENTICAL to the BGR entry point of the same name
+ * run on cv2.cvtColor(frame, cv2.COLOR_YUV2BGR_NV12) -- OpenCV's BT.601 limited-range fixed point with nearest
+ * chroma:  y' = max(0, Y - 16) * 1220542 + (1 << 19), u = Cb - 128, v = Cr - 128,
+ *          R = sat_u8((y' + 1673527 v) >> 20), G = sat_u8((y' - 852492 v - 409993 u) >> 20), B = sat_u8((y' + 2116026 u) >> 20).
+ * ROI masks are uint8 [src_h, src_w] (luma size); geometry, output formats, flags and the skip mask are those of the
+ * BGR calls.  Odd src_h / src_w and NULL planes are refused with B200VA_ERR_INVALID.  The chroma plane is read at
+ * row y >> 1 for luma row y; only NV12 (not I420, not BT.709, not full range) is accepted. */
+typedef struct b200va_nv12_frame {
+  const uint8_t* y;  /* DEVICE (HOST for the source side of b200va_upload_frames_nv12) luma plane [src_h, y_pitch]   */
+  const uint8_t* uv; /* chroma plane [src_h / 2, uv_pitch]: Cb, Cr byte pairs                                        */
+  int64_t y_pitch;   /* bytes between luma rows   (>= src_w) */
+  int64_t uv_pitch;  /* bytes between chroma rows (>= src_w) */
+} b200va_nv12_frame;
+
+/* b200va_preprocess for NV12 frames.  frames: HOST array [batch] of plane descriptors (DEVICE planes); every other
+ * argument as in b200va_preprocess. */
+B200VA_API int b200va_preprocess_nv12(b200va_handle h, const b200va_nv12_frame* frames, const int* src_h, const int* src_w,
+                                      int batch, const uint8_t* const* roi_masks, void* out, int dst_h, int dst_w,
+                                      int out_format, b200va_letterbox* meta_out, void* stream);
+/* b200va_resize_linear_u8 for NV12 frames: BGR uint8 HWC out (dst pitch = 3 * dst_w).  With dst == src size this is
+ * cv2.cvtColor(frame, COLOR_YUV2BGR_NV12) itself (masked pixels zeroed when a mask is given). */
+B200VA_API int b200va_resize_linear_u8_nv12(b200va_handle h, const b200va_nv12_frame* frames, const int* src_h,
+                                            const int* src_w, int batch, const uint8_t* const* roi_masks,
+                                            uint8_t* const* dst, const int* dst_h, const int* dst_w, void* stream);
+/* b200va_upload_frames for NV12 frames: host[i] (HOST planes, pinned for asynchronous copies) -> dev[i] (DEVICE
+ * planes, written through the const pointers).  rows_mode 0 copies both planes whole; rows_mode 1 copies only the
+ * luma rows b200va_preprocess_nv12 to dst_h x dst_w reads and the chroma rows those use (each once) -- e.g. 1,382,400
+ * bytes of a 1080p frame for 640 x 640 instead of 3,110,400 -- and the device frame is then valid for the letterbox
+ * only.  bytes_copied (HOST, may be NULL) receives the bytes put on the bus. */
+B200VA_API int b200va_upload_frames_nv12(b200va_handle h, const b200va_nv12_frame* host, const b200va_nv12_frame* dev,
+                                         const int* src_h, const int* src_w, int batch, int dst_h, int dst_w, int rows_mode,
+                                         int64_t* bytes_copied, void* stream);
+
 /* ---- a9: ROI polygons ----------------------------------------------------------------
  * Replaces the mask construction of utils.apply_roi (frame_filter.py:46-49): one cv2.fillPoly
  * per polygon (LINE_8, shift 0), union.  pts HOST [sum(poly_sizes), 2] int32 (x, y);
@@ -476,6 +514,10 @@ typedef struct b200va_tick_args {
   void* ev_pre_end;
 } b200va_tick_args;
 B200VA_API int b200va_tick(b200va_handle h, const b200va_tick_args* args, void* stream);
+/* b200va_tick with the letterbox reading NV12 frames (b200va_preprocess_nv12): frames HOST [args->batch] plane
+ * descriptors; args->frames and args->src_pitch are not read.  Every schedule, graph capture included; the results
+ * are those of b200va_tick on the frames converted by cv2.cvtColor(frame, COLOR_YUV2BGR_NV12). */
+B200VA_API int b200va_tick_nv12(b200va_handle h, const b200va_tick_args* args, const b200va_nv12_frame* frames, void* stream);
 
 /* ---- 8f-3: egress (the preview and the event the sink publishes) -------------------------------
  * Replaces, for a frame that is already in HBM, the pixel work of KafkaSink._render_frame

@@ -79,6 +79,12 @@ class RectOp(C.Structure):
                 ("b", C.c_uint8), ("g", C.c_uint8), ("r", C.c_uint8), ("pad_", C.c_uint8)]
 
 
+class Nv12Frame(C.Structure):
+    """``b200va_nv12_frame`` (include/b200va.h): the two planes of an NV12 frame, each with its own pitch."""
+
+    _fields_ = [("y", C.c_void_p), ("uv", C.c_void_p), ("y_pitch", C.c_int64), ("uv_pitch", C.c_int64)]
+
+
 class TickArgs(C.Structure):
     """``b200va_tick_args`` (include/b200va.h)."""
 
@@ -111,6 +117,7 @@ class TickPlan:
     def __init__(self, args: "TickArgs", keep: tuple):
         self.args = args
         self._keep = keep  # owners of every pointer inside `args`
+        self.nv12 = None   # Nv12Frame array: the letterbox reads NV12 frames (b200va_tick_nv12)
 
     def set_events(self, begin=None, end=None) -> None:
         """Optional (already recorded once) ``torch.cuda.Event`` pair around the letterbox launch."""
@@ -128,6 +135,7 @@ EXPORTS = (
     "b200va_motion_preprocess", "b200va_set_profiling", "b200va_get_phase_times",
     "b200va_read_status_async", "b200va_resize_area_u8", "b200va_draw_rects", "b200va_tracks_json",
     "b200va_gates_decide", "b200va_gates_commit", "b200va_gates_reset", "b200va_set_skip_mask",
+    "b200va_preprocess_nv12", "b200va_resize_linear_u8_nv12", "b200va_upload_frames_nv12", "b200va_tick_nv12",
 )
 PHASES = ("upload", "roi", "resize", "motion", "preprocess", "decode", "nms", "tracker", "dfl", "tick", "egress")  # enum b200va_phase
 
@@ -195,6 +203,12 @@ def load_library() -> C.CDLL:
     lib.b200va_gates_commit.argtypes = [vp, C.POINTER(Gate), C.c_int, vp, vp, vp, vp, vp]
     lib.b200va_gates_reset.argtypes = [vp, C.c_int, vp]
     lib.b200va_set_skip_mask.argtypes = [vp, vp]
+    nv = C.POINTER(Nv12Frame)
+    lib.b200va_preprocess_nv12.argtypes = [vp, nv, ip, ip, C.c_int, C.POINTER(vp), vp, C.c_int, C.c_int, C.c_int,
+                                           C.POINTER(Letterbox), vp]
+    lib.b200va_resize_linear_u8_nv12.argtypes = [vp, nv, ip, ip, C.c_int, C.POINTER(vp), C.POINTER(vp), ip, ip, vp]
+    lib.b200va_upload_frames_nv12.argtypes = [vp, nv, nv, ip, ip, C.c_int, C.c_int, C.c_int, C.c_int, i64p, vp]
+    lib.b200va_tick_nv12.argtypes = [vp, C.POINTER(TickArgs), nv, vp]
     lib.b200va_tracks_json.restype = C.c_int64
     lib.b200va_tracks_json.argtypes = [C.c_char_p, C.c_int64, vp, vp, vp, vp, C.c_int, C.c_char_p, vp, C.c_int64]
     for name in EXPORTS:
@@ -284,6 +298,61 @@ class FrameBatch:
                 if m is not None and not (m.is_cuda and m.dtype == t.uint8 and m.is_contiguous()
                                           and tuple(m.shape) == tuple(f.shape[:2])):
                     raise ValueError("roi masks must be contiguous CUDA uint8 tensors [H, W] matching their frame")
+            self.mask_ptrs = _ptr_array([m.data_ptr() if m is not None else None for m in self.masks])
+        self.metas = (Letterbox * max(n, 1))()
+
+    def __len__(self):
+        return self.n
+
+
+def is_nv12(frame) -> bool:
+    """True for an NV12 frame: a ``(y, uv)`` pair or a 2-D ``[3H/2, W]`` array / tensor (BGR frames are ``[H, W, 3]``)."""
+    return isinstance(frame, (tuple, list)) or getattr(frame, "ndim", 3) == 2
+
+
+def nv12_planes(frame):
+    """``(y [H, W], uv [H/2, W])`` of an NV12 frame given as one ``[3H/2, W]`` tensor (OpenCV's layout; any row pitch)
+    or as a ``(y, uv)`` pair (decoder surfaces: separate bases and pitches).  The planes are views, not copies."""
+    if isinstance(frame, (tuple, list)):
+        if len(frame) != 2:
+            raise ValueError("an NV12 plane pair is (y, uv)")
+        y, uv = frame
+    else:
+        if frame.dim() != 2 or frame.shape[0] % 3:
+            raise ValueError("an NV12 frame is a [3H/2, W] uint8 tensor")
+        h = frame.shape[0] * 2 // 3
+        y, uv = frame[:h], frame[h:]
+    return y, uv
+
+
+class Nv12Batch:
+    """``FrameBatch`` for NV12 frames: CUDA uint8 ``[3H/2, W]`` tensors (any ``stride(0)``, ``stride(1) == 1``) or
+    ``(y [H, W], uv [H/2, W])`` pairs of CUDA uint8 tensors; H and W even.  ROI masks are ``[H, W]`` (luma size)."""
+
+    def __init__(self, frames, roi_masks=None):
+        import torch as t
+
+        self.frames = list(frames)
+        self.planes = [nv12_planes(f) for f in self.frames]
+        for y, uv in self.planes:
+            if not all(p.is_cuda and p.dtype == t.uint8 and p.dim() == 2 and p.stride(1) == 1 for p in (y, uv)):
+                raise ValueError("NV12 planes must be CUDA uint8 tensors [H, W] / [H/2, W] with unit column stride")
+            if y.shape[0] % 2 or y.shape[1] % 2 or tuple(uv.shape) != (y.shape[0] // 2, y.shape[1]):
+                raise ValueError(f"NV12 needs an even size and a [H/2, W] chroma plane, got y {tuple(y.shape)}, "
+                                 f"uv {tuple(uv.shape)}")
+        n = len(self.frames)
+        self.n = n
+        self.nv = (Nv12Frame * max(n, 1))(*[Nv12Frame(y.data_ptr(), uv.data_ptr(), y.stride(0), uv.stride(0))
+                                             for y, uv in self.planes])
+        self.hs = _int_array([y.shape[0] for y, _ in self.planes])
+        self.ws = _int_array([y.shape[1] for y, _ in self.planes])
+        self.masks = list(roi_masks) if roi_masks is not None else None
+        self.mask_ptrs = None
+        if self.masks is not None and any(m is not None for m in self.masks):
+            for m, (y, _) in zip(self.masks, self.planes):
+                if m is not None and not (m.is_cuda and m.dtype == t.uint8 and m.is_contiguous()
+                                          and tuple(m.shape) == tuple(y.shape)):
+                    raise ValueError("roi masks must be contiguous CUDA uint8 tensors [H, W] matching their frame's luma")
             self.mask_ptrs = _ptr_array([m.data_ptr() if m is not None else None for m in self.masks])
         self.metas = (Letterbox * max(n, 1))()
 
@@ -384,8 +453,19 @@ class Handle:
         return {name: float(ms[i]) for i, name in enumerate(PHASES) if ms[i] >= 0.0}
 
     @staticmethod
-    def _batch(frames, roi_masks=None) -> FrameBatch:
-        return frames if isinstance(frames, FrameBatch) else FrameBatch(frames, roi_masks)
+    def _batch(frames, roi_masks=None, nv12_ok: bool = False):
+        """A ``FrameBatch``, or with ``nv12_ok`` an ``Nv12Batch`` for an ``Nv12Batch`` / a list of NV12 frames."""
+        if isinstance(frames, FrameBatch):
+            return frames
+        if not isinstance(frames, Nv12Batch):
+            frames = list(frames)
+            if not (frames and all(is_nv12(f) for f in frames)):
+                return FrameBatch(frames, roi_masks)
+            frames = Nv12Batch(frames, roi_masks) if nv12_ok else frames
+        if not nv12_ok:
+            raise ValueError("NV12 frames are taken by preprocess, resize and plan_tick; convert them with "
+                             "resize at their own size for the other calls")
+        return frames
 
     # -- staging ----------------------------------------------------------------------------
     def upload_frames(self, host_ptrs, dev_frames, sparse_for=None) -> int:
@@ -405,12 +485,29 @@ class Handle:
             1 if sparse_for else 0, C.byref(moved), self._stream()))
         return int(moved.value)
 
+    def upload_frames_nv12(self, host_frames, dev_frames, sparse_for=None) -> int:
+        """``upload_frames`` for NV12: ``host_frames[i]`` = ``Nv12Frame`` (host plane addresses and pitches; pinned for
+        a truly asynchronous copy), ``dev_frames`` the CUDA NV12 destinations (``[3H/2, W]`` tensors or ``(y, uv)``
+        pairs).  ``sparse_for=(dst_h, dst_w)`` copies only the luma rows the letterbox to that size reads and the
+        chroma rows they use.  Returns the bytes put on the bus."""
+        n = len(dev_frames)
+        if n == 0:
+            return 0
+        db = Nv12Batch(dev_frames)
+        hb = (Nv12Frame * n)(*host_frames)
+        moved = C.c_int64(0)
+        self._check(self.lib.b200va_upload_frames_nv12(
+            self._h, hb, db.nv, db.hs, db.ws, n, int(sparse_for[0]) if sparse_for else 0,
+            int(sparse_for[1]) if sparse_for else 0, 1 if sparse_for else 0, C.byref(moved), self._stream()))
+        return int(moved.value)
+
     # -- a1 ---------------------------------------------------------------------------------
     def preprocess(self, frames, dst_hw=(640, 640), fmt: int = OUT_F32_RGB_NCHW, roi_masks=None, out=None):
-        """Batched letterbox.  ``frames``: list of CUDA tensors or a ``FrameBatch``.
+        """Batched letterbox.  ``frames``: list of CUDA tensors or a ``FrameBatch``; NV12 frames (``[3H/2, W]`` tensors
+        or ``(y, uv)`` pairs) or an ``Nv12Batch`` give the result of the BGR call on their ``cv2.cvtColor`` conversion.
         Returns (tensor [B,3,H,W] or [B,H,W,3], list of Letterbox)."""
         t = self.torch
-        fb = self._batch(frames, roi_masks)
+        fb = self._batch(frames, roi_masks, nv12_ok=True)
         b = fb.n
         dh, dw = int(dst_hw[0]), int(dst_hw[1])
         dtype = {OUT_F32_RGB_NCHW: t.float32, OUT_F16_RGB_NCHW: t.float16}.get(fmt & 0xff, t.uint8)
@@ -419,7 +516,10 @@ class Handle:
             out = t.empty(shape, dtype=dtype, device=self.device)
         elif tuple(out.shape) != shape or out.dtype != dtype or not out.is_contiguous():
             raise ValueError("preprocess: `out` has the wrong shape / dtype / layout")
-        if b:
+        if b and isinstance(fb, Nv12Batch):
+            self._check(self.lib.b200va_preprocess_nv12(self._h, fb.nv, fb.hs, fb.ws, b, fb.mask_ptrs,
+                                                        C.c_void_p(out.data_ptr()), dh, dw, fmt, fb.metas, self._stream()))
+        elif b:
             self._check(self.lib.b200va_preprocess(self._h, fb.ptrs, fb.hs, fb.ws, fb.pitch, b, fb.mask_ptrs,
                                                    C.c_void_p(out.data_ptr()), dh, dw, fmt, fb.metas, self._stream()))
         return out, [fb.metas[i] for i in range(b)]
@@ -434,8 +534,12 @@ class Handle:
         elif any(tuple(o.shape) != (int(h), int(w), 3) or o.dtype != t.uint8 or not o.is_contiguous() or not o.is_cuda
                  for o, (h, w) in zip(outs, dst_hw_list)) or len(outs) != len(dst_hw_list):
             raise ValueError("resize: `outs` must be contiguous CUDA uint8 tensors [h, w, 3] matching dst_hw_list")
-        fb = self._batch(frames, roi_masks)
-        if fb.n:
+        fb = self._batch(frames, roi_masks, nv12_ok=True)
+        if fb.n and isinstance(fb, Nv12Batch):  # BGR out: at the frame's own size this is cv2.cvtColor itself
+            self._check(self.lib.b200va_resize_linear_u8_nv12(
+                self._h, fb.nv, fb.hs, fb.ws, fb.n, fb.mask_ptrs, _ptr_array([o.data_ptr() for o in outs]),
+                _int_array([h for h, _ in dst_hw_list]), _int_array([w for _, w in dst_hw_list]), self._stream()))
+        elif fb.n:
             self._check(self.lib.b200va_resize_linear_u8(
                 self._h, fb.ptrs, fb.hs, fb.ws, fb.pitch, fb.n, fb.mask_ptrs,
                 _ptr_array([o.data_ptr() for o in outs]), _int_array([h for h, _ in dst_hw_list]),
@@ -723,13 +827,16 @@ class Handle:
         a = TickArgs()
         keep = []
         if frames is not None:
-            fb = self._batch(frames, roi_masks)
+            fb = self._batch(frames, roi_masks, nv12_ok=True)
             dh, dw = int(dst_hw[0]), int(dst_hw[1])
             dtype = {OUT_F32_RGB_NCHW: t.float32, OUT_F16_RGB_NCHW: t.float16}.get(fmt & 0xff, t.uint8)
             shape = (fb.n, dh, dw, 3) if (fmt & 0xff) == OUT_U8_BGR_NHWC else (fb.n, 3, dh, dw)
             if net_out is None or tuple(net_out.shape) != shape or net_out.dtype != dtype or not net_out.is_contiguous():
                 raise ValueError("plan_tick: `net_out` must be a contiguous tensor of the letterbox output shape / dtype")
-            a.frames, a.src_h, a.src_w, a.src_pitch, a.batch = fb.ptrs, fb.hs, fb.ws, fb.pitch, fb.n
+            if isinstance(fb, Nv12Batch):
+                a.src_h, a.src_w, a.batch = fb.hs, fb.ws, fb.n
+            else:
+                a.frames, a.src_h, a.src_w, a.src_pitch, a.batch = fb.ptrs, fb.hs, fb.ws, fb.pitch, fb.n
             a.roi_masks = fb.mask_ptrs
             a.net_out, a.dst_h, a.dst_w, a.out_format, a.meta_out = net_out.data_ptr(), dh, dw, fmt, fb.metas
             keep += [fb, net_out]
@@ -770,11 +877,16 @@ class Handle:
         a.schedule = int(schedule)
         plan = TickPlan(a, tuple(keep))
         plan.dets, plan.tracks = dets, tracks
+        if frames is not None and isinstance(fb, Nv12Batch):
+            plan.nv12 = fb.nv
         return plan
 
     def tick(self, plan: TickPlan) -> None:
         """Run a prepared tick on the current stream (results land in the plan's buffers)."""
-        self._check(self.lib.b200va_tick(self._h, C.byref(plan.args), self._stream()))
+        if plan.nv12 is not None:
+            self._check(self.lib.b200va_tick_nv12(self._h, C.byref(plan.args), plan.nv12, self._stream()))
+        else:
+            self._check(self.lib.b200va_tick(self._h, C.byref(plan.args), self._stream()))
 
     # -- a12 on the device: gates --------------------------------------------------------------
     def gates_decide(self, gates, changed, skip_out) -> None:

@@ -17,6 +17,7 @@
 
 #include <algorithm>
 #include <cmath>
+#include <type_traits>
 
 #include "common.cuh"
 
@@ -392,6 +393,311 @@ __global__ void __launch_bounds__(kThreads) k_letterbox(const __grid_constant__ 
   TIMELINE_END(p.dbg, 42);
 }
 
+// ---- NV12 sources ---------------------------------------------------------------------------
+// The same letterbox / resize with cv2.cvtColor(frame, COLOR_YUV2BGR_NV12) folded into the taps: each tapped luma row
+// and the CbCr row it uses (row y >> 1 of the interleaved chroma plane; the two luma taps of an output row often share
+// it, and then it is fetched once) are staged by one bulk copy each, and every tap pixel is converted to B, G, R with
+// OpenCV's BT.601 limited-range fixed point and nearest chroma before the unchanged integer interpolation.  Two planes
+// per frame do not fit 64 frames in a 4 KB parameter block: an NV12 launch takes 32.
+struct Nv12Frame {
+  const uint8_t* y;
+  const uint8_t* uv;    // src_h / 2 rows of src_w bytes: Cb, Cr of each 2 x 2 block
+  const uint8_t* mask;  // optional ROI mask [src_h, src_w], 0 = outside
+  void* out;            // b200va_resize_linear_u8_nv12: this frame's own destination buffer
+  long long y_pitch, uv_pitch;
+  int src_h, src_w;
+  int xtab, ytab;
+  int bulk_ok;
+  int out_idx;
+};
+
+constexpr int kNv12LaunchFrames = 32;
+struct PreParamsNv12 {
+  Nv12Frame f[kNv12LaunchFrames];
+  const int4* tabs;
+  void* out;
+  int dst_h, dst_w, fmt, rows_per_cta;
+  int row_stride, mask_stride, stages, vec_ok;
+  int rows_per_stage;
+  int keep_pad_rows;
+  long long* dbg;
+  const uint8_t* skip;
+  int pdl_wait;
+};
+static_assert(sizeof(PreParamsNv12) <= 4000, "kernel parameter block too large");
+
+// cv::cvtColor YUV2BGR_NV12 (modules/imgproc/src/color_yuv.simd.hpp, 8-bit path): ITU-R BT.601 limited range in
+// 20-bit fixed point, rounded by the 1 << 19 bias and saturated.  `uv` = Cb | Cr << 8 of the pixel's 2 x 2 block.
+// Returns the pixel packed as B | G << 8 | R << 16 (byte 3 is zero).
+__device__ __forceinline__ uint32_t nv12_bgr(int Y, uint32_t uv) {
+  const int y = max(Y - 16, 0) * 1220542 + (1 << 19);
+  const int u = (int)(uv & 0xffu) - 128, v = (int)(uv >> 8) - 128;
+  const uint32_t b = (uint32_t)min(max((y + 2116026 * u) >> 20, 0), 255);
+  const uint32_t g = (uint32_t)min(max((y - 852492 * v - 409993 * u) >> 20, 0), 255);
+  const uint32_t r = (uint32_t)min(max((y + 1673527 * v) >> 20, 0), 255);
+  return b | (g << 8) | (r << 16);
+}
+
+// pixel x of a staged luma row and its chroma row (chroma rows start 128-byte aligned: the pair load is aligned)
+__device__ __forceinline__ uint32_t nv12_tap(const uint8_t* __restrict__ yr, const uint8_t* __restrict__ cr, int x) {
+  return nv12_bgr(yr[x], *reinterpret_cast<const uint16_t*>(cr + (x & ~1)));
+}
+
+// byte c of p and byte c of q in bytes 0 / 1, zeros above (byte 3 of a packed pixel is zero)
+__device__ __forceinline__ uint32_t pair_c(uint32_t p, uint32_t q, int c) {
+  return __byte_perm(p, q, (uint32_t)c | ((uint32_t)(4 + c) << 4) | 0x3300u);
+}
+
+// one tapped row: per channel a0 * p + a1 * q with one IDP.2A, as in taps_row
+__device__ __forceinline__ void nv12_taps_row(const uint8_t* __restrict__ yr, const uint8_t* __restrict__ cr, int i0, int i1,
+                                              uint32_t coef, int (&s)[3]) {
+  const uint32_t p = nv12_tap(yr, cr, i0), q = nv12_tap(yr, cr, i1);
+#pragma unroll
+  for (int c = 0; c < 3; ++c) s[c] = (int)__dp2a_lo(coef, pair_c(p, q, c), 0u);
+}
+
+template <bool MASK>
+__device__ __forceinline__ void nv12_px4_general(const TapX (&t)[4], const uint8_t* __restrict__ y0, const uint8_t* __restrict__ c0r,
+                                                 const uint8_t* __restrict__ y1, const uint8_t* __restrict__ c1r,
+                                                 const uint8_t* __restrict__ m0, const uint8_t* __restrict__ m1, int b0, int b1,
+                                                 int (&v)[4][3]) {
+#pragma unroll
+  for (int j = 0; j < 4; ++j) {
+    if (t[j].off0 < 0) {
+      v[j][0] = v[j][1] = v[j][2] = 114;  // copyMakeBorder value, detector.py:233-241
+      continue;
+    }
+    const int i0 = t[j].mx0 & 0xffff, i1 = (int)((unsigned)t[j].mx0 >> 16);
+    int s0[3] = {0, 0, 0}, s1[3] = {0, 0, 0};
+    if (b0) {
+      int a0 = t[j].a0, a1 = t[j].a1;
+      if (MASK) {  // apply_roi zeroes masked source pixels before the resize (pipeline.py:149-154)
+        a0 = m0[i0] ? a0 : 0;
+        a1 = m0[i1] ? a1 : 0;
+      }
+      nv12_taps_row(y0, c0r, i0, i1, (uint32_t)a0 | ((uint32_t)a1 << 16), s0);
+    }
+    if (b1) {
+      int a0 = t[j].a0, a1 = t[j].a1;
+      if (MASK) {
+        a0 = m1[i0] ? a0 : 0;
+        a1 = m1[i1] ? a1 : 0;
+      }
+      nv12_taps_row(y1, c1r, i0, i1, (uint32_t)a0 | ((uint32_t)a1 << 16), s1);
+    }
+#pragma unroll
+    for (int c = 0; c < 3; ++c) v[j][c] = (((b0 * (s0[c] >> 4)) >> 16) + ((b1 * (s1[c] >> 4)) >> 16) + 2) >> 2;
+  }
+}
+
+// 2 x 2 box (all four weights 1024): the rounded mean of the four converted pixels, as in px4_box
+__device__ __forceinline__ void nv12_px4_box(const TapX (&t)[4], const uint8_t* __restrict__ y0, const uint8_t* __restrict__ c0r,
+                                             const uint8_t* __restrict__ y1, const uint8_t* __restrict__ c1r, int (&v)[4][3]) {
+#pragma unroll
+  for (int j = 0; j < 4; ++j) {
+    if (t[j].off0 < 0) {
+      v[j][0] = v[j][1] = v[j][2] = 114;
+      continue;
+    }
+    const int x = t[j].mx0 & 0xffff;
+    const uint32_t p00 = nv12_tap(y0, c0r, x), p01 = nv12_tap(y0, c0r, x + 1);
+    const uint32_t p10 = nv12_tap(y1, c1r, x), p11 = nv12_tap(y1, c1r, x + 1);
+#pragma unroll
+    for (int c = 0; c < 3; ++c)
+      v[j][c] = (int)(__dp4a(pair_c(p00, p01, c), 0x0101u, __dp4a(pair_c(p10, p11, c), 0x0101u, 2u)) >> 2);
+  }
+}
+
+// every tap (2048, 0) on both axes: the converted source pixel itself
+template <bool MASK>
+__device__ __forceinline__ void nv12_px4_identity(const TapX (&t)[4], const uint8_t* __restrict__ y0, const uint8_t* __restrict__ c0r,
+                                                  const uint8_t* __restrict__ m0, int (&v)[4][3]) {
+#pragma unroll
+  for (int j = 0; j < 4; ++j) {
+    if (t[j].off0 < 0) {
+      v[j][0] = v[j][1] = v[j][2] = 114;
+      continue;
+    }
+    const int x = t[j].mx0 & 0xffff;
+    const uint32_t p = (!MASK || m0[x]) ? nv12_tap(y0, c0r, x) : 0u;
+#pragma unroll
+    for (int c = 0; c < 3; ++c) v[j][c] = (int)((p >> (8 * c)) & 0xffu);
+  }
+}
+
+// k_letterbox for NV12 frames.  A stage holds rows_per_stage luma rows, then as many chroma rows (row_stride bytes
+// apart); the ROI mask rows follow all stages, as in k_letterbox.
+template <int FMT, bool MASK>
+__global__ void __launch_bounds__(kThreads, 4) k_letterbox_nv12(const __grid_constant__ PreParamsNv12 p) {
+  extern __shared__ __align__(128) uint8_t smem[];
+  __shared__ __align__(8) uint64_t full[kMaxStages];
+  __shared__ TapY s_ty[kMaxRowsPerCta];
+
+  TIMELINE_BEGIN(p.dbg, 42);  // the tick's letterbox slot, whichever source format
+  const int frame = blockIdx.y;
+  const Nv12Frame& f = p.f[frame];
+  if (p.skip && p.skip[f.out_idx]) return;  // gated off on the device: nobody reads this frame's tensor
+  const TapX* __restrict__ xt = reinterpret_cast<const TapX*>(p.tabs + f.xtab);
+  const TapY* __restrict__ yt = reinterpret_cast<const TapY*>(p.tabs + f.ytab);
+  const int S = p.stages;
+  const int row_begin = blockIdx.x * p.rows_per_cta;
+  const int nrows = min(p.rows_per_cta, p.dst_h - row_begin);
+  const bool bulk = f.bulk_ok != 0;
+  const uint32_t chroma_off = (uint32_t)p.rows_per_stage * (uint32_t)p.row_stride;
+  const uint32_t stage_bytes = 2u * chroma_off;
+  const uint32_t mstage_bytes = (uint32_t)p.rows_per_stage * (uint32_t)p.mask_stride;
+  uint8_t* const rows_base = smem;
+  uint8_t* const mask_base = smem + (size_t)S * stage_bytes;
+  const uint32_t w = (uint32_t)f.src_w;  // bytes per luma row and per chroma row
+
+  if (threadIdx.x < nrows) s_ty[threadIdx.x] = yt[row_begin + threadIdx.x];
+  if (bulk && threadIdx.x == 0) {
+    for (int s = 0; s < S; ++s) mbar_init(&full[s], 1);
+    mbar_fence_init();
+  }
+  __syncthreads();
+  if (p.pdl_wait) griddep_wait();
+
+  auto shared_chroma = [](const TapY& ty) { return ty.b0 != 0 && ty.b1 != 0 && (ty.y0 >> 1) == (ty.y1 >> 1); };
+  auto issue = [&](int i, int s) {
+    const TapY ty = s_ty[i];
+    if (ty.y0 < 0) return;
+    const bool cs = shared_chroma(ty);
+    const uint32_t mb = MASK ? w : 0u;
+    mbar_expect_tx(&full[s], (ty.b0 ? 2u * w + mb : 0u) + (ty.b1 ? (cs ? w : 2u * w) + mb : 0u));
+    uint8_t* r0 = rows_base + (size_t)s * stage_bytes;
+    uint8_t* m0 = mask_base + (size_t)s * mstage_bytes;
+    if (ty.b0) {
+      bulk_g2s(r0, f.y + (long long)ty.y0 * f.y_pitch, w, &full[s]);
+      bulk_g2s(r0 + chroma_off, f.uv + (long long)(ty.y0 >> 1) * f.uv_pitch, w, &full[s]);
+      if (MASK) bulk_g2s(m0, f.mask + (size_t)ty.y0 * f.src_w, w, &full[s]);
+    }
+    if (ty.b1) {
+      bulk_g2s(r0 + p.row_stride, f.y + (long long)ty.y1 * f.y_pitch, w, &full[s]);
+      if (!cs) bulk_g2s(r0 + chroma_off + p.row_stride, f.uv + (long long)(ty.y1 >> 1) * f.uv_pitch, w, &full[s]);
+      if (MASK) bulk_g2s(m0 + p.mask_stride, f.mask + (size_t)ty.y1 * f.src_w, w, &full[s]);
+    }
+  };
+
+  int s_issue = 0;
+  if (bulk && threadIdx.x == 0) {
+    for (int i = 0; i < S - 1 && i < nrows; ++i) {
+      issue(i, s_issue);
+      s_issue = s_issue + 1 == S ? 0 : s_issue + 1;
+    }
+  }
+
+  const int ngroups = (p.dst_w + 3) >> 2;
+  const int nthreads = blockDim.x;
+  TapX tx[4];
+  bool ident = true, box = !MASK;
+  {
+    const int g = threadIdx.x;
+#pragma unroll
+    for (int j = 0; j < 4; ++j) {
+      const int x = 4 * g + j;
+      if (g < ngroups && x < p.dst_w) {
+        int4 e = __ldg(reinterpret_cast<const int4*>(xt) + x);
+        tx[j] = *reinterpret_cast<TapX*>(&e);
+      } else {
+        tx[j].off0 = -1;
+        tx[j].off1 = -1;
+        tx[j].a0 = tx[j].a1 = 0;
+        tx[j].mx0 = 0;
+      }
+      ident = ident && (tx[j].off0 < 0 || (tx[j].a0 == 2048 && tx[j].a1 == 0));
+      box = box && (tx[j].off0 < 0 || (tx[j].a0 == 1024 && tx[j].a1 == 1024 && tx[j].off1 == tx[j].off0 + 3));
+    }
+  }
+  const size_t plane = (size_t)p.dst_h * p.dst_w;
+  const size_t esize = FMT == B200VA_OUT_F32_RGB_NCHW ? 4 : (FMT == B200VA_OUT_F16_RGB_NCHW ? 2 : 1);
+  const bool nhwc = FMT == B200VA_OUT_U8_BGR_NHWC;
+  uint8_t* optr = (f.out ? (uint8_t*)f.out : (uint8_t*)p.out + ((size_t)f.out_idx * 3 * plane) * esize) +
+                  (nhwc ? ((size_t)row_begin * p.dst_w + 4 * threadIdx.x) * 3
+                        : ((size_t)row_begin * p.dst_w + 4 * threadIdx.x) * esize);
+  const size_t row_step = nhwc ? (size_t)p.dst_w * 3 : (size_t)p.dst_w * esize;
+  const bool vec_ok = p.vec_ok != 0;
+  const int nvalid0 = min(4, p.dst_w - 4 * (int)threadIdx.x);
+
+  uint32_t phase_bits = 0;
+  int s = 0;
+  for (int i = 0; i < nrows; ++i, optr += row_step) {
+    const TapY ty = s_ty[i];
+    const bool pad_row = ty.y0 < 0;
+    const int sc = bulk ? s : 0;
+    const uint8_t* y0 = rows_base + (size_t)sc * stage_bytes;
+    const uint8_t* y1 = y0 + p.row_stride;
+    const uint8_t* c0 = y0 + chroma_off;
+    const uint8_t* c1 = shared_chroma(ty) ? c0 : c0 + p.row_stride;
+    const uint8_t* m0 = mask_base + (size_t)sc * mstage_bytes;
+    const uint8_t* m1 = m0 + p.mask_stride;
+
+    if (bulk) {
+      if (threadIdx.x == 0 && i + S - 1 < nrows) {
+        issue(i + S - 1, s_issue);
+        s_issue = s_issue + 1 == S ? 0 : s_issue + 1;
+      }
+      if (!pad_row) {
+        mbar_wait(&full[s], (phase_bits >> s) & 1u);
+        phase_bits ^= 1u << s;
+      }
+    } else if (!pad_row) {
+      if (ty.b0) {
+        coop_copy(const_cast<uint8_t*>(y0), f.y + (long long)ty.y0 * f.y_pitch, w);
+        coop_copy(const_cast<uint8_t*>(c0), f.uv + (long long)(ty.y0 >> 1) * f.uv_pitch, w);
+        if (MASK) coop_copy(const_cast<uint8_t*>(m0), f.mask + (size_t)ty.y0 * f.src_w, w);
+      }
+      if (ty.b1) {
+        coop_copy(const_cast<uint8_t*>(y1), f.y + (long long)ty.y1 * f.y_pitch, w);
+        if (c1 != c0) coop_copy(const_cast<uint8_t*>(c1), f.uv + (long long)(ty.y1 >> 1) * f.uv_pitch, w);
+        if (MASK) coop_copy(const_cast<uint8_t*>(m1), f.mask + (size_t)ty.y1 * f.src_w, w);
+      }
+      __syncthreads();
+    }
+
+    const bool skip_row = pad_row && p.keep_pad_rows;
+    if ((int)threadIdx.x < ngroups && !skip_row) {
+      int v[4][3];
+      if (pad_row) {
+#pragma unroll
+        for (int j = 0; j < 4; ++j) v[j][0] = v[j][1] = v[j][2] = 114;
+      } else if (ident && ty.b0 == 2048 && ty.b1 == 0) {
+        nv12_px4_identity<MASK>(tx, y0, c0, m0, v);
+      } else if (box && ty.b0 == 1024 && ty.b1 == 1024) {
+        nv12_px4_box(tx, y0, c0, y1, c1, v);
+      } else {
+        nv12_px4_general<MASK>(tx, y0, c0, y1, c1, m0, m1, ty.b0, ty.b1, v);
+      }
+      store_px4<FMT>(optr, plane, vec_ok, nvalid0, v);
+    }
+    for (int g = threadIdx.x + nthreads; g < ngroups && !skip_row; g += nthreads) {
+      TapX t[4];
+#pragma unroll
+      for (int j = 0; j < 4; ++j) {
+        const int x = 4 * g + j;
+        if (x < p.dst_w) {
+          int4 e = __ldg(reinterpret_cast<const int4*>(xt) + x);
+          t[j] = *reinterpret_cast<TapX*>(&e);
+        } else {
+          t[j].off0 = -1;
+        }
+      }
+      int v[4][3];
+      if (pad_row) {
+#pragma unroll
+        for (int j = 0; j < 4; ++j) v[j][0] = v[j][1] = v[j][2] = 114;
+      } else {
+        nv12_px4_general<MASK>(t, y0, c0, y1, c1, m0, m1, ty.b0, ty.b1, v);
+      }
+      store_px4<FMT>(optr + (size_t)(g - (int)threadIdx.x) * 4 * (nhwc ? 3 : esize), plane, vec_ok,
+                     min(4, p.dst_w - 4 * g), v);
+    }
+    if (!pad_row) __syncthreads();
+    s = s + 1 == S ? 0 : s + 1;
+  }
+  TIMELINE_END(p.dbg, 42);
+}
+
 // ---- host side ---------------------------------------------------------------------------
 
 struct TapKey {
@@ -613,23 +919,32 @@ static cudaError_t launch_one(const PreParams& p, dim3 grid, size_t smem, cudaSt
   return launch_pdl(k_letterbox<FMT, MASK>, grid, dim3(kThreads), smem, st, pdl, p);
 }
 
-template <int FMT>
-static cudaError_t launch_letterbox(const PreParams& p, bool mask, dim3 grid, size_t smem, cudaStream_t st, bool pdl) {
+template <int FMT, bool MASK>
+static cudaError_t launch_one(const PreParamsNv12& p, dim3 grid, size_t smem, cudaStream_t st, bool pdl) {
+  return launch_pdl(k_letterbox_nv12<FMT, MASK>, grid, dim3(kThreads), smem, st, pdl, p);
+}
+
+template <int FMT, typename P>
+static cudaError_t launch_letterbox(const P& p, bool mask, dim3 grid, size_t smem, cudaStream_t st, bool pdl) {
   return mask ? launch_one<FMT, true>(p, grid, smem, st, pdl) : launch_one<FMT, false>(p, grid, smem, st, pdl);
 }
 
 static const int kLetterboxSmemMax = 200 * 1024;
 
+template <typename K>
+static cudaError_t configure_kernel(K kernel, bool uniform_carveout) {
+  cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kLetterboxSmemMax + 128);
+  if (e != cudaSuccess || !uniform_carveout) return e;
+  return prefer_max_shared(kernel);
+}
+
 template <int FMT>
 static cudaError_t configure_fmt(bool uniform_carveout) {
-  cudaError_t e = cudaFuncSetAttribute(k_letterbox<FMT, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kLetterboxSmemMax + 128);
-  if (e != cudaSuccess) return e;
-  e = cudaFuncSetAttribute(k_letterbox<FMT, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kLetterboxSmemMax + 128);
-  if (e != cudaSuccess) return e;
-  if (!uniform_carveout) return e;
-  e = prefer_max_shared(k_letterbox<FMT, false>);
-  if (e != cudaSuccess) return e;
-  return prefer_max_shared(k_letterbox<FMT, true>);
+  cudaError_t e = configure_kernel(k_letterbox<FMT, false>, uniform_carveout);
+  if (e == cudaSuccess) e = configure_kernel(k_letterbox<FMT, true>, uniform_carveout);
+  if (e == cudaSuccess) e = configure_kernel(k_letterbox_nv12<FMT, false>, uniform_carveout);
+  if (e == cudaSuccess) e = configure_kernel(k_letterbox_nv12<FMT, true>, uniform_carveout);
+  return e;
 }
 
 int preprocess_configure(b200va_ctx* h) {
@@ -640,12 +955,50 @@ int preprocess_configure(b200va_ctx* h) {
   return B200VA_OK;
 }
 
-// Shared by b200va_preprocess (letterbox geometry) and b200va_resize_linear_u8 (no padding).
+// The source frames of one resample call: packed BGR (frames + pitches) or NV12 planes.
+struct SrcFrames {
+  const uint8_t* const* bgr = nullptr;
+  const int64_t* pitch = nullptr;         // BGR row pitches (NULL = 3 * w)
+  const b200va_nv12_frame* nv12 = nullptr;
+};
+
+// Fills the source fields of one frame descriptor; returns the bytes of one staged source row (-1: refused).
+static int set_source(b200va_ctx* h, const SrcFrames& src, int b, int src_h, int src_w, PreFrame& f) {
+  REQUIRE(h, src.bgr[b] != nullptr, "frame %d is NULL", b);
+  const int64_t pitch = src.pitch ? src.pitch[b] : (int64_t)3 * src_w;
+  REQUIRE(h, pitch >= (int64_t)3 * src_w, "frame %d: pitch %lld < 3*width", b, (long long)pitch);
+  f.src = src.bgr[b];
+  f.pitch = pitch;
+  const int rb = 3 * src_w;
+  f.bulk_ok = ((uintptr_t)f.src % 16 == 0) && (pitch % 16 == 0) && (rb % 16 == 0);
+  return B200VA_OK;
+}
+
+static int set_source(b200va_ctx* h, const SrcFrames& src, int b, int src_h, int src_w, Nv12Frame& f) {
+  const b200va_nv12_frame& n = src.nv12[b];
+  REQUIRE(h, n.y != nullptr && n.uv != nullptr, "frame %d: NULL plane", b);
+  REQUIRE(h, src_h % 2 == 0 && src_w % 2 == 0, "frame %d: NV12 needs an even size, got %dx%d", b, src_w, src_h);
+  REQUIRE(h, n.y_pitch >= src_w && n.uv_pitch >= src_w, "frame %d: plane pitch %lld / %lld < width %d", b,
+          (long long)n.y_pitch, (long long)n.uv_pitch, src_w);
+  f.y = n.y;
+  f.uv = n.uv;
+  f.y_pitch = n.y_pitch;
+  f.uv_pitch = n.uv_pitch;
+  f.bulk_ok = ((uintptr_t)n.y % 16 == 0) && ((uintptr_t)n.uv % 16 == 0) && (n.y_pitch % 16 == 0) && (n.uv_pitch % 16 == 0) &&
+              (src_w % 16 == 0);
+  return B200VA_OK;
+}
+
+// Shared by b200va_preprocess* (letterbox geometry) and b200va_resize_linear_u8* (no padding).
 // Frames with and without an ROI mask go to separate launches (the mask is a template switch).
-static int run_resample(b200va_ctx* h, const uint8_t* const* frames, const int* src_h, const int* src_w,
-                        const int64_t* src_pitch, int batch, const uint8_t* const* roi_masks, void* out,
-                        const int* new_h, const int* new_w, const int* pad_top, const int* pad_left, int dst_h,
-                        int dst_w, int fmt_and_flags, cudaStream_t st, uint8_t* const* outs = nullptr) {
+// P = PreParams (BGR frames, k_letterbox) or PreParamsNv12 (NV12 frames, k_letterbox_nv12).
+template <typename P>
+static int run_resample(b200va_ctx* h, const SrcFrames& src, const int* src_h, const int* src_w, int batch,
+                        const uint8_t* const* roi_masks, void* out, const int* new_h, const int* new_w, const int* pad_top,
+                        const int* pad_left, int dst_h, int dst_w, int fmt_and_flags, cudaStream_t st,
+                        uint8_t* const* outs = nullptr) {
+  constexpr bool kNv12 = std::is_same<P, PreParamsNv12>::value;
+  constexpr int kGroup = kNv12 ? kNv12LaunchFrames : B200VA_LAUNCH_FRAMES;
   const int fmt = fmt_and_flags & 0xff;
   REQUIRE(h, fmt >= 0 && fmt <= 3 && (fmt_and_flags & ~(0xff | B200VA_OUT_FLAG_PADS_VALID)) == 0, "unknown output format %d",
           fmt_and_flags);
@@ -654,36 +1007,32 @@ static int run_resample(b200va_ctx* h, const uint8_t* const* frames, const int* 
   for (int b = 0; b < batch; ++b) order[(roi_masks && roi_masks[b]) ? 1 : 0].push_back(b);
   for (int with_mask = 0; with_mask < 2; ++with_mask) {
     const std::vector<int>& idx = order[with_mask];
-    for (size_t base = 0; base < idx.size(); base += B200VA_LAUNCH_FRAMES) {
-      const int n = (int)std::min<size_t>(B200VA_LAUNCH_FRAMES, idx.size() - base);
-      PreParams p;
+    for (size_t base = 0; base < idx.size(); base += kGroup) {
+      const int n = (int)std::min<size_t>(kGroup, idx.size() - base);
+      P p;
       memset(&p, 0, sizeof(p));
       int max_row = 0, max_w = 0;
       bool all_single = true;
       for (int i = 0; i < n; ++i) {
         const int b = idx[base + i];
-        PreFrame& f = p.f[i];
-        REQUIRE(h, frames[b] != nullptr, "frame %d is NULL", b);
+        auto& f = p.f[i];
         REQUIRE(h, src_h[b] > 0 && src_w[b] > 0 && src_w[b] < 65536, "frame %d has unsupported size %dx%d", b, src_w[b], src_h[b]);
-        const int64_t pitch = src_pitch ? src_pitch[b] : (int64_t)3 * src_w[b];
-        REQUIRE(h, pitch >= (int64_t)3 * src_w[b], "frame %d: pitch %lld < 3*width", b, (long long)pitch);
+        int rc = set_source(h, src, b, src_h[b], src_w[b], f);
+        if (rc) return rc;
         REQUIRE(h, new_h[b] > 0 && new_w[b] > 0, "frame %d: resized size %dx%d is empty (cv2.resize would raise)", b, new_w[b], new_h[b]);
-        f.src = frames[b];
         f.mask = with_mask ? roi_masks[b] : nullptr;
-        f.pitch = pitch;
         f.src_h = src_h[b];
         f.src_w = src_w[b];
         f.out_idx = b;
         f.out = outs ? outs[b] : nullptr;
         bool single = true;
-        int rc = get_table(h, 0, src_w[b], new_w[b], pad_left[b], dst_w, &f.xtab, nullptr);
+        rc = get_table(h, 0, src_w[b], new_w[b], pad_left[b], dst_w, &f.xtab, nullptr);
         if (rc) return rc;
         rc = get_table(h, 1, src_h[b], new_h[b], pad_top[b], dst_h, &f.ytab, &single);
         if (rc) return rc;
         all_single = all_single && single;
-        const int rb = 3 * src_w[b];
-        f.bulk_ok = ((uintptr_t)f.src % 16 == 0) && (pitch % 16 == 0) && (rb % 16 == 0) &&
-                    (!f.mask || (((uintptr_t)f.mask % 16 == 0) && (src_w[b] % 16 == 0)));
+        const int rb = (kNv12 ? 1 : 3) * src_w[b];  // one staged source row (NV12: a luma row, and a chroma row as long)
+        f.bulk_ok = f.bulk_ok && (!f.mask || (((uintptr_t)f.mask % 16 == 0) && (src_w[b] % 16 == 0)));
         if (rb > max_row) max_row = rb;
         if (src_w[b] > max_w) max_w = src_w[b];
       }
@@ -699,7 +1048,8 @@ static int run_resample(b200va_ctx* h, const uint8_t* const* frames, const int* 
       p.row_stride = (max_row + 127) & ~127;
       p.mask_stride = with_mask ? ((max_w + 127) & ~127) : 0;
       p.rows_per_stage = all_single ? 1 : 2;
-      const size_t per_stage = (size_t)p.rows_per_stage * ((size_t)p.row_stride + p.mask_stride);
+      // an NV12 stage holds each luma row and its chroma row: 2 * src_w bytes per tapped row against 3 * src_w
+      const size_t per_stage = (size_t)p.rows_per_stage * ((kNv12 ? 2 : 1) * (size_t)p.row_stride + p.mask_stride);
       // ring depth: up to kMaxStages, but shallow enough that several CTAs share an SM -- with whole 4K rows a
       // 4-deep ring is 90-120 KB and leaves ONE 160-thread CTA per SM (7.6 % warps active, 0.59 of HBM peak)
       // (measured, 32 x 4K + ROI: 133 us with the deepest ring, 84 us = 0.94 of peak with a 32-56 KB budget)
@@ -746,6 +1096,17 @@ static int run_resample(b200va_ctx* h, const uint8_t* const* frames, const int* 
     }
   }
   return B200VA_OK;
+}
+
+static int run_resample(b200va_ctx* h, const uint8_t* const* frames, const int* src_h, const int* src_w,
+                        const int64_t* src_pitch, int batch, const uint8_t* const* roi_masks, void* out,
+                        const int* new_h, const int* new_w, const int* pad_top, const int* pad_left, int dst_h,
+                        int dst_w, int fmt_and_flags, cudaStream_t st, uint8_t* const* outs = nullptr) {
+  SrcFrames src;
+  src.bgr = frames;
+  src.pitch = src_pitch;
+  return run_resample<PreParams>(h, src, src_h, src_w, batch, roi_masks, out, new_h, new_w, pad_top, pad_left, dst_h, dst_w,
+                                 fmt_and_flags, st, outs);
 }
 
 extern "C" int b200va_preprocess(b200va_handle h, const uint8_t* const* frames, const int* src_h, const int* src_w,
@@ -873,6 +1234,74 @@ extern "C" int b200va_resize_linear_u8(b200va_handle h, const uint8_t* const* fr
   return B200VA_OK;
 }
 
+extern "C" int b200va_preprocess_nv12(b200va_handle h, const b200va_nv12_frame* frames, const int* src_h, const int* src_w,
+                                      int batch, const uint8_t* const* roi_masks, void* out, int dst_h, int dst_w,
+                                      int out_format, b200va_letterbox* meta_out, void* stream) {
+  if (!h) return B200VA_ERR_INVALID;
+  std::lock_guard<std::recursive_mutex> lock(h->mu);
+  DeviceGuard guard(h->cfg.device);
+  REQUIRE(h, frames && src_h && src_w && out, "NULL argument");
+  REQUIRE(h, batch >= 0 && batch <= h->cfg.max_batch, "batch %d outside [0, %d]", batch, h->cfg.max_batch);
+  REQUIRE(h, dst_h > 0 && dst_w > 0 && dst_w < 65536, "bad destination size %dx%d", dst_w, dst_h);
+  if (batch == 0) return B200VA_OK;
+  std::vector<int> nh(batch), nw(batch), pt(batch), pl(batch);
+  for (int b = 0; b < batch; ++b) {
+    b200va_letterbox m;
+    REQUIRE(h, b200va_letterbox_meta(src_h[b], src_w[b], dst_h, dst_w, &m) == B200VA_OK, "frame %d: bad size %dx%d", b, src_w[b], src_h[b]);
+    nh[b] = m.new_h;
+    nw[b] = m.new_w;
+    pt[b] = m.pad_top;
+    pl[b] = m.pad_left;
+    if (meta_out) meta_out[b] = m;
+  }
+  SrcFrames src;
+  src.nv12 = frames;
+  return run_resample<PreParamsNv12>(h, src, src_h, src_w, batch, roi_masks, out, nh.data(), nw.data(), pt.data(), pl.data(),
+                                     dst_h, dst_w, out_format, (cudaStream_t)stream);
+}
+
+extern "C" int b200va_resize_linear_u8_nv12(b200va_handle h, const b200va_nv12_frame* frames, const int* src_h,
+                                            const int* src_w, int batch, const uint8_t* const* roi_masks,
+                                            uint8_t* const* dst, const int* dst_h, const int* dst_w, void* stream) {
+  if (!h) return B200VA_ERR_INVALID;
+  std::lock_guard<std::recursive_mutex> lock(h->mu);
+  DeviceGuard guard(h->cfg.device);
+  REQUIRE(h, frames && src_h && src_w && dst && dst_h && dst_w, "NULL argument");
+  REQUIRE(h, batch >= 0 && batch <= h->cfg.max_batch, "batch %d outside [0, %d]", batch, h->cfg.max_batch);
+  // frames that share a destination size go out in one launch, as in b200va_resize_linear_u8
+  std::map<std::pair<int, int>, std::vector<int>> groups;
+  for (int b = 0; b < batch; ++b) {
+    REQUIRE(h, dst[b] != nullptr, "dst %d is NULL", b);
+    REQUIRE(h, dst_h[b] > 0 && dst_w[b] > 0 && dst_w[b] < 65536, "frame %d: bad destination size %dx%d", b, dst_w[b], dst_h[b]);
+    groups[{dst_h[b], dst_w[b]}].push_back(b);
+  }
+  for (const auto& kv : groups) {
+    const std::vector<int>& idx = kv.second;
+    const int n = (int)idx.size();
+    std::vector<b200va_nv12_frame> g_frames(n);
+    std::vector<const uint8_t*> g_masks(n);
+    std::vector<uint8_t*> g_out(n);
+    std::vector<int> g_h(n), g_w(n), g_nh(n, kv.first.first), g_nw(n, kv.first.second), g_zero(n, 0);
+    bool any_mask = false;
+    for (int i = 0; i < n; ++i) {
+      const int b = idx[i];
+      g_frames[i] = frames[b];
+      g_masks[i] = roi_masks ? roi_masks[b] : nullptr;
+      any_mask = any_mask || g_masks[i] != nullptr;
+      g_out[i] = dst[b];
+      g_h[i] = src_h[b];
+      g_w[i] = src_w[b];
+    }
+    SrcFrames src;
+    src.nv12 = g_frames.data();
+    int rc = run_resample<PreParamsNv12>(h, src, g_h.data(), g_w.data(), n, any_mask ? g_masks.data() : nullptr, g_out[0],
+                                         g_nh.data(), g_nw.data(), g_zero.data(), g_zero.data(), kv.first.first,
+                                         kv.first.second, B200VA_OUT_U8_BGR_NHWC, (cudaStream_t)stream, g_out.data());
+    if (rc) return rc;
+  }
+  return B200VA_OK;
+}
+
 // ---- host -> device staging of decoded frames ---------------------------------------------------
 // The letterbox reads only the source rows that carry a non-zero vertical weight (every third row
 // for 1080p -> 640x360, two rows in six for 4K).  With rows_mode = 1 only those rows cross PCIe, into
@@ -970,6 +1399,107 @@ extern "C" int b200va_upload_frames(b200va_handle h, const uint8_t* const* host_
         CUDA_TRY(h, cudaMemcpy2DAsync(dev_frames[b], dp, host_frames[b], hp, rb, src_h[b], cudaMemcpyHostToDevice, st));
       total += (int64_t)rb * src_h[b];
     }
+  }
+  if (bytes_copied) *bytes_copied = total;
+  return B200VA_OK;
+}
+
+namespace {
+// One plane's needed rows as at most `max_runs` strided copies (start, step, count): from the first row not yet
+// covered, the longest arithmetic progression through one of the next four such rows.  1080p -> 640 x 640 needs luma
+// rows 1, 4, 7, ... (one progression) and chroma rows 0, 2, 3, 5, 6, ... = {0, 3, 6, ...} + {2, 5, 8, ...}.
+// Returns false when the rows need more copies than that.
+struct RowRun {
+  int start, step, count;
+};
+bool row_progressions(const std::vector<char>& need, size_t max_runs, std::vector<RowRun>* out) {
+  const int n = (int)need.size();
+  std::vector<char> left(need);
+  out->clear();
+  for (int r = 0; r < n; ++r) {
+    if (!left[r]) continue;
+    if (out->size() == max_runs) return false;
+    RowRun best{r, 1, 1};
+    int tried = 0;
+    for (int q = r + 1; q < n && tried < 4; ++q) {
+      if (!left[q]) continue;
+      ++tried;
+      int count = 1;
+      for (int y = q; y < n && left[y]; y += q - r) ++count;
+      if (count > best.count) best = RowRun{r, q - r, count};
+    }
+    for (int k = 0; k < best.count; ++k) left[r + k * best.step] = 0;
+    out->push_back(best);
+  }
+  return true;
+}
+
+// Copies the needed rows of one plane (every row when `need` is empty or the rows are too scattered to gain).
+int copy_plane_rows(b200va_ctx* h, uint8_t* dst, int64_t dp, const uint8_t* src, int64_t hp, int64_t row_bytes, int rows,
+                    const std::vector<char>& need, cudaStream_t st, int64_t* moved) {
+  if (!need.empty()) {
+    std::vector<RowRun> runs;
+    int64_t n = 0;
+    for (char c : need) n += c ? 1 : 0;
+    // nothing to gain when (nearly) every row is needed
+    if (n * 10 <= (int64_t)rows * 8 && row_progressions(need, 8, &runs)) {
+      for (const RowRun& r : runs)
+        CUDA_TRY(h, cudaMemcpy2DAsync(dst + (size_t)r.start * dp, (size_t)r.step * dp, src + (size_t)r.start * hp,
+                                      (size_t)r.step * hp, (size_t)row_bytes, r.count, cudaMemcpyHostToDevice, st));
+      *moved += n * row_bytes;
+      return B200VA_OK;
+    }
+  }
+  if (hp == row_bytes && dp == row_bytes)
+    CUDA_TRY(h, cudaMemcpyAsync(dst, src, (size_t)row_bytes * rows, cudaMemcpyHostToDevice, st));
+  else
+    CUDA_TRY(h, cudaMemcpy2DAsync(dst, dp, src, hp, (size_t)row_bytes, rows, cudaMemcpyHostToDevice, st));
+  *moved += row_bytes * rows;
+  return B200VA_OK;
+}
+}  // namespace
+
+extern "C" int b200va_upload_frames_nv12(b200va_handle h, const b200va_nv12_frame* host, const b200va_nv12_frame* dev,
+                                         const int* src_h, const int* src_w, int batch, int dst_h, int dst_w, int rows_mode,
+                                         int64_t* bytes_copied, void* stream) {
+  if (!h) return B200VA_ERR_INVALID;
+  std::lock_guard<std::recursive_mutex> lock(h->mu);
+  DeviceGuard guard(h->cfg.device);
+  cudaStream_t st = (cudaStream_t)stream;
+  REQUIRE(h, host && dev && src_h && src_w, "NULL argument");
+  REQUIRE(h, batch >= 0, "negative batch");
+  REQUIRE(h, rows_mode == 0 || rows_mode == 1, "unknown rows_mode %d", rows_mode);
+  for (int b = 0; b < batch; ++b) {
+    REQUIRE(h, host[b].y && host[b].uv && dev[b].y && dev[b].uv, "frame %d: NULL plane", b);
+    REQUIRE(h, src_h[b] > 0 && src_w[b] > 0 && src_h[b] % 2 == 0 && src_w[b] % 2 == 0, "frame %d: NV12 needs an even size, got %dx%d",
+            b, src_w[b], src_h[b]);
+    REQUIRE(h, host[b].y_pitch >= src_w[b] && host[b].uv_pitch >= src_w[b] && dev[b].y_pitch >= src_w[b] &&
+                   dev[b].uv_pitch >= src_w[b],
+            "frame %d: plane pitch smaller than the width", b);
+  }
+  PhaseScope phase(h, B200VA_PHASE_UPLOAD, st);
+  int64_t total = 0;
+  for (int b = 0; b < batch; ++b) {
+    const int H = src_h[b], W = src_w[b];
+    std::vector<char> need_y, need_uv;
+    if (rows_mode == 1) {
+      b200va_letterbox m;
+      REQUIRE(h, b200va_letterbox_meta(H, W, dst_h, dst_w, &m) == B200VA_OK && m.new_h > 0, "frame %d: bad letterbox geometry", b);
+      need_y.assign((size_t)H, 0);
+      need_uv.assign((size_t)H / 2, 0);
+      for (int d = 0; d < m.new_h; ++d) {
+        int y0, y1;
+        short b0, b1;
+        linear_tap(H, m.new_h, d, false, &y0, &y1, &b0, &b1);
+        if (b0) need_y[y0] = need_uv[y0 >> 1] = 1;
+        if (b1) need_y[y1] = need_uv[y1 >> 1] = 1;
+      }
+    }
+    int rc = copy_plane_rows(h, const_cast<uint8_t*>(dev[b].y), dev[b].y_pitch, host[b].y, host[b].y_pitch, W, H, need_y, st, &total);
+    if (rc) return rc;
+    rc = copy_plane_rows(h, const_cast<uint8_t*>(dev[b].uv), dev[b].uv_pitch, host[b].uv, host[b].uv_pitch, W, H / 2, need_uv, st,
+                         &total);
+    if (rc) return rc;
   }
   if (bytes_copied) *bytes_copied = total;
   return B200VA_OK;

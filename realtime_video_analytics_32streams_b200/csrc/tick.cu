@@ -7,8 +7,16 @@ int postprocess_then_track(b200va_handle h, const b200va_tick_args* a, void* str
 int postprocess_run_pending(b200va_handle h, void* stream);            // postprocess.cu
 bool postprocess_has_pending(b200va_handle h);                         // postprocess.cu
 
-extern "C" int b200va_tick(b200va_handle h, const b200va_tick_args* a, void* stream) {
-  if (!h || !a) return B200VA_ERR_INVALID;
+// The letterbox of one tick: BGR frames (a->frames) or, when `nv12` is given, NV12 frames.
+static int tick_letterbox(b200va_handle h, const b200va_tick_args* a, const b200va_nv12_frame* nv12, cudaStream_t st) {
+  if (nv12)
+    return b200va_preprocess_nv12(h, nv12, a->src_h, a->src_w, a->batch, a->roi_masks, a->net_out, a->dst_h, a->dst_w,
+                                  a->out_format, a->meta_out, st);
+  return b200va_preprocess(h, a->frames, a->src_h, a->src_w, a->src_pitch, a->batch, a->roi_masks, a->net_out, a->dst_h,
+                           a->dst_w, a->out_format, a->meta_out, st);
+}
+
+static int tick_impl(b200va_handle h, const b200va_tick_args* a, const b200va_nv12_frame* nv12, void* stream) {
   std::lock_guard<std::recursive_mutex> lock(h->mu);
   DeviceGuard guard(h->cfg.device);
   REQUIRE(h, a->schedule >= 0 && a->schedule <= 6, "unknown schedule %d", a->schedule);
@@ -21,7 +29,7 @@ extern "C" int b200va_tick(b200va_handle h, const b200va_tick_args* a, void* str
   // against 0.129 ms).
   const int schedule = a->schedule == 6 ? ((h->nms_dense_ttl > 0 || a->batch < 24) ? 1 : 3) : a->schedule;
   cudaStream_t main_st = (cudaStream_t)stream;
-  const bool has_pre = a->frames != nullptr && a->batch > 0;
+  const bool has_pre = (nv12 != nullptr || a->frames != nullptr) && a->batch > 0;
   const bool has_post = a->head != nullptr && a->head_batch > 0;
   const bool has_trk = a->stream_slots != nullptr && a->trk_batch > 0;
   // schedule 4, the software-pipelined tick: this call only DECODES its head; NMS + tracker of the head decoded by the
@@ -60,9 +68,7 @@ extern "C" int b200va_tick(b200va_handle h, const b200va_tick_args* a, void* str
                                  a->id_base, a->tracks, a->new_counts, main_st);
     if (rc == B200VA_OK && has_pre) {
       if (a->ev_pre_begin) note(cudaEventRecord((cudaEvent_t)a->ev_pre_begin, main_st), "cudaEventRecord(pre_begin)");
-      if (rc == B200VA_OK)
-        rc = b200va_preprocess(h, a->frames, a->src_h, a->src_w, a->src_pitch, a->batch, a->roi_masks, a->net_out, a->dst_h,
-                               a->dst_w, a->out_format, a->meta_out, main_st);
+      if (rc == B200VA_OK) rc = tick_letterbox(h, a, nv12, main_st);
       if (rc == B200VA_OK && a->ev_pre_end) note(cudaEventRecord((cudaEvent_t)a->ev_pre_end, main_st), "cudaEventRecord(pre_end)");
     }
     if (side) note(cudaStreamWaitEvent(main_st, h->ev_join, 0), "cudaStreamWaitEvent(join)");
@@ -107,13 +113,25 @@ extern "C" int b200va_tick(b200va_handle h, const b200va_tick_args* a, void* str
   h->pdl_preprocess_wait = schedule == 5;
   if (rc == B200VA_OK && has_pre) {
     if (a->ev_pre_begin) note(cudaEventRecord((cudaEvent_t)a->ev_pre_begin, main_st), "cudaEventRecord(pre_begin)");
-    if (rc == B200VA_OK)
-      rc = b200va_preprocess(h, a->frames, a->src_h, a->src_w, a->src_pitch, a->batch, a->roi_masks, a->net_out, a->dst_h,
-                             a->dst_w, a->out_format, a->meta_out, main_st);
+    if (rc == B200VA_OK) rc = tick_letterbox(h, a, nv12, main_st);
     if (rc == B200VA_OK && a->ev_pre_end) note(cudaEventRecord((cudaEvent_t)a->ev_pre_end, main_st), "cudaEventRecord(pre_end)");
   }
   h->pdl_preprocess = false;
   h->pdl_preprocess_wait = false;
   if (joined) note(cudaStreamWaitEvent(main_st, h->ev_join, 0), "cudaStreamWaitEvent(join)");
   return rc;
+}
+
+extern "C" int b200va_tick(b200va_handle h, const b200va_tick_args* a, void* stream) {
+  if (!h || !a) return B200VA_ERR_INVALID;
+  return tick_impl(h, a, nullptr, stream);
+}
+
+extern "C" int b200va_tick_nv12(b200va_handle h, const b200va_tick_args* a, const b200va_nv12_frame* frames, void* stream) {
+  if (!h || !a) return B200VA_ERR_INVALID;
+  if (!frames && a->batch > 0) {
+    std::lock_guard<std::recursive_mutex> lock(h->mu);
+    return set_error(h, B200VA_ERR_INVALID, "b200va_tick_nv12: NULL frames for a batch of %d", a->batch);
+  }
+  return tick_impl(h, a, frames, stream);
 }

@@ -34,6 +34,14 @@ from .types import Detection, MotionFilterConfig, Track
 LOGGER = logging.getLogger(__name__)
 
 
+def _hw(frame):
+    """(height, width) of a BGR [H, W, 3] frame or of an NV12 frame's luma."""
+    if _native.is_nv12(frame):
+        y, _ = _native.nv12_planes(frame)
+        return int(y.shape[0]), int(y.shape[1])
+    return int(frame.shape[0]), int(frame.shape[1])
+
+
 @dataclass
 class _StreamState:
     """Host-side gate state of one stream (pipeline.py:88-116)."""
@@ -221,19 +229,38 @@ class HotPathEngine:
 
     # --------------------------------------------------------------------------------------
     def _frame_batch(self, frames, masks):
-        """Argument arrays are cached per set of device pointers (staging buffers are persistent)."""
+        """Argument arrays are cached per set of device pointers (staging buffers are persistent).  ``frames`` are
+        all BGR or all NV12."""
+        make = _native.Nv12Batch if _native.is_nv12(frames[0]) else _native.FrameBatch
         if not all(self.stager.owns(f) or id(f) in self._persistent for f in frames):
             # caller-supplied CUDA frames: their addresses change from tick to tick, and a cached batch would
             # keep the tensors (and their HBM) alive -- build the argument arrays for this tick only
-            return _native.FrameBatch(frames, masks)
+            return make(frames, masks)
         key = tuple((f.data_ptr(), f.shape[0], f.shape[1], f.stride(0), m.data_ptr() if m is not None else 0)
                     for f, m in zip(frames, masks))
         fb = self._batches.get(key)
         if fb is None:
             if len(self._batches) > 64:
                 self._batches.clear()
-            fb = self._batches[key] = _native.FrameBatch(frames, masks)
+            fb = self._batches[key] = make(frames, masks)
         return fb
+
+    def _letterbox(self, frames, masks, fmt, out, skip=None):
+        """``preprocess`` of a batch whose frames may mix BGR and NV12: one call per run of consecutive frames of one
+        kind, into the rows of ``out`` (and, with device-side gates, the entries of ``skip``) at their positions."""
+        kinds = [_native.is_nv12(f) for f in frames]
+        metas = []
+        b = 0
+        while b < len(frames):
+            e = b + 1
+            while e < len(frames) and kinds[e] == kinds[b]:
+                e += 1
+            if skip is not None and (b, e) != (0, len(frames)):
+                self.h.set_skip_mask(skip[b:e])
+            _, m = self.h.preprocess(self._frame_batch(frames[b:e], masks[b:e]), self.detector.input_hw, fmt, out=out[b:e])
+            metas += m
+            b = e
+        return out, metas
 
     def _net_in(self, n: int):
         t = self.h.torch
@@ -243,10 +270,19 @@ class HotPathEngine:
             self._net_shapes = [None] * self._net.shape[0]  # source (h, w) whose pad rows each position holds
         return self._net[:n]
 
+    def _bgr_buffer(self, pos: int, hw, full: bool = False):
+        """One persistent BGR buffer per (stream position, size, purpose): stable addresses, no per-tick allocation."""
+        key = (pos, tuple(hw), full)
+        buf = self._small.get(key)
+        if buf is None:
+            buf = self._small[key] = self.h.torch.empty((hw[0], hw[1], 3), dtype=self.h.torch.uint8, device=self.h.device)
+            self._persistent.add(id(buf))
+        return buf
+
     def _pads_flag(self, frames) -> int:
         """B200VA_OUT_FLAG_PADS_VALID when every batch position was last written from a frame of the same size
         (same letterbox geometry, same format): its pad rows are already in the persistent buffer."""
-        shapes = [(int(f.shape[0]), int(f.shape[1])) for f in frames]
+        shapes = [_hw(f) for f in frames]
         valid = all(self._net_shapes[k] == sh for k, sh in enumerate(shapes))
         for k, sh in enumerate(shapes):
             self._net_shapes[k] = sh
@@ -255,7 +291,9 @@ class HotPathEngine:
     # --------------------------------------------------------------------------------------
     def tick(self, frames: Sequence, frame_ids: Optional[Sequence[int]] = None, infer_ctx=None) -> List[FrameResult]:
         """``frames[i]`` is the new frame of ``streams[i]`` (host array, pinned CPU tensor or CUDA
-        tensor) or None when that stream delivered nothing this tick."""
+        tensor) or None when that stream delivered nothing this tick.  A frame may be BGR ``[H, W, 3]`` or NV12: a
+        2-D ``[3H/2, W]`` uint8 host array / CPU tensor / CUDA tensor, or a ``(y, uv)`` pair of CUDA planes.  NV12
+        results equal those of the same engine fed ``cv2.cvtColor(frame, cv2.COLOR_YUV2BGR_NV12)``."""
         ctx = self.submit(frames, frame_ids, infer_ctx)
         return self.collect(ctx) if ctx is not None else []
 
@@ -288,27 +326,33 @@ class HotPathEngine:
         masks, ratios = [], []
         for st, f in zip(states, dev_frames):
             polys = getattr(st.cfg, "roi_polygons", None) or []
-            masks.append(roi_mask(polys, f.shape[0], f.shape[1], self.h) if polys else None)
+            masks.append(roi_mask(polys, *_hw(f), self.h) if polys else None)
             ratios.append(float(getattr(st.cfg, "downsample_ratio", 1.0)))
         down = [k for k, r in enumerate(ratios) if r < 0.999]
         work = list(dev_frames)
         work_masks = list(masks)
         if down:
-            sizes = [(int(dev_frames[k].shape[0] * ratios[k]), int(dev_frames[k].shape[1] * ratios[k])) for k in down]
-            outs = []
-            for k, sz in zip(down, sizes):  # one persistent output per (stream, size): stable addresses, no per-tick allocation
-                key = (live[k], sz)
-                buf = self._small.get(key)
-                if buf is None:
-                    buf = self._small[key] = self.h.torch.empty((sz[0], sz[1], 3), dtype=self.h.torch.uint8, device=self.h.device)
-                    self._persistent.add(id(buf))
-                outs.append(buf)
-            small = self.h.resize([dev_frames[k] for k in down], sizes, [masks[k] for k in down], outs=outs)
-            for k, s in zip(down, small):
-                work[k] = s
-                work_masks[k] = None  # the ROI is already baked into the downsampled frame
+            sizes = {k: (int(_hw(dev_frames[k])[0] * ratios[k]), int(_hw(dev_frames[k])[1] * ratios[k])) for k in down}
+            # NV12 frames are converted in the same taps (resize_linear_u8_nv12); one call per source format
+            for group in ([k for k in down if not _native.is_nv12(dev_frames[k])], [k for k in down if _native.is_nv12(dev_frames[k])]):
+                if not group:
+                    continue
+                outs = [self._bgr_buffer(live[k], sizes[k]) for k in group]
+                small = self.h.resize([dev_frames[k] for k in group], [sizes[k] for k in group], [masks[k] for k in group],
+                                      outs=outs)
+                for k, s in zip(group, small):
+                    work[k] = s
+                    work_masks[k] = None  # the ROI is already baked into the downsampled frame
 
         mot = [k for k, st in enumerate(states) if getattr(st.cfg, "motion_filter", False)]
+        # the motion gate reads BGR: an NV12 frame it sees is converted at its own size (cv2.cvtColor) into a
+        # persistent per-stream buffer, which the letterbox then reads too
+        cvt = [k for k in mot if _native.is_nv12(work[k])]
+        if cvt:
+            outs = [self._bgr_buffer(live[k], _hw(work[k]), full=True) for k in cvt]
+            full = self.h.resize([work[k] for k in cvt], [_hw(work[k]) for k in cvt], outs=outs)
+            for k, f in zip(cvt, full):
+                work[k] = f
         if self.device_gates:
             return self._submit_device_gates(ctx, live, names, states, ids, work, work_masks, ratios, mot, infer_ctx)
 
@@ -346,9 +390,8 @@ class HotPathEngine:
         if n_act:
             net = self._net_in(n_act)
             act_frames = [work[k] for k in active]
-            tensor, metas = self.h.preprocess(self._frame_batch(act_frames, [work_masks[k] for k in active]),
-                                              self.detector.input_hw, self.detector._fmt | self._pads_flag(act_frames),
-                                              out=net)
+            tensor, metas = self._letterbox(act_frames, [work_masks[k] for k in active],
+                                            self.detector._fmt | self._pads_flag(act_frames), net)
             # which stream each row of `tensor` belongs to (index into self.streams), for callers whose forward
             # is per-stream (model selection, synthetic heads in tests)
             self.active_streams = [live[k] for k in active]
@@ -402,7 +445,7 @@ class HotPathEngine:
             g.max_process_every = max(st.max_process_every, 1)
             g.idle_tolerance = max(st.idle_tolerance, 1)
             g.motion_threshold = float(st.cfg.motion_threshold) if k in where else 0.0
-            g.pixels = int(work[k].shape[0]) * int(work[k].shape[1])
+            g.pixels = _hw(work[k])[0] * _hw(work[k])[1]
         skip = ctx.skip[:nb]
         h.gates_decide(gates, changed, skip)
         dets = {k_: v[:nb] for k_, v in ctx.dets.items() if not k_.startswith("_")}
@@ -412,8 +455,7 @@ class HotPathEngine:
             pads = self._pads_flag(work)
             # a batch position whose pad rows were never written must be letterboxed whatever its gate says
             h.set_skip_mask(skip if pads else None)
-            tensor, metas = h.preprocess(self._frame_batch(work, work_masks), self.detector.input_hw,
-                                         self.detector._fmt | pads, out=net)
+            tensor, metas = self._letterbox(work, work_masks, self.detector._fmt | pads, net, skip if pads else None)
             h.set_skip_mask(skip)
             self.active_streams = list(live)
             head = self.detector._infer(tensor) if infer_ctx is None else self.detector._infer_fn(tensor, infer_ctx)

@@ -108,16 +108,42 @@ class FrameStager:
         return buf
 
     def upload(self, frames: Sequence, sparse_for=None, sparse_ok: Optional[Sequence[bool]] = None) -> List:
-        """Return CUDA uint8 [H,W,3] tensors for ``frames``; CUDA tensors pass through untouched."""
+        """Return CUDA uint8 [H,W,3] tensors for ``frames``; CUDA tensors pass through untouched.  Host NV12 frames
+        (uint8 ``[3H/2, W]`` NumPy arrays or CPU tensors, OpenCV's layout) land in CUDA ``[3H/2, W]`` tensors, half the
+        bytes of BGR, sparsely under the same ``sparse_ok`` rule; ``(y, uv)`` pairs of CUDA planes pass through."""
         t = self.h.torch
         out: List = [None] * len(frames)
         groups = {False: ([], []), True: ([], [])}
+        nv12 = {False: ([], []), True: ([], [])}
         keep = []
         for k, f in enumerate(frames):
             if f is None:
                 continue
-            if t.is_tensor(f) and f.is_cuda:
+            if (t.is_tensor(f) and f.is_cuda) or isinstance(f, (tuple, list)):
                 out[k] = f
+                continue
+            sparse = bool(sparse_for) and (sparse_ok is None or bool(sparse_ok[k]))
+            if _native.is_nv12(f):
+                a = f if t.is_tensor(f) else np.asarray(f)
+                if t.is_tensor(a):
+                    if a.dtype != t.uint8 or a.stride(1) != 1:
+                        raise ValueError("NV12 frames must be uint8 [3H/2, W] with unit column stride")
+                    ptr, pitch = a.data_ptr(), a.stride(0)
+                else:
+                    if a.dtype != np.uint8:
+                        raise ValueError("NV12 frames must be uint8 [3H/2, W]")
+                    if a.strides[1] != 1:
+                        a = np.ascontiguousarray(a)
+                    ptr, pitch = a.ctypes.data, a.strides[0]
+                rows, w = int(a.shape[0]), int(a.shape[1])
+                if rows % 3 or (rows // 3) % 2 or w % 2:
+                    raise ValueError(f"NV12 frames are [3H/2, W] with H and W even, got {(rows, w)}")
+                h = rows * 2 // 3
+                keep.append(a)
+                dev = self.device_buffer(k, (rows, w))
+                out[k] = dev
+                nv12[sparse][0].append(_native.Nv12Frame(ptr, ptr + h * pitch, pitch, pitch))
+                nv12[sparse][1].append(dev)
                 continue
             if t.is_tensor(f):
                 if f.dtype != t.uint8 or f.dim() != 3 or f.shape[2] != 3 or f.stride(2) != 1 or f.stride(1) != 3:
@@ -134,11 +160,13 @@ class FrameStager:
             keep.append(f)
             dev = self.device_buffer(k, shape)
             out[k] = dev
-            sparse = bool(sparse_for) and (sparse_ok is None or bool(sparse_ok[k]))
             groups[sparse][0].append((ptr, pitch))
             groups[sparse][1].append(dev)
         for sparse, (ptrs, devs) in groups.items():
             if devs:
                 self.bytes_moved += self.h.upload_frames(ptrs, devs, sparse_for if sparse else None)
+        for sparse, (hosts, devs) in nv12.items():
+            if devs:
+                self.bytes_moved += self.h.upload_frames_nv12(hosts, devs, sparse_for if sparse else None)
         self._keep = keep  # sources stay alive until the caller synchronises (end of the tick)
         return out
