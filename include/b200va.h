@@ -265,6 +265,14 @@ B200VA_API int b200va_preprocess_nv12(b200va_handle h, const b200va_nv12_frame* 
 B200VA_API int b200va_resize_linear_u8_nv12(b200va_handle h, const b200va_nv12_frame* frames, const int* src_h,
                                             const int* src_w, int batch, const uint8_t* const* roi_masks,
                                             uint8_t* const* dst, const int* dst_h, const int* dst_w, void* stream);
+/* b200va_resize_area_u8 (the 8f-3 preview downscale, below) for NV12 frames: BGR uint8 HWC out (dst pitch = 3 * dst_w),
+ * byte-identical to cv2.resize(cv2.cvtColor(frame, COLOR_YUV2BGR_NV12), (dst_w, dst_h), interpolation=cv2.INTER_AREA);
+ * every source pixel is converted and saturated before it is summed.  With dst == src size this is cv2.cvtColor itself.
+ * Frames are grouped by (source, destination) size, at most 64 per launch, under B200VA_PHASE_EGRESS.  Shrinking only;
+ * odd source sizes, NULL planes, plane pitches below src_w and enlarging are refused with B200VA_ERR_INVALID. */
+B200VA_API int b200va_resize_area_u8_nv12(b200va_handle h, const b200va_nv12_frame* frames, const int* src_h,
+                                          const int* src_w, int batch, uint8_t* const* dst, const int* dst_h,
+                                          const int* dst_w, void* stream);
 /* b200va_upload_frames for NV12 frames: host[i] (HOST planes, pinned for asynchronous copies) -> dev[i] (DEVICE
  * planes, written through the const pointers).  rows_mode 0 copies both planes whole; rows_mode 1 copies only the
  * luma rows b200va_preprocess_nv12 to dst_h x dst_w reads and the chroma rows those use (each once) -- e.g. 1,382,400
@@ -529,7 +537,7 @@ B200VA_API int b200va_tick_nv12(b200va_handle h, const b200va_tick_args* args, c
  * shrinking only (kafka_sink.py:227-232 downscales frames above 1920x1080).  Bit-exact with OpenCV 4.x: whole 2x2
  * blocks round half up ((a+b+c+d+2)>>2, the vector kernel), other whole blocks multiply by float(1/area) and round
  * half to even, fractional ratios accumulate float32 products in computeResizeAreaTab order.
- * frames / dst: HOST arrays [batch] of DEVICE pointers; dst pitch = 3 * dst_w. */
+ * frames / dst: HOST arrays [batch] of DEVICE pointers; dst pitch = 3 * dst_w.  NV12 frames: b200va_resize_area_u8_nv12. */
 B200VA_API int b200va_resize_area_u8(b200va_handle h, const uint8_t* const* frames, const int* src_h, const int* src_w,
                                      const int64_t* src_pitch, int batch, uint8_t* const* dst, const int* dst_h,
                                      const int* dst_w, void* stream);

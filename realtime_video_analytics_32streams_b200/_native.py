@@ -136,6 +136,7 @@ EXPORTS = (
     "b200va_read_status_async", "b200va_resize_area_u8", "b200va_draw_rects", "b200va_tracks_json",
     "b200va_gates_decide", "b200va_gates_commit", "b200va_gates_reset", "b200va_set_skip_mask",
     "b200va_preprocess_nv12", "b200va_resize_linear_u8_nv12", "b200va_upload_frames_nv12", "b200va_tick_nv12",
+    "b200va_resize_area_u8_nv12",
 )
 PHASES = ("upload", "roi", "resize", "motion", "preprocess", "decode", "nms", "tracker", "dfl", "tick", "egress")  # enum b200va_phase
 
@@ -209,6 +210,7 @@ def load_library() -> C.CDLL:
     lib.b200va_resize_linear_u8_nv12.argtypes = [vp, nv, ip, ip, C.c_int, C.POINTER(vp), C.POINTER(vp), ip, ip, vp]
     lib.b200va_upload_frames_nv12.argtypes = [vp, nv, nv, ip, ip, C.c_int, C.c_int, C.c_int, C.c_int, i64p, vp]
     lib.b200va_tick_nv12.argtypes = [vp, C.POINTER(TickArgs), nv, vp]
+    lib.b200va_resize_area_u8_nv12.argtypes = [vp, nv, ip, ip, C.c_int, C.POINTER(vp), ip, ip, vp]
     lib.b200va_tracks_json.restype = C.c_int64
     lib.b200va_tracks_json.argtypes = [C.c_char_p, C.c_int64, vp, vp, vp, vp, C.c_int, C.c_char_p, vp, C.c_int64]
     for name in EXPORTS:
@@ -308,6 +310,16 @@ class FrameBatch:
 def is_nv12(frame) -> bool:
     """True for an NV12 frame: a ``(y, uv)`` pair or a 2-D ``[3H/2, W]`` array / tensor (BGR frames are ``[H, W, 3]``)."""
     return isinstance(frame, (tuple, list)) or getattr(frame, "ndim", 3) == 2
+
+
+def frame_hw(frame):
+    """(height, width) of a BGR ``[H, W, 3]`` frame, or of an NV12 frame's luma: ``H`` of a ``[3H/2, W]`` array /
+    tensor (host or CUDA) or the ``y`` plane's size of a ``(y, uv)`` pair."""
+    if isinstance(frame, (tuple, list)):
+        return int(frame[0].shape[0]), int(frame[0].shape[1])
+    if is_nv12(frame):
+        return int(frame.shape[0]) * 2 // 3, int(frame.shape[1])
+    return int(frame.shape[0]), int(frame.shape[1])
 
 
 def nv12_planes(frame):
@@ -463,8 +475,8 @@ class Handle:
                 return FrameBatch(frames, roi_masks)
             frames = Nv12Batch(frames, roi_masks) if nv12_ok else frames
         if not nv12_ok:
-            raise ValueError("NV12 frames are taken by preprocess, resize and plan_tick; convert them with "
-                             "resize at their own size for the other calls")
+            raise ValueError("NV12 frames are taken by preprocess, resize, resize_area and plan_tick; convert them "
+                             "with resize at their own size for the other calls")
         return frames
 
     # -- staging ----------------------------------------------------------------------------
@@ -548,18 +560,24 @@ class Handle:
 
     # -- 8f-3 -------------------------------------------------------------------------------
     def resize_area(self, frames, dst_hw_list, outs=None):
-        """``cv2.resize(frame, (w, h), interpolation=cv2.INTER_AREA)`` per frame, shrinking only (kafka_sink.py:227-232)."""
+        """``cv2.resize(frame, (w, h), interpolation=cv2.INTER_AREA)`` per frame, shrinking only (kafka_sink.py:227-232).
+        NV12 frames (``[3H/2, W]`` tensors, ``(y, uv)`` pairs or an ``Nv12Batch``) give the result of the BGR call on
+        their ``cv2.cvtColor`` conversion; at their own size that is the conversion itself."""
         t = self.torch
         if outs is None:
             outs = [t.empty((int(h), int(w), 3), dtype=t.uint8, device=self.device) for h, w in dst_hw_list]
         elif any(tuple(o.shape) != (int(h), int(w), 3) or o.dtype != t.uint8 or not o.is_contiguous() or not o.is_cuda
                  for o, (h, w) in zip(outs, dst_hw_list)) or len(outs) != len(dst_hw_list):
             raise ValueError("resize_area: `outs` must be contiguous CUDA uint8 tensors [h, w, 3] matching dst_hw_list")
-        fb = self._batch(frames)
-        if fb.n:
+        fb = self._batch(frames, nv12_ok=True)
+        hs, ws = _int_array([h for h, _ in dst_hw_list]), _int_array([w for _, w in dst_hw_list])
+        if fb.n and isinstance(fb, Nv12Batch):
+            self._check(self.lib.b200va_resize_area_u8_nv12(
+                self._h, fb.nv, fb.hs, fb.ws, fb.n, _ptr_array([o.data_ptr() for o in outs]), hs, ws, self._stream()))
+        elif fb.n:
             self._check(self.lib.b200va_resize_area_u8(
-                self._h, fb.ptrs, fb.hs, fb.ws, fb.pitch, fb.n, _ptr_array([o.data_ptr() for o in outs]),
-                _int_array([h for h, _ in dst_hw_list]), _int_array([w for _, w in dst_hw_list]), self._stream()))
+                self._h, fb.ptrs, fb.hs, fb.ws, fb.pitch, fb.n, _ptr_array([o.data_ptr() for o in outs]), hs, ws,
+                self._stream()))
         return outs
 
     @staticmethod

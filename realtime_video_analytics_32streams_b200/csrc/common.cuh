@@ -330,4 +330,30 @@ template <int N>
 __device__ __forceinline__ void cp_async_wait() {
   asm volatile("cp.async.wait_group %0;\n" ::"n"(N) : "memory");
 }
+
+// ---- NV12 -> BGR (preprocess.cu's letterbox taps, egress.cu's INTER_AREA) ---------------------
+// cv::cvtColor YUV2BGR_NV12 (modules/imgproc/src/color_yuv.simd.hpp, 8-bit path): ITU-R BT.601 limited range in
+// 20-bit fixed point, rounded by the 1 << 19 bias and saturated.  `uv` = Cb | Cr << 8 of the pixel's 2 x 2 block.
+// Returns the pixel packed as B | G << 8 | R << 16 (byte 3 is zero).
+constexpr int kNv12Y = 1220542, kNv12UB = 2116026, kNv12VG = 852492, kNv12UG = 409993, kNv12VR = 1673527;
+__device__ __forceinline__ uint32_t nv12_bgr(int Y, uint32_t uv) {
+  const int y = max(Y - 16, 0) * kNv12Y + (1 << 19);
+  const int u = (int)(uv & 0xffu) - 128, v = (int)(uv >> 8) - 128;
+  const uint32_t b = (uint32_t)min(max((y + kNv12UB * u) >> 20, 0), 255);
+  const uint32_t g = (uint32_t)min(max((y - kNv12VG * v - kNv12UG * u) >> 20, 0), 255);
+  const uint32_t r = (uint32_t)min(max((y + kNv12VR * v) >> 20, 0), 255);
+  return b | (g << 8) | (r << 16);
+}
+
+// The same conversion split for pixels that share one chroma pair (a 2 x 2 block starting at an even x and y): the
+// three chroma terms once, then per luma value y = nv12_luma(Y) the channels (y + term) >> 20, saturated.  The sums
+// are nv12_bgr's (no term overflows int), so each channel is bit for bit the same.  nv12_sat clamps before the shift,
+// min(max(y + term, 0), 2^28 - 1) >> 20 == min(max((y + term) >> 20, 0), 255), as one fused add / min / relu
+// (VIADDMNMX.RELU, sm_90 and later) and a shift instead of an add, a shift and two min / max.
+__device__ __forceinline__ int nv12_luma(int Y) { return max(Y - 16, 0) * kNv12Y + (1 << 19); }
+__device__ __forceinline__ int3 nv12_chroma(uint32_t uv) {
+  const int u = (int)(uv & 0xffu) - 128, v = (int)(uv >> 8) - 128;
+  return make_int3(kNv12UB * u, -kNv12VG * v - kNv12UG * u, kNv12VR * v);
+}
+__device__ __forceinline__ uint32_t nv12_sat(int y, int term) { return (uint32_t)(__viaddmin_s32_relu(y, term, (1 << 28) - 1) >> 20); }
 #endif

@@ -2,6 +2,7 @@
 // (sinks/kafka_sink.py:93-149, 200-310 of the reference) do to a frame and its tracks before the encoder:
 //
 //   b200va_resize_area_u8   cv2.resize(image, (new_w, new_h), interpolation=cv2.INTER_AREA)        kafka_sink.py:227-232
+//   b200va_resize_area_u8_nv12  the same on cv2.cvtColor(frame, COLOR_YUV2BGR_NV12), converted in the taps
 //   b200va_draw_rects       cv2.rectangle(.., color, 2) and cv2.rectangle(.., color, -1) in order   kafka_sink.py:240, 249-255
 //   b200va_tracks_json      json.dumps(payload) of the track event (host code, no device work)      kafka_sink.py:88, 105-134
 //
@@ -23,6 +24,15 @@ struct AreaEntry {
   int32_t src;   // source column (x table) or row (y table)
   float alpha;   // weight (float32, computed in double and narrowed like OpenCV's DecimateAlpha)
 };
+// what a launch's frames share: one (source, destination) size
+struct AreaGeom {
+  int dst_h, dst_w;
+  int iscale_x, iscale_y;          // integer block (fast path) -- 0 when the general tables are used
+  const int32_t* xofs;             // [dst_w + 1] CSR offsets into xtab
+  const AreaEntry* xtab;
+  const int32_t* yofs;             // [dst_h + 1]
+  const AreaEntry* ytab;
+};
 struct AreaFrame {
   const uint8_t* src;
   uint8_t* dst;
@@ -31,41 +41,113 @@ struct AreaFrame {
 };
 struct AreaParams {
   AreaFrame f[B200VA_LAUNCH_FRAMES];
-  int dst_h, dst_w;
-  int iscale_x, iscale_y;          // integer block (fast path) -- 0 when the general tables are used
-  const int32_t* xofs;             // [dst_w + 1] CSR offsets into xtab
-  const AreaEntry* xtab;
-  const int32_t* yofs;             // [dst_h + 1]
-  const AreaEntry* ytab;
+  AreaGeom g;
+};
+// b200va_resize_area_u8_nv12: the two planes of each frame, each with its own base and pitch
+struct AreaFrameNv12 {
+  const uint8_t* y;
+  const uint8_t* uv;   // src_h / 2 rows of src_w bytes: Cb, Cr of each 2 x 2 block
+  uint8_t* dst;
+  long long y_pitch, uv_pitch;
+  int src_h, src_w;
+};
+struct AreaParamsNv12 {
+  AreaFrameNv12 f[B200VA_LAUNCH_FRAMES];
+  AreaGeom g;
+};
+static_assert(sizeof(AreaParamsNv12) <= 4000, "kernel parameter block too large");
+
+// Source pixel loaders of the INTER_AREA bodies: src.row(y) is source row y, src.block(dx, sx, dy, sy) the same source
+// seen from block (dx, dy) of sx x sy pixels on, and row.px(x, b, g, r) reads pixel x of a row.  Packed BGR: three
+// bytes.  NV12: luma byte x of the row and the Cb, Cr pair at (x & ~1) of its chroma row, converted and saturated per
+// pixel (cv2 converts first and resizes the BGR image), so every sum below adds converted pixels.
+struct BgrRow {
+  const uint8_t* p;
+  __device__ __forceinline__ void px(int x, int& b, int& g, int& r) const {
+    b = p[3 * x];
+    g = p[3 * x + 1];
+    r = p[3 * x + 2];
+  }
+};
+struct BgrSrc {
+  const uint8_t* src;
+  long long pitch;
+  __device__ __forceinline__ BgrSrc(const AreaFrame& f) : src(f.src), pitch(f.pitch) {}
+  __device__ __forceinline__ BgrRow row(int y) const { return BgrRow{src + (long long)y * pitch}; }
+  __device__ __forceinline__ BgrSrc block(int dx, int sx, int dy, int sy) const {
+    return BgrSrc(src + (long long)dy * sy * pitch + (size_t)dx * sx * 3, pitch);
+  }
+  __device__ __forceinline__ BgrSrc(const uint8_t* s, long long p) : src(s), pitch(p) {}
+};
+struct Nv12Row {
+  const uint8_t* y;
+  const uint8_t* uv;
+  int x0;
+  __device__ __forceinline__ void px(int x, int& b, int& g, int& r) const {
+    x += x0;
+    const uint8_t* c = uv + (x & ~1);  // two byte loads: a chroma row may start at any address
+    const uint32_t v = nv12_bgr(y[x], (uint32_t)c[0] | ((uint32_t)c[1] << 8));
+    b = (int)(v & 0xffu);
+    g = (int)((v >> 8) & 0xffu);
+    r = (int)(v >> 16);
+  }
+};
+struct Nv12Src {
+  const uint8_t* y;
+  const uint8_t* uv;
+  long long y_pitch, uv_pitch;
+  int x0 = 0, y0 = 0;  // the chroma pair of a pixel depends on its absolute position
+  __device__ __forceinline__ Nv12Src(const AreaFrameNv12& f) : y(f.y), uv(f.uv), y_pitch(f.y_pitch), uv_pitch(f.uv_pitch) {}
+  __device__ __forceinline__ Nv12Row row(int r) const {
+    r += y0;
+    return Nv12Row{y + (long long)r * y_pitch, uv + (long long)(r >> 1) * uv_pitch, x0};
+  }
+  __device__ __forceinline__ Nv12Src block(int dx, int sx, int dy, int sy) const {
+    Nv12Src s = *this;
+    s.x0 = dx * sx;
+    s.y0 = dy * sy;
+    return s;
+  }
 };
 
 // whole iscale_x x iscale_y source blocks per destination pixel (ResizeAreaFast_).  2 x 2: the vector kernel's
 // (a + b + c + d + 2) >> 2; any other block: saturate_cast<uchar>(sum * (1.f / area)), float multiply, ties to even.
-__global__ void __launch_bounds__(256) k_area_fast(const __grid_constant__ AreaParams p) {
-  const AreaFrame& f = p.f[blockIdx.z];
+template <class Src, class F>
+__device__ __forceinline__ void area_fast_body(const AreaGeom& g, const F& f) {
   const int dx = blockIdx.x * blockDim.x + threadIdx.x, dy = blockIdx.y;
-  if (dx >= p.dst_w) return;
-  const uint8_t* s = f.src + (long long)dy * p.iscale_y * f.pitch + (size_t)dx * p.iscale_x * 3;
+  if (dx >= g.dst_w) return;
+  const Src src = Src(f).block(dx, g.iscale_x, dy, g.iscale_y);
   int sb = 0, sg = 0, sr = 0;
-  for (int y = 0; y < p.iscale_y; ++y) {
-    const uint8_t* row = s + (long long)y * f.pitch;
-    for (int x = 0; x < p.iscale_x; ++x) {
-      sb += row[3 * x];
-      sg += row[3 * x + 1];
-      sr += row[3 * x + 2];
+  for (int y = 0; y < g.iscale_y; ++y) {
+    const auto row = src.row(y);
+    for (int x = 0; x < g.iscale_x; ++x) {
+      int b, gg, r;
+      row.px(x, b, gg, r);
+      sb += b;
+      sg += gg;
+      sr += r;
     }
   }
-  uint8_t* d = f.dst + ((size_t)dy * p.dst_w + dx) * 3;
-  if (p.iscale_x == 2 && p.iscale_y == 2) {
+  uint8_t* d = f.dst + ((size_t)dy * g.dst_w + dx) * 3;
+  if (g.iscale_x == 2 && g.iscale_y == 2) {
     d[0] = (uint8_t)((sb + 2) >> 2);
     d[1] = (uint8_t)((sg + 2) >> 2);
     d[2] = (uint8_t)((sr + 2) >> 2);
   } else {
-    const float scale = 1.f / (float)(p.iscale_x * p.iscale_y);
+    const float scale = 1.f / (float)(g.iscale_x * g.iscale_y);
     d[0] = (uint8_t)min(255, max(0, __float2int_rn(__fmul_rn((float)sb, scale))));
     d[1] = (uint8_t)min(255, max(0, __float2int_rn(__fmul_rn((float)sg, scale))));
     d[2] = (uint8_t)min(255, max(0, __float2int_rn(__fmul_rn((float)sr, scale))));
   }
+}
+
+__global__ void __launch_bounds__(256) k_area_fast(const __grid_constant__ AreaParams p) {
+  area_fast_body<BgrSrc>(p.g, p.f[blockIdx.z]);
+}
+
+// NV12 blocks of any size: 1 x 1 is cv2.cvtColor itself; an odd block may see the chroma pair change inside it
+__global__ void __launch_bounds__(256) k_area_nv12_fast(const __grid_constant__ AreaParamsNv12 p) {
+  area_fast_body<Nv12Src>(p.g, p.f[blockIdx.z]);
 }
 
 // The 2 x 2 case on aligned frames (what a 4K camera sends): a thread owns four destination pixels -- two source rows
@@ -75,7 +157,7 @@ __device__ __forceinline__ uint32_t byte_of(const uint32_t (&w)[6], int i) { ret
 __global__ void __launch_bounds__(256) k_area_2x2_vec(const __grid_constant__ AreaParams p) {
   const AreaFrame& f = p.f[blockIdx.z];
   const int q = blockIdx.x * blockDim.x + threadIdx.x, dy = blockIdx.y;  // q: group of four destination pixels
-  if (q * 4 >= p.dst_w) return;
+  if (q * 4 >= p.g.dst_w) return;
   const uint8_t* s0 = f.src + (long long)(2 * dy) * f.pitch + (size_t)q * 24;
   const uint8_t* s1 = s0 + f.pitch;
   uint32_t a[6], b[6];
@@ -97,7 +179,41 @@ __global__ void __launch_bounds__(256) k_area_2x2_vec(const __grid_constant__ Ar
       o[ob >> 2] |= v << ((ob & 3) * 8);
     }
   }
-  uint32_t* d = reinterpret_cast<uint32_t*>(f.dst + ((size_t)dy * p.dst_w + (size_t)q * 4) * 3);
+  uint32_t* d = reinterpret_cast<uint32_t*>(f.dst + ((size_t)dy * p.g.dst_w + (size_t)q * 4) * 3);
+  __stcs(d, o[0]);
+  __stcs(d + 1, o[1]);
+  __stcs(d + 2, o[2]);
+}
+
+// The 2 x 2 case on aligned NV12 frames (4K -> 1080p): a thread owns four destination pixels and loads 8 bytes each of
+// luma rows 2 dy and 2 dy + 1 and of chroma row dy -- the eight luma columns of its four blocks and their four Cb, Cr
+// pairs.  A block starts at an even x and y, so its four pixels share one pair: the chroma terms are computed once per
+// destination pixel, each of the four pixels is saturated on its own, then (a + b + c + d + 2) >> 2 per channel.
+__global__ void __launch_bounds__(256) k_area_nv12_2x2_vec(const __grid_constant__ AreaParamsNv12 p) {
+  const AreaFrameNv12& f = p.f[blockIdx.z];
+  const int q = blockIdx.x * blockDim.x + threadIdx.x, dy = blockIdx.y;
+  if (q * 4 >= p.g.dst_w) return;
+  const uint8_t* y0 = f.y + (long long)(2 * dy) * f.y_pitch + (size_t)q * 8;
+  const uint2 l0 = __ldcs(reinterpret_cast<const uint2*>(y0));
+  const uint2 l1 = __ldcs(reinterpret_cast<const uint2*>(y0 + f.y_pitch));
+  const uint2 cc = __ldcs(reinterpret_cast<const uint2*>(f.uv + (long long)dy * f.uv_pitch + (size_t)q * 8));
+  uint32_t o[3] = {0u, 0u, 0u};
+#pragma unroll
+  for (int j = 0; j < 4; ++j) {
+    const uint32_t w0 = j < 2 ? l0.x : l0.y, w1 = j < 2 ? l1.x : l1.y, wc = j < 2 ? cc.x : cc.y;
+    const int sh = (j & 1) * 16;  // block j: luma bytes 2j, 2j + 1 of both rows, chroma pair j
+    const int3 t = nv12_chroma((wc >> sh) & 0xffffu);
+    const int ya = nv12_luma((w0 >> sh) & 0xff), yb = nv12_luma((w0 >> (sh + 8)) & 0xff);
+    const int yc = nv12_luma((w1 >> sh) & 0xff), yd = nv12_luma((w1 >> (sh + 8)) & 0xff);
+    const int term[3] = {t.x, t.y, t.z};
+#pragma unroll
+    for (int c = 0; c < 3; ++c) {
+      const uint32_t v = (nv12_sat(ya, term[c]) + nv12_sat(yb, term[c]) + nv12_sat(yc, term[c]) + nv12_sat(yd, term[c]) + 2u) >> 2;
+      const int ob = 3 * j + c;
+      o[ob >> 2] |= v << ((ob & 3) * 8);
+    }
+  }
+  uint32_t* d = reinterpret_cast<uint32_t*>(f.dst + ((size_t)dy * p.g.dst_w + (size_t)q * 4) * 3);
   __stcs(d, o[0]);
   __stcs(d + 1, o[1]);
   __stcs(d + 2, o[2]);
@@ -106,23 +222,25 @@ __global__ void __launch_bounds__(256) k_area_2x2_vec(const __grid_constant__ Ar
 // ResizeArea_<uchar, float>: for every source row of the destination row (y table order) a horizontal float sum in
 // x table order starting from 0, then sum = beta * buf for the first row and sum += beta * buf for the others; no
 // contraction (the file is compiled with -fmad=false and the operations are spelled out).
-__global__ void __launch_bounds__(256) k_area_general(const __grid_constant__ AreaParams p) {
-  const AreaFrame& f = p.f[blockIdx.z];
+template <class Src, class F>
+__device__ __forceinline__ void area_general_body(const AreaGeom& g, const F& f) {
   const int dx = blockIdx.x * blockDim.x + threadIdx.x, dy = blockIdx.y;
-  if (dx >= p.dst_w) return;
-  const int x0 = p.xofs[dx], x1 = p.xofs[dx + 1];
-  const int y0 = p.yofs[dy], y1 = p.yofs[dy + 1];
+  if (dx >= g.dst_w) return;
+  const Src src(f);
+  const int x0 = g.xofs[dx], x1 = g.xofs[dx + 1];
+  const int y0 = g.yofs[dy], y1 = g.yofs[dy + 1];
   float ab = 0.f, ag = 0.f, ar = 0.f;
   for (int j = y0; j < y1; ++j) {
-    const AreaEntry ye = p.ytab[j];
-    const uint8_t* row = f.src + (long long)ye.src * f.pitch;
+    const AreaEntry ye = g.ytab[j];
+    const auto row = src.row(ye.src);
     float bb = 0.f, bg = 0.f, br = 0.f;
     for (int k = x0; k < x1; ++k) {
-      const AreaEntry xe = p.xtab[k];
-      const uint8_t* px = row + (size_t)xe.src * 3;
-      bb = __fadd_rn(bb, __fmul_rn((float)px[0], xe.alpha));
-      bg = __fadd_rn(bg, __fmul_rn((float)px[1], xe.alpha));
-      br = __fadd_rn(br, __fmul_rn((float)px[2], xe.alpha));
+      const AreaEntry xe = g.xtab[k];
+      int b, gg, r;
+      row.px(xe.src, b, gg, r);
+      bb = __fadd_rn(bb, __fmul_rn((float)b, xe.alpha));
+      bg = __fadd_rn(bg, __fmul_rn((float)gg, xe.alpha));
+      br = __fadd_rn(br, __fmul_rn((float)r, xe.alpha));
     }
     if (j == y0) {
       ab = __fmul_rn(ye.alpha, bb);
@@ -134,10 +252,18 @@ __global__ void __launch_bounds__(256) k_area_general(const __grid_constant__ Ar
       ar = __fadd_rn(ar, __fmul_rn(ye.alpha, br));
     }
   }
-  uint8_t* d = f.dst + ((size_t)dy * p.dst_w + dx) * 3;
+  uint8_t* d = f.dst + ((size_t)dy * g.dst_w + dx) * 3;
   d[0] = (uint8_t)min(255, max(0, __float2int_rn(ab)));
   d[1] = (uint8_t)min(255, max(0, __float2int_rn(ag)));
   d[2] = (uint8_t)min(255, max(0, __float2int_rn(ar)));
+}
+
+__global__ void __launch_bounds__(256) k_area_general(const __grid_constant__ AreaParams p) {
+  area_general_body<BgrSrc>(p.g, p.f[blockIdx.z]);
+}
+
+__global__ void __launch_bounds__(256) k_area_nv12_general(const __grid_constant__ AreaParamsNv12 p) {
+  area_general_body<Nv12Src>(p.g, p.f[blockIdx.z]);
 }
 
 // computeResizeAreaTab (resize.cpp), double arithmetic, float weights; CSR per destination index
@@ -266,6 +392,52 @@ void egress_destroy(b200va_ctx* h) {
   h->egress = nullptr;
 }
 
+// The geometry of one (source, destination) size group: cv::resize's integer-block test and, for fractional ratios,
+// the cached x / y tables (they depend on the sizes only, so BGR and NV12 frames share them).  Sets *fast.
+static int area_geom(b200va_ctx* h, int sh, int sw, int dh, int dw, AreaGeom& g, bool* fast) {
+  // cv::resize: inv_scale = dsize / ssize, scale = 1 / inv_scale (double)
+  const double scale_x = 1.0 / ((double)dw / sw), scale_y = 1.0 / ((double)dh / sh);
+  const int iscale_x = (int)std::nearbyint(scale_x), iscale_y = (int)std::nearbyint(scale_y);
+  *fast = std::fabs(scale_x - iscale_x) < 2.220446049250313e-16 && std::fabs(scale_y - iscale_y) < 2.220446049250313e-16;
+  memset(&g, 0, sizeof(g));
+  g.dst_h = dh;
+  g.dst_w = dw;
+  if (*fast) {
+    g.iscale_x = iscale_x;
+    g.iscale_y = iscale_y;
+    return B200VA_OK;
+  }
+  EgressState* e = egress(h);
+  AreaTables& t = e->tables[{{sh, sw}, {dh, dw}}];
+  if (!t.base) {
+    std::vector<int32_t> xo, yo;
+    std::vector<AreaEntry> xt, yt;
+    area_tab(sw, dw, scale_x, xo, xt);
+    area_tab(sh, dh, scale_y, yo, yt);
+    auto al = [](size_t b) { return (b + 255) & ~(size_t)255; };
+    const size_t o1 = al(xo.size() * 4), o2 = o1 + al(xt.size() * sizeof(AreaEntry)), o3 = o2 + al(yo.size() * 4),
+                 total = o3 + al(yt.size() * sizeof(AreaEntry));
+    CUDA_TRY(h, cudaMalloc(&t.base, total));
+    uint8_t* b = (uint8_t*)t.base;
+    t.xofs = (int32_t*)b;
+    t.xtab = (AreaEntry*)(b + o1);
+    t.yofs = (int32_t*)(b + o2);
+    t.ytab = (AreaEntry*)(b + o3);
+    // (synchronous copies: the tables of a geometry are built once)
+    CUDA_TRY(h, cudaMemcpy(t.xofs, xo.data(), xo.size() * 4, cudaMemcpyHostToDevice));
+    CUDA_TRY(h, cudaMemcpy(t.xtab, xt.data(), xt.size() * sizeof(AreaEntry), cudaMemcpyHostToDevice));
+    CUDA_TRY(h, cudaMemcpy(t.yofs, yo.data(), yo.size() * 4, cudaMemcpyHostToDevice));
+    CUDA_TRY(h, cudaMemcpy(t.ytab, yt.data(), yt.size() * sizeof(AreaEntry), cudaMemcpyHostToDevice));
+  }
+  g.xofs = t.xofs;
+  g.xtab = t.xtab;
+  g.yofs = t.yofs;
+  g.ytab = t.ytab;
+  return B200VA_OK;
+}
+
+using AreaGroups = std::map<std::pair<std::pair<int, int>, std::pair<int, int>>, std::vector<int>>;
+
 extern "C" int b200va_resize_area_u8(b200va_handle h, const uint8_t* const* frames, const int* src_h, const int* src_w,
                                      const int64_t* src_pitch, int batch, uint8_t* const* dst, const int* dst_h,
                                      const int* dst_w, void* stream) {
@@ -277,7 +449,7 @@ extern "C" int b200va_resize_area_u8(b200va_handle h, const uint8_t* const* fram
   cudaStream_t st = (cudaStream_t)stream;
   PhaseScope phase(h, B200VA_PHASE_EGRESS, st);
   // frames that share source and destination size go out in one launch
-  std::map<std::pair<std::pair<int, int>, std::pair<int, int>>, std::vector<int>> groups;
+  AreaGroups groups;
   for (int b = 0; b < batch; ++b) {
     REQUIRE(h, frames[b] && dst[b], "frame %d: NULL pointer", b);
     REQUIRE(h, src_h[b] > 0 && src_w[b] > 0 && dst_h[b] > 0 && dst_w[b] > 0, "frame %d: bad size", b);
@@ -288,45 +460,11 @@ extern "C" int b200va_resize_area_u8(b200va_handle h, const uint8_t* const* fram
   }
   for (const auto& kv : groups) {
     const int sh = kv.first.first.first, sw = kv.first.first.second, dh = kv.first.second.first, dw = kv.first.second.second;
-    // cv::resize: inv_scale = dsize / ssize, scale = 1 / inv_scale (double)
-    const double scale_x = 1.0 / ((double)dw / sw), scale_y = 1.0 / ((double)dh / sh);
-    const int iscale_x = (int)std::nearbyint(scale_x), iscale_y = (int)std::nearbyint(scale_y);
-    const bool fast = std::fabs(scale_x - iscale_x) < 2.220446049250313e-16 && std::fabs(scale_y - iscale_y) < 2.220446049250313e-16;
     AreaParams p;
     memset(&p, 0, sizeof(p));
-    p.dst_h = dh;
-    p.dst_w = dw;
-    if (fast) {
-      p.iscale_x = iscale_x;
-      p.iscale_y = iscale_y;
-    } else {
-      EgressState* e = egress(h);
-      AreaTables& t = e->tables[kv.first];
-      if (!t.base) {
-        std::vector<int32_t> xo, yo;
-        std::vector<AreaEntry> xt, yt;
-        area_tab(sw, dw, scale_x, xo, xt);
-        area_tab(sh, dh, scale_y, yo, yt);
-        auto al = [](size_t b) { return (b + 255) & ~(size_t)255; };
-        const size_t o1 = al(xo.size() * 4), o2 = o1 + al(xt.size() * sizeof(AreaEntry)), o3 = o2 + al(yo.size() * 4),
-                     total = o3 + al(yt.size() * sizeof(AreaEntry));
-        CUDA_TRY(h, cudaMalloc(&t.base, total));
-        uint8_t* b = (uint8_t*)t.base;
-        t.xofs = (int32_t*)b;
-        t.xtab = (AreaEntry*)(b + o1);
-        t.yofs = (int32_t*)(b + o2);
-        t.ytab = (AreaEntry*)(b + o3);
-        // (synchronous copies: the tables of a geometry are built once)
-        CUDA_TRY(h, cudaMemcpy(t.xofs, xo.data(), xo.size() * 4, cudaMemcpyHostToDevice));
-        CUDA_TRY(h, cudaMemcpy(t.xtab, xt.data(), xt.size() * sizeof(AreaEntry), cudaMemcpyHostToDevice));
-        CUDA_TRY(h, cudaMemcpy(t.yofs, yo.data(), yo.size() * 4, cudaMemcpyHostToDevice));
-        CUDA_TRY(h, cudaMemcpy(t.ytab, yt.data(), yt.size() * sizeof(AreaEntry), cudaMemcpyHostToDevice));
-      }
-      p.xofs = t.xofs;
-      p.xtab = t.xtab;
-      p.yofs = t.yofs;
-      p.ytab = t.ytab;
-    }
+    bool fast = false;
+    const int rc = area_geom(h, sh, sw, dh, dw, p.g, &fast);
+    if (rc) return rc;
     const std::vector<int>& idx = kv.second;
     for (size_t base = 0; base < idx.size(); base += B200VA_LAUNCH_FRAMES) {
       const int n = (int)std::min<size_t>(B200VA_LAUNCH_FRAMES, idx.size() - base);
@@ -335,12 +473,64 @@ extern "C" int b200va_resize_area_u8(b200va_handle h, const uint8_t* const* fram
         p.f[i] = AreaFrame{frames[b], dst[b], src_pitch ? (long long)src_pitch[b] : 3ll * sw, sh, sw};
       }
       const dim3 grid((dw + 255) / 256, dh, n);
-      bool vec = fast && iscale_x == 2 && iscale_y == 2 && dw % 4 == 0;
+      bool vec = fast && p.g.iscale_x == 2 && p.g.iscale_y == 2 && dw % 4 == 0;
       for (int i = 0; i < n && vec; ++i)
         vec = ((uintptr_t)p.f[i].src % 8 == 0) && (p.f[i].pitch % 8 == 0) && ((uintptr_t)p.f[i].dst % 4 == 0);
       if (vec) k_area_2x2_vec<<<dim3((dw / 4 + 255) / 256, dh, n), 256, 0, st>>>(p);
       else if (fast) k_area_fast<<<grid, 256, 0, st>>>(p);
       else k_area_general<<<grid, 256, 0, st>>>(p);
+      LAUNCH_CHECK(h);
+    }
+  }
+  return B200VA_OK;
+}
+
+extern "C" int b200va_resize_area_u8_nv12(b200va_handle h, const b200va_nv12_frame* frames, const int* src_h,
+                                          const int* src_w, int batch, uint8_t* const* dst, const int* dst_h,
+                                          const int* dst_w, void* stream) {
+  if (!h) return B200VA_ERR_INVALID;
+  std::lock_guard<std::recursive_mutex> lock(h->mu);
+  DeviceGuard guard(h->cfg.device);
+  REQUIRE(h, frames && src_h && src_w && dst && dst_h && dst_w, "NULL argument");
+  REQUIRE(h, batch >= 0 && batch <= h->cfg.max_batch, "batch %d outside [0, %d]", batch, h->cfg.max_batch);
+  cudaStream_t st = (cudaStream_t)stream;
+  PhaseScope phase(h, B200VA_PHASE_EGRESS, st);
+  AreaGroups groups;
+  for (int b = 0; b < batch; ++b) {
+    const b200va_nv12_frame& n = frames[b];
+    REQUIRE(h, n.y && n.uv, "frame %d: NULL plane", b);
+    REQUIRE(h, dst[b], "dst %d is NULL", b);
+    REQUIRE(h, src_h[b] > 0 && src_w[b] > 0 && dst_h[b] > 0 && dst_w[b] > 0, "frame %d: bad size", b);
+    REQUIRE(h, src_h[b] % 2 == 0 && src_w[b] % 2 == 0, "frame %d: NV12 needs an even size, got %dx%d", b, src_w[b], src_h[b]);
+    REQUIRE(h, n.y_pitch >= src_w[b] && n.uv_pitch >= src_w[b], "frame %d: plane pitch %lld / %lld < width %d", b,
+            (long long)n.y_pitch, (long long)n.uv_pitch, src_w[b]);
+    REQUIRE(h, dst_h[b] <= src_h[b] && dst_w[b] <= src_w[b], "frame %d: INTER_AREA is implemented for shrinking only (%dx%d -> %dx%d)", b,
+            src_w[b], src_h[b], dst_w[b], dst_h[b]);
+    REQUIRE(h, dst_h[b] < 65536, "frame %d: destination too tall", b);
+    groups[{{src_h[b], src_w[b]}, {dst_h[b], dst_w[b]}}].push_back(b);
+  }
+  for (const auto& kv : groups) {
+    const int sh = kv.first.first.first, sw = kv.first.first.second, dh = kv.first.second.first, dw = kv.first.second.second;
+    AreaParamsNv12 p;
+    memset(&p, 0, sizeof(p));
+    bool fast = false;
+    const int rc = area_geom(h, sh, sw, dh, dw, p.g, &fast);
+    if (rc) return rc;
+    const std::vector<int>& idx = kv.second;
+    for (size_t base = 0; base < idx.size(); base += B200VA_LAUNCH_FRAMES) {
+      const int n = (int)std::min<size_t>(B200VA_LAUNCH_FRAMES, idx.size() - base);
+      bool vec = fast && p.g.iscale_x == 2 && p.g.iscale_y == 2 && dw % 4 == 0;
+      for (int i = 0; i < n; ++i) {
+        const int b = idx[base + i];
+        const b200va_nv12_frame& s = frames[b];
+        p.f[i] = AreaFrameNv12{s.y, s.uv, dst[b], (long long)s.y_pitch, (long long)s.uv_pitch, sh, sw};
+        vec = vec && (uintptr_t)s.y % 8 == 0 && (uintptr_t)s.uv % 8 == 0 && s.y_pitch % 8 == 0 && s.uv_pitch % 8 == 0 &&
+              (uintptr_t)dst[b] % 4 == 0;
+      }
+      const dim3 grid((dw + 255) / 256, dh, n);
+      if (vec) k_area_nv12_2x2_vec<<<dim3((dw / 4 + 255) / 256, dh, n), 256, 0, st>>>(p);
+      else if (fast) k_area_nv12_fast<<<grid, 256, 0, st>>>(p);
+      else k_area_nv12_general<<<grid, 256, 0, st>>>(p);
       LAUNCH_CHECK(h);
     }
   }

@@ -426,18 +426,6 @@ struct PreParamsNv12 {
 };
 static_assert(sizeof(PreParamsNv12) <= 4000, "kernel parameter block too large");
 
-// cv::cvtColor YUV2BGR_NV12 (modules/imgproc/src/color_yuv.simd.hpp, 8-bit path): ITU-R BT.601 limited range in
-// 20-bit fixed point, rounded by the 1 << 19 bias and saturated.  `uv` = Cb | Cr << 8 of the pixel's 2 x 2 block.
-// Returns the pixel packed as B | G << 8 | R << 16 (byte 3 is zero).
-__device__ __forceinline__ uint32_t nv12_bgr(int Y, uint32_t uv) {
-  const int y = max(Y - 16, 0) * 1220542 + (1 << 19);
-  const int u = (int)(uv & 0xffu) - 128, v = (int)(uv >> 8) - 128;
-  const uint32_t b = (uint32_t)min(max((y + 2116026 * u) >> 20, 0), 255);
-  const uint32_t g = (uint32_t)min(max((y - 852492 * v - 409993 * u) >> 20, 0), 255);
-  const uint32_t r = (uint32_t)min(max((y + 1673527 * v) >> 20, 0), 255);
-  return b | (g << 8) | (r << 16);
-}
-
 // pixel x of a staged luma row and its chroma row (chroma rows start 128-byte aligned: the pair load is aligned)
 __device__ __forceinline__ uint32_t nv12_tap(const uint8_t* __restrict__ yr, const uint8_t* __restrict__ cr, int x) {
   return nv12_bgr(yr[x], *reinterpret_cast<const uint16_t*>(cr + (x & ~1)));

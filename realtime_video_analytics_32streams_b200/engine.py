@@ -34,14 +34,6 @@ from .types import Detection, MotionFilterConfig, Track
 LOGGER = logging.getLogger(__name__)
 
 
-def _hw(frame):
-    """(height, width) of a BGR [H, W, 3] frame or of an NV12 frame's luma."""
-    if _native.is_nv12(frame):
-        y, _ = _native.nv12_planes(frame)
-        return int(y.shape[0]), int(y.shape[1])
-    return int(frame.shape[0]), int(frame.shape[1])
-
-
 @dataclass
 class _StreamState:
     """Host-side gate state of one stream (pipeline.py:88-116)."""
@@ -282,7 +274,7 @@ class HotPathEngine:
     def _pads_flag(self, frames) -> int:
         """B200VA_OUT_FLAG_PADS_VALID when every batch position was last written from a frame of the same size
         (same letterbox geometry, same format): its pad rows are already in the persistent buffer."""
-        shapes = [_hw(f) for f in frames]
+        shapes = [_native.frame_hw(f) for f in frames]
         valid = all(self._net_shapes[k] == sh for k, sh in enumerate(shapes))
         for k, sh in enumerate(shapes):
             self._net_shapes[k] = sh
@@ -326,13 +318,13 @@ class HotPathEngine:
         masks, ratios = [], []
         for st, f in zip(states, dev_frames):
             polys = getattr(st.cfg, "roi_polygons", None) or []
-            masks.append(roi_mask(polys, *_hw(f), self.h) if polys else None)
+            masks.append(roi_mask(polys, *_native.frame_hw(f), self.h) if polys else None)
             ratios.append(float(getattr(st.cfg, "downsample_ratio", 1.0)))
         down = [k for k, r in enumerate(ratios) if r < 0.999]
         work = list(dev_frames)
         work_masks = list(masks)
         if down:
-            sizes = {k: (int(_hw(dev_frames[k])[0] * ratios[k]), int(_hw(dev_frames[k])[1] * ratios[k])) for k in down}
+            sizes = {k: tuple(int(v * ratios[k]) for v in _native.frame_hw(dev_frames[k])) for k in down}
             # NV12 frames are converted in the same taps (resize_linear_u8_nv12); one call per source format
             for group in ([k for k in down if not _native.is_nv12(dev_frames[k])], [k for k in down if _native.is_nv12(dev_frames[k])]):
                 if not group:
@@ -349,8 +341,8 @@ class HotPathEngine:
         # persistent per-stream buffer, which the letterbox then reads too
         cvt = [k for k in mot if _native.is_nv12(work[k])]
         if cvt:
-            outs = [self._bgr_buffer(live[k], _hw(work[k]), full=True) for k in cvt]
-            full = self.h.resize([work[k] for k in cvt], [_hw(work[k]) for k in cvt], outs=outs)
+            outs = [self._bgr_buffer(live[k], _native.frame_hw(work[k]), full=True) for k in cvt]
+            full = self.h.resize([work[k] for k in cvt], [_native.frame_hw(work[k]) for k in cvt], outs=outs)
             for k, f in zip(cvt, full):
                 work[k] = f
         if self.device_gates:
@@ -445,7 +437,8 @@ class HotPathEngine:
             g.max_process_every = max(st.max_process_every, 1)
             g.idle_tolerance = max(st.idle_tolerance, 1)
             g.motion_threshold = float(st.cfg.motion_threshold) if k in where else 0.0
-            g.pixels = _hw(work[k])[0] * _hw(work[k])[1]
+            fh, fw = _native.frame_hw(work[k])
+            g.pixels = fh * fw
         skip = ctx.skip[:nb]
         h.gates_decide(gates, changed, skip)
         dets = {k_: v[:nb] for k_, v in ctx.dets.items() if not k_.startswith("_")}

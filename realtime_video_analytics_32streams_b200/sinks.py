@@ -23,6 +23,7 @@ from __future__ import annotations
 import asyncio
 import base64
 import logging
+import threading
 import time
 from typing import Dict, Iterable, List, Optional, Sequence, Tuple
 
@@ -104,6 +105,7 @@ class PreviewRenderer:
         self._bufs: Dict[tuple, tuple] = {}   # (h, w) -> (device preview, pinned host mirror)
         self._label_sizes: Dict[str, Tuple[int, int, int]] = {}
         self.replayed = 0                    # frames whose overlay had to be replayed in order on the host
+        self._lock = threading.Lock()
 
     def _label_size(self, label: str) -> Tuple[int, int, int]:
         s = self._label_sizes.get(label)
@@ -123,26 +125,34 @@ class PreviewRenderer:
         return b
 
     def render(self, frame, track_list: Sequence[dict]) -> np.ndarray:
-        """``frame``: host ndarray [H, W, 3] uint8 (uploaded whole) or CUDA uint8 tensor; ``track_list``: the dicts of
-        kafka_sink.py:105-123 (``track_id``, ``class_id``, ``bbox_xyxy``).  Returns the annotated preview the reference
-        would hand to ``cv2.imencode``."""
+        """``frame``: host ndarray [H, W, 3] uint8 (uploaded whole) or CUDA uint8 tensor, or an NV12 frame as
+        ``HotPathEngine`` takes it -- a host ``[3H/2, W]`` array / CPU tensor (uploaded whole, 1.5 bytes per pixel), a
+        CUDA ``[3H/2, W]`` tensor or a ``(y, uv)`` pair of CUDA planes; ``track_list``: the dicts of kafka_sink.py:105-123
+        (``track_id``, ``class_id``, ``bbox_xyxy``).  Returns the annotated preview the reference would hand to
+        ``cv2.imencode`` (for NV12: the one it would for ``cv2.cvtColor(frame, COLOR_YUV2BGR_NV12)``)."""
         cv2, t = self.cv2, self.h.torch
-        dev = frame if (hasattr(frame, "is_cuda") and frame.is_cuda) else self._stager.upload([frame])[0]
-        fh, fw = int(dev.shape[0]), int(dev.shape[1])
-        sf, nw, nh = preview_geometry(fh, fw)
-        img_dev, img_host = self._buffers(nh, nw)
-        if (nh, nw) != (fh, fw):
-            self.h.resize_area([dev], [(nh, nw)], outs=[img_dev])
-        else:
-            img_dev.copy_(dev)  # image = frame.copy() (kafka_sink.py:220)
-        ops, texts, conflict = overlay_plan(track_list, sf, self._label_size)
-        if not conflict and ops:
-            self.h.draw_rects([img_dev], [ops])
-        img_host.copy_(img_dev, non_blocking=True)
-        t.cuda.current_stream().synchronize()
-        image = img_host.numpy()
+        # B200KafkaSink renders in worker threads (send_tracks -> asyncio.to_thread), and frames of one size share the
+        # staging and preview buffers: one render at a time uses them, and the host image leaves as a private copy
+        with self._lock:
+            on_device = isinstance(frame, (tuple, list)) or (hasattr(frame, "is_cuda") and frame.is_cuda)
+            dev = frame if on_device else self._stager.upload([frame])[0]
+            fh, fw = _native.frame_hw(dev)
+            sf, nw, nh = preview_geometry(fh, fw)
+            img_dev, img_host = self._buffers(nh, nw)
+            # NV12 is converted in the INTER_AREA taps, at the frame's own size too (there the call is cv2.cvtColor)
+            if (nh, nw) != (fh, fw) or _native.is_nv12(dev):
+                self.h.resize_area([dev], [(nh, nw)], outs=[img_dev])
+            else:
+                img_dev.copy_(dev)  # image = frame.copy() (kafka_sink.py:220)
+            ops, texts, conflict = overlay_plan(track_list, sf, self._label_size)
+            if not conflict and ops:
+                self.h.draw_rects([img_dev], [ops])
+            img_host.copy_(img_dev, non_blocking=True)
+            t.cuda.current_stream().synchronize()
+            image = img_host.numpy().copy()
+            if conflict:
+                self.replayed += 1
         if conflict:
-            self.replayed += 1
             for (kind, x1, y1, x2, y2, color), k in zip(ops, range(len(ops))):
                 cv2.rectangle(image, (x1, y1), (x2, y2), color, -1 if kind else 2)
                 if kind:  # the label follows its background (kafka_sink.py:258-267)
