@@ -349,7 +349,11 @@ B200VA_API int b200va_postprocess(b200va_handle h, const void* head, int layout,
  * [batch, 4*reg_max + num_classes, A]; level_hw HOST [n_levels][2] grid sizes (80x80, 40x40, 20x20 at
  * 640x640), level_stride HOST [n_levels] (8, 16, 32); out DEVICE float32 [batch, 4 + num_classes, A]
  * with A = sum(h*w): rows 0-3 = (cx, cy, w, h) in input pixels, rows 4.. = sigmoid(class logits).
- * Floating point (exp): matches a float32 reference within 1e-5 relative; not bit-exact. */
+ * Floating point (exp), not bit-exact: every output is within a bound derived from the float32 operation
+ * order of the float64 decode of the same inputs (tests/dfl_bound.py).  A side with a NaN or +inf bin, or
+ * only -inf bins, decodes to NaN in its two outputs (l, r: cx and w; t, b: cy and h).
+ * Refuses (B200VA_ERR_INVALID) NULL pointers, batch or num_classes < 0, reg_max outside [1, 64], n_levels
+ * outside [1, 8], a level with h or w <= 0, and more than INT_MAX anchors in all. */
 B200VA_API int b200va_dfl_decode(b200va_handle h, const float* raw, int batch, int num_classes, int reg_max,
                                  const int* level_hw, const float* level_stride, int n_levels, float* out,
                                  void* stream);

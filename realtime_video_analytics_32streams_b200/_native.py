@@ -779,15 +779,22 @@ class Handle:
     # -- a14 --------------------------------------------------------------------------------
     def dfl_decode(self, raw, num_classes: int, reg_max: int = 16, levels=((80, 80), (40, 40), (20, 20)),
                    strides=(8.0, 16.0, 32.0), out=None):
-        """Raw Detect head [B, 4*reg_max + nc, A] -> decoded [B, 4 + nc, A] (tolerance-level parity)."""
+        """Raw Detect head [B, 4*reg_max + nc, A] -> decoded [B, 4 + nc, A] (within a derived float32 error bound of
+        the float64 decode, tests/dfl_bound.py)."""
         t = self.torch
         b = raw.shape[0]
         a = sum(h * w for h, w in levels)
+        if len(strides) != len(levels):
+            raise ValueError("dfl_decode: one stride per level")
         if not (raw.is_cuda and raw.dtype == t.float32 and raw.is_contiguous()
                 and tuple(raw.shape) == (b, 4 * reg_max + num_classes, a)):
             raise ValueError("raw must be a contiguous CUDA float32 tensor [B, 4*reg_max + nc, sum(h*w)]")
         if out is None:
             out = t.empty((b, 4 + num_classes, a), dtype=t.float32, device=self.device)
+        elif not (out.is_cuda and out.device == self.device and out.dtype == t.float32 and out.is_contiguous()
+                  and tuple(out.shape) == (b, 4 + num_classes, a)):
+            raise ValueError("dfl_decode: `out` must be a contiguous float32 tensor [B, 4 + nc, sum(h*w)] on the "
+                             "handle's device")
         hw = _int_array([v for lv in levels for v in lv])
         st = (C.c_float * len(strides))(*[float(s) for s in strides])
         self._check(self.lib.b200va_dfl_decode(self._h, C.c_void_p(raw.data_ptr()), b, int(num_classes), int(reg_max),

@@ -8,8 +8,11 @@
 //   x1y1 = anchor - (l, t), x2y2 = anchor + (r, b);  (cx, cy) = (x1y1 + x2y2) / 2, (w, h) = x2y2 - x1y1;
 //   all four times the level's stride;  class scores = sigmoid(logits).
 // Output [B, 4 + nc, A] is exactly what b200va_postprocess reads (channel major).  Floating point with
-// exp: parity is tolerance based (1e-5 relative, oracle/dfl.py), "parity unpinned" by the reference.
+// exp: compared with the float64 decode (oracle/dfl.py) under an error bound derived from the float32
+// operation order below (tests/dfl_bound.py), "parity unpinned" by the reference.
 // HBM bound: (4*reg_max + nc) * A * 4 bytes read + (4 + nc) * A * 4 written per frame (7.7 MB at nc = 80).
+#include <climits>
+
 #include "common.cuh"
 
 namespace {
@@ -166,26 +169,28 @@ extern "C" int b200va_dfl_decode(b200va_handle h, const float* raw, int batch, i
   if (batch == 0) return B200VA_OK;
   DflParams p;
   memset(&p, 0, sizeof(p));
-  int total = 0;
+  // the kernel's anchor indices are int: count in 64 bits and refuse what would wrap
+  int64_t total = 0;
   for (int l = 0; l < n_levels; ++l) {
     REQUIRE(h, level_hw[2 * l] > 0 && level_hw[2 * l + 1] > 0, "level %d has an empty grid", l);
-    p.off[l] = total;
+    p.off[l] = (int)total;
     p.w[l] = level_hw[2 * l + 1];
     p.stride[l] = level_stride[l];
-    total += level_hw[2 * l] * level_hw[2 * l + 1];
+    total += (int64_t)level_hw[2 * l] * level_hw[2 * l + 1];
+    REQUIRE(h, total <= INT_MAX, "more than %d anchors", INT_MAX);
   }
-  p.off[n_levels] = total;
+  p.off[n_levels] = (int)total;
   p.raw = raw;
   p.out = out;
   p.nc = num_classes;
   p.reg_max = reg_max;
-  p.A = total;
+  p.A = (int)total;
   p.n_levels = n_levels;
   PhaseScope phase(h, B200VA_PHASE_DFL, (cudaStream_t)stream);
   // four anchors per thread when every channel row starts 16-byte aligned
   const bool vec = total % 4 == 0 && (uintptr_t)raw % 16 == 0 && (uintptr_t)out % 16 == 0;
   const int per_block = 128 * (vec ? 4 : 1);
-  dim3 grid((total + per_block - 1) / per_block, batch, 1 + (num_classes + kClsRows - 1) / kClsRows);
+  dim3 grid((unsigned)((total + per_block - 1) / per_block), batch, 1 + (num_classes + kClsRows - 1) / kClsRows);
   cudaStream_t st = (cudaStream_t)stream;
   if (reg_max == 16) {
     if (vec) k_dfl_decode<16, 4><<<grid, 128, 0, st>>>(p);
