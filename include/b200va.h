@@ -445,6 +445,26 @@ B200VA_API int b200va_preprocess_geom(b200va_handle h, const uint8_t* const* fra
                                       const int64_t* src_pitch, int batch, const uint8_t* const* roi_masks,
                                       const b200va_letterbox* geom, void* out, int dst_h, int dst_w, int out_format,
                                       void* stream);
+/* b200va_preprocess_geom for NV12 frames (b200va_nv12_frame, below): the letterbox of b200va_preprocess_nv12 with the
+ * caller's geometry, byte-identical to b200va_preprocess_geom on cv2.cvtColor(frame, COLOR_YUV2BGR_NV12).  The checks of
+ * both calls apply: the geometry matches each frame and fits the canvas; odd sizes and NULL planes are refused. */
+B200VA_API int b200va_preprocess_geom_nv12(b200va_handle h, const b200va_nv12_frame* frames, const int* src_h,
+                                           const int* src_w, int batch, const uint8_t* const* roi_masks,
+                                           const b200va_letterbox* geom, void* out, int dst_h, int dst_w, int out_format,
+                                           void* stream);
+/* b200va_upload_frames / b200va_upload_frames_nv12 in rows mode 1 for frames that b200va_preprocess_geom* letterboxes
+ * with the caller's geometry: geom HOST [batch] (geom[i].src_h / src_w must be the frame's size) instead of dst_h /
+ * dst_w.  Only the rows the letterbox to geom[i].new_h rows reads cross the bus (NV12: those luma rows and the chroma
+ * rows they use); the LetterBox geometry of b200va_letterbox_meta_ultralytics rounds new_h where the reference
+ * geometry truncates it, so it can read rows the reference-geometry upload skips.  Rows that need more than eight
+ * strided copies, or more than 80 % of a plane, go whole; bytes_copied receives the bytes put on the bus. */
+B200VA_API int b200va_upload_frames_geom(b200va_handle h, const uint8_t* const* host_frames, uint8_t* const* dev_frames,
+                                         const int* src_h, const int* src_w, const int64_t* host_pitch,
+                                         const int64_t* dev_pitch, int batch, const b200va_letterbox* geom,
+                                         int64_t* bytes_copied, void* stream);
+B200VA_API int b200va_upload_frames_nv12_geom(b200va_handle h, const b200va_nv12_frame* host, const b200va_nv12_frame* dev,
+                                              const int* src_h, const int* src_w, int batch, const b200va_letterbox* geom,
+                                              int64_t* bytes_copied, void* stream);
 /* ops.non_max_suppression + ops.scale_boxes for a decoded head [B, 4 + nc, A] / [B, A, 4 + nc]:
  * score_k = head[4 + k], candidate iff max_k > conf_thr (strict, float32); xywh -> xyxy in network-input pixels;
  * NMS on boxes shifted by class * 7680 in float32 (agnostic != 0: no shift) with torchvision's test
@@ -530,6 +550,20 @@ B200VA_API int b200va_tick(b200va_handle h, const b200va_tick_args* args, void* 
  * descriptors; args->frames and args->src_pitch are not read.  Every schedule, graph capture included; the results
  * are those of b200va_tick on the frames converted by cv2.cvtColor(frame, COLOR_YUV2BGR_NV12). */
 B200VA_API int b200va_tick_nv12(b200va_handle h, const b200va_tick_args* args, const b200va_nv12_frame* frames, void* stream);
+/* b200va_tick with Ultralytics semantics: the letterbox half is b200va_preprocess_geom (BGR, frames == NULL) or
+ * b200va_preprocess_geom_nv12 (frames: HOST [args->batch] NV12 plane descriptors) with u->geom, the post half is
+ * b200va_postprocess_ultralytics with u->src_h / src_w / in_h / in_w / agnostic / max_det, and the tracker half is
+ * unchanged.  args->meta, args->score_mode and args->nms_mode are not read, and args->meta_out is not written.  Every
+ * schedule, graph capture and the skip mask included; the results are those of the three separate calls. */
+typedef struct b200va_tick_ultra {
+  const b200va_letterbox* geom; /* HOST [args->batch] letterbox geometry of each frame (b200va_letterbox_meta_ultralytics) */
+  const int* src_h;             /* HOST [args->head_batch] original frame sizes of the head's frames (scale_boxes)    */
+  const int* src_w;
+  int in_h, in_w;               /* network-input shape the head was computed from                                   */
+  int agnostic, max_det;
+} b200va_tick_ultra;
+B200VA_API int b200va_tick_ultralytics(b200va_handle h, const b200va_tick_args* args, const b200va_tick_ultra* u,
+                                       const b200va_nv12_frame* frames /* NULL = BGR */, void* stream);
 
 /* ---- 8f-3: egress (the preview and the event the sink publishes) -------------------------------
  * Replaces, for a frame that is already in HBM, the pixel work of KafkaSink._render_frame

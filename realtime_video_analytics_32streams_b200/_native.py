@@ -104,6 +104,13 @@ class TickArgs(C.Structure):
     ]
 
 
+class TickUltra(C.Structure):
+    """``b200va_tick_ultra`` (include/b200va.h): the Ultralytics halves of ``b200va_tick_ultralytics``."""
+
+    _fields_ = [("geom", C.POINTER(Letterbox)), ("src_h", C.POINTER(C.c_int)), ("src_w", C.POINTER(C.c_int)),
+                ("in_h", C.c_int), ("in_w", C.c_int), ("agnostic", C.c_int), ("max_det", C.c_int)]
+
+
 SCHEDULE_SERIAL, SCHEDULE_PRE_AFTER_DECODE, SCHEDULE_PRE_PARALLEL, SCHEDULE_PRE_BESIDE_DECODE = 0, 1, 2, 3
 SCHEDULE_PRE_BEHIND_DECODE = 5  # like 3, the letterbox waits for the decode grid to drain (griddepcontrol.wait)
 SCHEDULE_AUTO = 6  # 3 for large sparse batches, 1 for small batches and dense scenes (the default; include/b200va.h)
@@ -118,6 +125,7 @@ class TickPlan:
         self.args = args
         self._keep = keep  # owners of every pointer inside `args`
         self.nv12 = None   # Nv12Frame array: the letterbox reads NV12 frames (b200va_tick_nv12)
+        self.ultra = None  # TickUltra: Ultralytics semantics (b200va_tick_ultralytics)
 
     def set_events(self, begin=None, end=None) -> None:
         """Optional (already recorded once) ``torch.cuda.Event`` pair around the letterbox launch."""
@@ -136,7 +144,8 @@ EXPORTS = (
     "b200va_read_status_async", "b200va_resize_area_u8", "b200va_draw_rects", "b200va_tracks_json",
     "b200va_gates_decide", "b200va_gates_commit", "b200va_gates_reset", "b200va_set_skip_mask",
     "b200va_preprocess_nv12", "b200va_resize_linear_u8_nv12", "b200va_upload_frames_nv12", "b200va_tick_nv12",
-    "b200va_resize_area_u8_nv12",
+    "b200va_resize_area_u8_nv12", "b200va_preprocess_geom_nv12", "b200va_upload_frames_geom",
+    "b200va_upload_frames_nv12_geom", "b200va_tick_ultralytics",
 )
 PHASES = ("upload", "roi", "resize", "motion", "preprocess", "decode", "nms", "tracker", "dfl", "tick", "egress")  # enum b200va_phase
 
@@ -211,6 +220,11 @@ def load_library() -> C.CDLL:
     lib.b200va_upload_frames_nv12.argtypes = [vp, nv, nv, ip, ip, C.c_int, C.c_int, C.c_int, C.c_int, i64p, vp]
     lib.b200va_tick_nv12.argtypes = [vp, C.POINTER(TickArgs), nv, vp]
     lib.b200va_resize_area_u8_nv12.argtypes = [vp, nv, ip, ip, C.c_int, C.POINTER(vp), ip, ip, vp]
+    lb = C.POINTER(Letterbox)
+    lib.b200va_preprocess_geom_nv12.argtypes = [vp, nv, ip, ip, C.c_int, C.POINTER(vp), lb, vp, C.c_int, C.c_int, C.c_int, vp]
+    lib.b200va_upload_frames_geom.argtypes = [vp, C.POINTER(vp), C.POINTER(vp), ip, ip, i64p, i64p, C.c_int, lb, i64p, vp]
+    lib.b200va_upload_frames_nv12_geom.argtypes = [vp, nv, nv, ip, ip, C.c_int, lb, i64p, vp]
+    lib.b200va_tick_ultralytics.argtypes = [vp, C.POINTER(TickArgs), C.POINTER(TickUltra), nv, vp]
     lib.b200va_tracks_json.restype = C.c_int64
     lib.b200va_tracks_json.argtypes = [C.c_char_p, C.c_int64, vp, vp, vp, vp, C.c_int, C.c_char_p, vp, C.c_int64]
     for name in EXPORTS:
@@ -475,20 +489,35 @@ class Handle:
                 return FrameBatch(frames, roi_masks)
             frames = Nv12Batch(frames, roi_masks) if nv12_ok else frames
         if not nv12_ok:
-            raise ValueError("NV12 frames are taken by preprocess, resize, resize_area and plan_tick; convert them "
+            raise ValueError("NV12 frames are taken by preprocess, preprocess_geom, resize, resize_area and plan_tick; "
+                             "convert them "
                              "with resize at their own size for the other calls")
         return frames
 
     # -- staging ----------------------------------------------------------------------------
-    def upload_frames(self, host_ptrs, dev_frames, sparse_for=None) -> int:
+    @staticmethod
+    def _geom_array(geoms, n: int):
+        if len(geoms) != n:
+            raise ValueError("one letterbox geometry per frame")
+        return geoms if isinstance(geoms, C.Array) else (Letterbox * max(n, 1))(*geoms)
+
+    def upload_frames(self, host_ptrs, dev_frames, sparse_for=None, geoms=None) -> int:
         """Asynchronous host -> device copy of decoded frames.  ``host_ptrs[i]`` = (address, pitch) of
         frame i in host memory (pinned for a truly asynchronous copy); ``dev_frames`` the CUDA
         uint8 [H,W,3] destination buffers.  ``sparse_for=(dst_h, dst_w)`` copies only the rows the
-        letterbox to that size reads.  Returns the bytes put on the bus."""
+        letterbox to that size reads; ``geoms`` (one ``Letterbox`` per frame, e.g. from ``letterbox_meta_ultralytics``)
+        only the rows ``preprocess_geom`` with that geometry reads.  Returns the bytes put on the bus."""
         n = len(dev_frames)
         if n == 0:
             return 0
         moved = C.c_int64(0)
+        if geoms is not None:
+            self._check(self.lib.b200va_upload_frames_geom(
+                self._h, _ptr_array([p for p, _ in host_ptrs]), _ptr_array([d.data_ptr() for d in dev_frames]),
+                _int_array([d.shape[0] for d in dev_frames]), _int_array([d.shape[1] for d in dev_frames]),
+                (C.c_int64 * n)(*[int(pt) for _, pt in host_ptrs]), (C.c_int64 * n)(*[d.stride(0) for d in dev_frames]),
+                n, self._geom_array(geoms, n), C.byref(moved), self._stream()))
+            return int(moved.value)
         self._check(self.lib.b200va_upload_frames(
             self._h, _ptr_array([p for p, _ in host_ptrs]), _ptr_array([d.data_ptr() for d in dev_frames]),
             _int_array([d.shape[0] for d in dev_frames]), _int_array([d.shape[1] for d in dev_frames]),
@@ -497,17 +526,22 @@ class Handle:
             1 if sparse_for else 0, C.byref(moved), self._stream()))
         return int(moved.value)
 
-    def upload_frames_nv12(self, host_frames, dev_frames, sparse_for=None) -> int:
+    def upload_frames_nv12(self, host_frames, dev_frames, sparse_for=None, geoms=None) -> int:
         """``upload_frames`` for NV12: ``host_frames[i]`` = ``Nv12Frame`` (host plane addresses and pitches; pinned for
         a truly asynchronous copy), ``dev_frames`` the CUDA NV12 destinations (``[3H/2, W]`` tensors or ``(y, uv)``
         pairs).  ``sparse_for=(dst_h, dst_w)`` copies only the luma rows the letterbox to that size reads and the
-        chroma rows they use.  Returns the bytes put on the bus."""
+        chroma rows they use; ``geoms`` those of ``preprocess_geom`` with one ``Letterbox`` per frame.  Returns the
+        bytes put on the bus."""
         n = len(dev_frames)
         if n == 0:
             return 0
         db = Nv12Batch(dev_frames)
         hb = (Nv12Frame * n)(*host_frames)
         moved = C.c_int64(0)
+        if geoms is not None:
+            self._check(self.lib.b200va_upload_frames_nv12_geom(self._h, hb, db.nv, db.hs, db.ws, n, self._geom_array(geoms, n),
+                                                                C.byref(moved), self._stream()))
+            return int(moved.value)
         self._check(self.lib.b200va_upload_frames_nv12(
             self._h, hb, db.nv, db.hs, db.ws, n, int(sparse_for[0]) if sparse_for else 0,
             int(sparse_for[1]) if sparse_for else 0, 1 if sparse_for else 0, C.byref(moved), self._stream()))
@@ -741,9 +775,10 @@ class Handle:
     # -- Ultralytics semantics (SURVEY 8f row 2) ---------------------------------------------
     def preprocess_geom(self, frames, geoms, dst_hw, fmt: int = OUT_F32_RGB_NCHW, roi_masks=None, out=None):
         """Letterbox with caller-supplied geometry (``geoms``: one ``Letterbox`` per frame, e.g. from
-        ``letterbox_meta_ultralytics``) into a ``dst_hw`` canvas."""
+        ``letterbox_meta_ultralytics``) into a ``dst_hw`` canvas.  NV12 frames (``[3H/2, W]`` tensors, ``(y, uv)``
+        pairs or an ``Nv12Batch``) give the result of the BGR call on their ``cv2.cvtColor`` conversion."""
         t = self.torch
-        fb = self._batch(frames, roi_masks)
+        fb = self._batch(frames, roi_masks, nv12_ok=True)
         b = fb.n
         dh, dw = int(dst_hw[0]), int(dst_hw[1])
         dtype = {OUT_F32_RGB_NCHW: t.float32, OUT_F16_RGB_NCHW: t.float16}.get(fmt & 0xff, t.uint8)
@@ -752,8 +787,11 @@ class Handle:
             out = t.empty(shape, dtype=dtype, device=self.device)
         elif tuple(out.shape) != shape or out.dtype != dtype or not out.is_contiguous():
             raise ValueError("preprocess_geom: `out` has the wrong shape / dtype / layout")
-        garr = geoms if isinstance(geoms, C.Array) else (Letterbox * max(b, 1))(*geoms)
-        if b:
+        garr = self._geom_array(geoms, b) if not isinstance(geoms, C.Array) else geoms
+        if b and isinstance(fb, Nv12Batch):
+            self._check(self.lib.b200va_preprocess_geom_nv12(self._h, fb.nv, fb.hs, fb.ws, b, fb.mask_ptrs, garr,
+                                                             C.c_void_p(out.data_ptr()), dh, dw, fmt, self._stream()))
+        elif b:
             self._check(self.lib.b200va_preprocess_geom(self._h, fb.ptrs, fb.hs, fb.ws, fb.pitch, b, fb.mask_ptrs, garr,
                                                         C.c_void_p(out.data_ptr()), dh, dw, fmt, self._stream()))
         return out
@@ -844,13 +882,21 @@ class Handle:
                   head=None, metas=None, conf_thr: float = 0.25, iou_thr: float = 0.45, classes=None, layout=None,
                   filter_conf: Optional[float] = None, dets=None, score_mode: int = SCORE_REF_COMPAT,
                   nms_mode: int = NMS_AGNOSTIC, slots=None, tracker_cfg=None, det_scale=None, skip=None,
-                  tracks=None, schedule: int = SCHEDULE_AUTO) -> TickPlan:
+                  tracks=None, schedule: int = SCHEDULE_AUTO, ultralytics: Optional[dict] = None) -> TickPlan:
         """Prepare a ``b200va_tick``: the letterbox of ``frames`` into ``net_out`` and the post-process
         of ``head`` into ``dets`` followed by the tracker update of ``slots`` into ``tracks``.  Either
-        half may be omitted.  ``tracker_cfg`` = (max_age, min_hits, max_iou_distance)."""
+        half may be omitted.  ``tracker_cfg`` = (max_age, min_hits, max_iou_distance).
+        ``ultralytics=dict(geoms=..., frame_hw=..., in_hw=..., agnostic=False, max_det=300)`` makes it a
+        ``b200va_tick_ultralytics``: the letterbox is ``preprocess_geom`` with ``geoms`` (one ``Letterbox`` per frame) into
+        a ``dst_hw`` canvas, the post-process is ``postprocess_ultralytics`` with ``frame_hw`` (one (h, w) per head frame)
+        and ``in_hw``; ``metas``, ``score_mode`` and ``nms_mode`` are not used."""
         t = self.torch
         a = TickArgs()
         keep = []
+        u = None
+        if ultralytics is not None:
+            u = TickUltra()
+            keep.append(u)
         if frames is not None:
             fb = self._batch(frames, roi_masks, nv12_ok=True)
             dh, dw = int(dst_hw[0]), int(dst_hw[1])
@@ -865,9 +911,25 @@ class Handle:
             a.roi_masks = fb.mask_ptrs
             a.net_out, a.dst_h, a.dst_w, a.out_format, a.meta_out = net_out.data_ptr(), dh, dw, fmt, fb.metas
             keep += [fb, net_out]
+            if u is not None:
+                if ultralytics.get("geoms") is None:
+                    raise ValueError("plan_tick: the Ultralytics letterbox needs `geoms`")
+                garr = self._geom_array(ultralytics["geoms"], fb.n)
+                u.geom = C.cast(garr, C.POINTER(Letterbox))
+                keep.append(garr)
         if head is not None:
             b, layout, channels, anchors = self._head_args(head, layout)
-            marr = metas if isinstance(metas, C.Array) else (Letterbox * max(b, 1))(*metas)
+            if u is not None:
+                hw = list(ultralytics["frame_hw"])
+                if len(hw) != b:
+                    raise ValueError("plan_tick: `frame_hw` needs one (h, w) per head frame")
+                u.src_h, u.src_w = _int_array([v[0] for v in hw]), _int_array([v[1] for v in hw])
+                u.in_h, u.in_w = int(ultralytics["in_hw"][0]), int(ultralytics["in_hw"][1])
+                u.agnostic, u.max_det = 1 if ultralytics.get("agnostic", False) else 0, int(ultralytics.get("max_det", 300))
+                keep += [u.src_h, u.src_w]
+                marr = None
+            else:
+                marr = metas if isinstance(metas, C.Array) else (Letterbox * max(b, 1))(*metas)
             cls_arr = (C.c_int32 * len(classes))(*[int(c) for c in classes]) if classes else None
             if dets is None:
                 dets = self.alloc_dets(b)
@@ -904,11 +966,15 @@ class Handle:
         plan.dets, plan.tracks = dets, tracks
         if frames is not None and isinstance(fb, Nv12Batch):
             plan.nv12 = fb.nv
+        plan.ultra = u
         return plan
 
     def tick(self, plan: TickPlan) -> None:
         """Run a prepared tick on the current stream (results land in the plan's buffers)."""
-        if plan.nv12 is not None:
+        if plan.ultra is not None:
+            self._check(self.lib.b200va_tick_ultralytics(self._h, C.byref(plan.args), C.byref(plan.ultra), plan.nv12,
+                                                         self._stream()))
+        elif plan.nv12 is not None:
             self._check(self.lib.b200va_tick_nv12(self._h, C.byref(plan.args), plan.nv12, self._stream()))
         else:
             self._check(self.lib.b200va_tick(self._h, C.byref(plan.args), self._stream()))

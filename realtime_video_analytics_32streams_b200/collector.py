@@ -255,8 +255,9 @@ def install(rpipe, engine_factory: Callable, max_wait_s: float = 0.010) -> None:
 
 
 def default_engine_factory(streams: Sequence, detector, pipeline_config):
-    """``HotPathEngine`` over ``streams`` with the forward, thresholds and handle of the pipeline's ``B200Detector``."""
+    """``HotPathEngine`` over ``streams`` with the pipeline's detector: its forward, thresholds, handle and semantics (a
+    ``B200UltralyticsDetector`` gives an engine that runs LetterBox / non_max_suppression / scale_boxes)."""
     from .engine import HotPathEngine
 
-    return HotPathEngine(streams, detector.config, pipeline_config.tracker, infer=detector._infer_fn,
-                         handle=detector.h, input_hw=detector.input_hw, on_overflow="warn")
+    return HotPathEngine(streams, detector.config, pipeline_config.tracker, infer=detector._infer_fn, on_overflow="warn",
+                         detector=detector)

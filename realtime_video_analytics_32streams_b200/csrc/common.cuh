@@ -264,6 +264,13 @@ int letterbox_fuse_plan(b200va_ctx* h, int src_h, int src_w, int new_h, int new_
                         int dst_w, FusePlan* out);
 const int4* tap_arena(b200va_ctx* h);
 
+// The Ultralytics post-process options (b200va_postprocess_ultralytics, b200va_tick_ultralytics; postprocess.cu).
+struct UltraOpts {
+  const int* src_h;
+  const int* src_w;
+  int in_h, in_w, agnostic, max_det;
+};
+
 // per-module state owned by the handle
 int tap_cache_create(b200va_ctx* h);
 void tap_cache_destroy(b200va_ctx* h);

@@ -2245,11 +2245,6 @@ struct PendingChain {
   int n;         // frames
 };
 
-struct UltraOpts {  // b200va_postprocess_ultralytics
-  const int* src_h;
-  const int* src_w;
-  int in_h, in_w, agnostic, max_det;
-};
 }  // namespace
 
 static int postprocess_impl(b200va_handle h, const void* head, int layout, int batch, int channels, int anchors,
@@ -2634,13 +2629,16 @@ void postprocess_release(b200va_ctx* h) {
 }
 
 // b200va_tick: post-process followed by the tracker update of the same rows; *fused tells the caller whether the
-// tracker already ran inside the post-process's second kernel.
-int postprocess_then_track(b200va_handle h, const b200va_tick_args* a, void* stream, bool* fused, bool* tail_on_side, bool defer) {
+// tracker already ran inside the post-process's second kernel.  ultra != NULL: the post-process is
+// b200va_postprocess_ultralytics (a->meta, a->score_mode and a->nms_mode are not read).
+int postprocess_then_track(b200va_handle h, const b200va_tick_args* a, const UltraOpts* ultra, void* stream, bool* fused,
+                           bool* tail_on_side, bool defer) {
   FuseReq f{a->stream_slots, a->trk_batch, a->max_dets, a->det_scale, a->skip, a->trk_cfg, a->id_base, a->tracks, a->new_counts, false, false, defer};
   const bool want = a->stream_slots != nullptr && a->trk_batch > 0 && a->trk_batch == a->head_batch && a->trk_cfg != nullptr;
-  const int rc = postprocess_impl(h, a->head, a->layout, a->head_batch, a->channels, a->anchors, a->meta, a->conf_thr, a->iou_thr,
-                                  a->classes, a->n_classes, a->score_mode, a->nms_mode, a->filter_conf_thr_f64, a->use_filter,
-                                  a->dets, stream, nullptr, &f);
+  const int rc = postprocess_impl(h, a->head, a->layout, a->head_batch, a->channels, a->anchors, ultra ? nullptr : a->meta,
+                                  a->conf_thr, a->iou_thr, a->classes, a->n_classes,
+                                  ultra ? B200VA_SCORE_V8_NATIVE : a->score_mode, ultra ? B200VA_NMS_AGNOSTIC : a->nms_mode,
+                                  a->filter_conf_thr_f64, a->use_filter, a->dets, stream, ultra, &f);
   *fused = f.done;
   *tail_on_side = f.tail_on_side;
   (void)want;

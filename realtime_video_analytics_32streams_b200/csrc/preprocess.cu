@@ -1151,14 +1151,15 @@ extern "C" int b200va_letterbox_meta_ultralytics(int src_h, int src_w, int dst_h
   return B200VA_OK;
 }
 
-extern "C" int b200va_preprocess_geom(b200va_handle h, const uint8_t* const* frames, const int* src_h, const int* src_w,
-                                      const int64_t* src_pitch, int batch, const uint8_t* const* roi_masks,
-                                      const b200va_letterbox* geom, void* out, int dst_h, int dst_w, int out_format,
-                                      void* stream) {
+// b200va_preprocess_geom*: the caller's geometry must describe each frame and fit the dst_h x dst_w canvas.
+template <typename P>
+static int preprocess_geom_impl(b200va_handle h, const SrcFrames& src, const int* src_h, const int* src_w, int batch,
+                                const uint8_t* const* roi_masks, const b200va_letterbox* geom, void* out, int dst_h,
+                                int dst_w, int out_format, void* stream) {
   if (!h) return B200VA_ERR_INVALID;
   std::lock_guard<std::recursive_mutex> lock(h->mu);
   DeviceGuard guard(h->cfg.device);
-  REQUIRE(h, frames && src_h && src_w && out && geom, "NULL argument");
+  REQUIRE(h, (src.bgr || src.nv12) && src_h && src_w && out && geom, "NULL argument");
   REQUIRE(h, batch >= 0 && batch <= h->cfg.max_batch, "batch %d outside [0, %d]", batch, h->cfg.max_batch);
   REQUIRE(h, dst_h > 0 && dst_w > 0 && dst_w < 65536, "bad destination size %dx%d", dst_w, dst_h);
   if (batch == 0) return B200VA_OK;
@@ -1175,8 +1176,28 @@ extern "C" int b200va_preprocess_geom(b200va_handle h, const uint8_t* const* fra
     pt[b] = m.pad_top;
     pl[b] = m.pad_left;
   }
-  return run_resample(h, frames, src_h, src_w, src_pitch, batch, roi_masks, out, nh.data(), nw.data(), pt.data(), pl.data(),
-                      dst_h, dst_w, out_format, (cudaStream_t)stream);
+  return run_resample<P>(h, src, src_h, src_w, batch, roi_masks, out, nh.data(), nw.data(), pt.data(), pl.data(), dst_h,
+                         dst_w, out_format, (cudaStream_t)stream);
+}
+
+extern "C" int b200va_preprocess_geom(b200va_handle h, const uint8_t* const* frames, const int* src_h, const int* src_w,
+                                      const int64_t* src_pitch, int batch, const uint8_t* const* roi_masks,
+                                      const b200va_letterbox* geom, void* out, int dst_h, int dst_w, int out_format,
+                                      void* stream) {
+  SrcFrames src;
+  src.bgr = frames;
+  src.pitch = src_pitch;
+  return preprocess_geom_impl<PreParams>(h, src, src_h, src_w, batch, roi_masks, geom, out, dst_h, dst_w, out_format, stream);
+}
+
+extern "C" int b200va_preprocess_geom_nv12(b200va_handle h, const b200va_nv12_frame* frames, const int* src_h,
+                                           const int* src_w, int batch, const uint8_t* const* roi_masks,
+                                           const b200va_letterbox* geom, void* out, int dst_h, int dst_w, int out_format,
+                                           void* stream) {
+  SrcFrames src;
+  src.nv12 = frames;
+  return preprocess_geom_impl<PreParamsNv12>(h, src, src_h, src_w, batch, roi_masks, geom, out, dst_h, dst_w, out_format,
+                                             stream);
 }
 
 extern "C" int b200va_resize_linear_u8(b200va_handle h, const uint8_t* const* frames, const int* src_h,
@@ -1303,11 +1324,8 @@ struct RowPattern {
 std::map<std::pair<int, int>, RowPattern> g_row_patterns;
 std::mutex g_row_mu;
 
-RowPattern needed_rows(int src_h, int new_h) {
-  std::lock_guard<std::mutex> lock(g_row_mu);
-  auto key = std::make_pair(src_h, new_h);
-  auto it = g_row_patterns.find(key);
-  if (it != g_row_patterns.end()) return it->second;
+// The source rows a letterbox that resizes src_h rows to new_h reads: those with a non-zero vertical tap weight.
+std::vector<char> tapped_rows(int src_h, int new_h) {
   std::vector<char> need((size_t)src_h, 0);
   for (int d = 0; d < new_h; ++d) {
     int y0, y1;
@@ -1316,6 +1334,15 @@ RowPattern needed_rows(int src_h, int new_h) {
     if (b0) need[y0] = 1;
     if (b1) need[y1] = 1;
   }
+  return need;
+}
+
+RowPattern needed_rows(int src_h, int new_h) {
+  std::lock_guard<std::mutex> lock(g_row_mu);
+  auto key = std::make_pair(src_h, new_h);
+  auto it = g_row_patterns.find(key);
+  if (it != g_row_patterns.end()) return it->second;
+  const std::vector<char> need = tapped_rows(src_h, new_h);
   std::vector<std::pair<int, int>> runs;  // (start, length)
   for (int y = 0; y < src_h;) {
     if (!need[y]) {
@@ -1342,55 +1369,31 @@ RowPattern needed_rows(int src_h, int new_h) {
   g_row_patterns[key] = rp;
   return rp;
 }
-}  // namespace
 
-extern "C" int b200va_upload_frames(b200va_handle h, const uint8_t* const* host_frames, uint8_t* const* dev_frames,
-                                    const int* src_h, const int* src_w, const int64_t* host_pitch,
-                                    const int64_t* dev_pitch, int batch, int dst_h, int dst_w, int rows_mode,
-                                    int64_t* bytes_copied, void* stream) {
-  if (!h) return B200VA_ERR_INVALID;
-  std::lock_guard<std::recursive_mutex> lock(h->mu);
-  DeviceGuard guard(h->cfg.device);
-  cudaStream_t st = (cudaStream_t)stream;
-  REQUIRE(h, host_frames && dev_frames && src_h && src_w, "NULL argument");
+// The resized height of each frame whose tapped rows alone are to be uploaded: from the reference geometry to
+// dst_h x dst_w (geom == NULL) or from the caller's per-frame geometry.  Empty when rows_mode asks for every row.
+int upload_heights(b200va_ctx* h, const int* src_h, const int* src_w, int batch, int dst_h, int dst_w, int rows_mode,
+                   const b200va_letterbox* geom, std::vector<int>* new_h) {
+  new_h->clear();
+  if (rows_mode != 1) return B200VA_OK;
+  REQUIRE(h, src_h && src_w, "NULL argument");
   REQUIRE(h, batch >= 0, "negative batch");
-  PhaseScope phase(h, B200VA_PHASE_UPLOAD, st);
-  int64_t total = 0;
+  new_h->resize(batch);
   for (int b = 0; b < batch; ++b) {
-    REQUIRE(h, host_frames[b] && dev_frames[b] && src_h[b] > 0 && src_w[b] > 0, "frame %d: bad arguments", b);
-    const size_t rb = (size_t)3 * src_w[b];
-    const size_t hp = host_pitch ? (size_t)host_pitch[b] : rb, dp = dev_pitch ? (size_t)dev_pitch[b] : rb;
-    REQUIRE(h, hp >= rb && dp >= rb, "frame %d: pitch smaller than 3*width", b);
-    RowPattern rp;
-    if (rows_mode == 1) {
+    if (geom) {
+      const b200va_letterbox& m = geom[b];
+      REQUIRE(h, m.src_h == src_h[b] && m.src_w == src_w[b] && m.new_h > 0, "frame %d: geometry is for %dx%d (new_h %d), frame is %dx%d",
+              b, m.src_w, m.src_h, m.new_h, src_w[b], src_h[b]);
+      (*new_h)[b] = m.new_h;
+    } else {
       b200va_letterbox m;
       REQUIRE(h, b200va_letterbox_meta(src_h[b], src_w[b], dst_h, dst_w, &m) == B200VA_OK && m.new_h > 0, "frame %d: bad letterbox geometry", b);
-      rp = needed_rows(src_h[b], m.new_h);
-    }
-    if (rp.regular) {
-      if (hp == rb && dp == rb) {
-        // a run of consecutive rows is one contiguous span
-        CUDA_TRY(h, cudaMemcpy2DAsync(dev_frames[b] + (size_t)rp.first * dp, (size_t)rp.period * dp,
-                                      host_frames[b] + (size_t)rp.first * hp, (size_t)rp.period * hp,
-                                      (size_t)rp.run * rb, rp.count, cudaMemcpyHostToDevice, st));
-      } else {
-        for (int r = 0; r < rp.run; ++r)
-          CUDA_TRY(h, cudaMemcpy2DAsync(dev_frames[b] + (size_t)(rp.first + r) * dp, (size_t)rp.period * dp,
-                                        host_frames[b] + (size_t)(rp.first + r) * hp, (size_t)rp.period * hp, rb,
-                                        rp.count, cudaMemcpyHostToDevice, st));
-      }
-      total += (int64_t)rp.run * rp.count * (int64_t)rb;
-    } else {
-      if (hp == rb && dp == rb)
-        CUDA_TRY(h, cudaMemcpyAsync(dev_frames[b], host_frames[b], rb * (size_t)src_h[b], cudaMemcpyHostToDevice, st));
-      else
-        CUDA_TRY(h, cudaMemcpy2DAsync(dev_frames[b], dp, host_frames[b], hp, rb, src_h[b], cudaMemcpyHostToDevice, st));
-      total += (int64_t)rb * src_h[b];
+      (*new_h)[b] = m.new_h;
     }
   }
-  if (bytes_copied) *bytes_copied = total;
   return B200VA_OK;
 }
+}  // namespace
 
 namespace {
 // One plane's needed rows as at most `max_runs` strided copies (start, step, count): from the first row not yet
@@ -1447,16 +1450,79 @@ int copy_plane_rows(b200va_ctx* h, uint8_t* dst, int64_t dp, const uint8_t* src,
 }
 }  // namespace
 
-extern "C" int b200va_upload_frames_nv12(b200va_handle h, const b200va_nv12_frame* host, const b200va_nv12_frame* dev,
-                                         const int* src_h, const int* src_w, int batch, int dst_h, int dst_w, int rows_mode,
+// new_h empty: every row of every frame; else the rows the letterbox to new_h[b] rows reads.
+static int upload_bgr(b200va_handle h, const uint8_t* const* host_frames, uint8_t* const* dev_frames, const int* src_h,
+                      const int* src_w, const int64_t* host_pitch, const int64_t* dev_pitch, int batch,
+                      const std::vector<int>& new_h, int64_t* bytes_copied, cudaStream_t st) {
+  REQUIRE(h, host_frames && dev_frames && src_h && src_w, "NULL argument");
+  REQUIRE(h, batch >= 0, "negative batch");
+  PhaseScope phase(h, B200VA_PHASE_UPLOAD, st);
+  int64_t total = 0;
+  for (int b = 0; b < batch; ++b) {
+    REQUIRE(h, host_frames[b] && dev_frames[b] && src_h[b] > 0 && src_w[b] > 0, "frame %d: bad arguments", b);
+    const size_t rb = (size_t)3 * src_w[b];
+    const size_t hp = host_pitch ? (size_t)host_pitch[b] : rb, dp = dev_pitch ? (size_t)dev_pitch[b] : rb;
+    REQUIRE(h, hp >= rb && dp >= rb, "frame %d: pitch smaller than 3*width", b);
+    RowPattern rp;
+    if (!new_h.empty()) rp = needed_rows(src_h[b], new_h[b]);
+    if (rp.regular) {
+      if (hp == rb && dp == rb) {
+        // a run of consecutive rows is one contiguous span
+        CUDA_TRY(h, cudaMemcpy2DAsync(dev_frames[b] + (size_t)rp.first * dp, (size_t)rp.period * dp,
+                                      host_frames[b] + (size_t)rp.first * hp, (size_t)rp.period * hp,
+                                      (size_t)rp.run * rb, rp.count, cudaMemcpyHostToDevice, st));
+      } else {
+        for (int r = 0; r < rp.run; ++r)
+          CUDA_TRY(h, cudaMemcpy2DAsync(dev_frames[b] + (size_t)(rp.first + r) * dp, (size_t)rp.period * dp,
+                                        host_frames[b] + (size_t)(rp.first + r) * hp, (size_t)rp.period * hp, rb,
+                                        rp.count, cudaMemcpyHostToDevice, st));
+      }
+      total += (int64_t)rp.run * rp.count * (int64_t)rb;
+    } else {
+      // irregular rows go as a few strided copies, like an NV12 plane (every row when they are too scattered)
+      const int rc = copy_plane_rows(h, dev_frames[b], dp, host_frames[b], hp, rb, src_h[b],
+                                     new_h.empty() ? std::vector<char>() : tapped_rows(src_h[b], new_h[b]), st, &total);
+      if (rc) return rc;
+    }
+  }
+  if (bytes_copied) *bytes_copied = total;
+  return B200VA_OK;
+}
+
+extern "C" int b200va_upload_frames(b200va_handle h, const uint8_t* const* host_frames, uint8_t* const* dev_frames,
+                                    const int* src_h, const int* src_w, const int64_t* host_pitch,
+                                    const int64_t* dev_pitch, int batch, int dst_h, int dst_w, int rows_mode,
+                                    int64_t* bytes_copied, void* stream) {
+  if (!h) return B200VA_ERR_INVALID;
+  std::lock_guard<std::recursive_mutex> lock(h->mu);
+  DeviceGuard guard(h->cfg.device);
+  std::vector<int> new_h;
+  const int rc = upload_heights(h, src_h, src_w, batch, dst_h, dst_w, rows_mode, nullptr, &new_h);
+  if (rc) return rc;
+  return upload_bgr(h, host_frames, dev_frames, src_h, src_w, host_pitch, dev_pitch, batch, new_h, bytes_copied,
+                    (cudaStream_t)stream);
+}
+
+extern "C" int b200va_upload_frames_geom(b200va_handle h, const uint8_t* const* host_frames, uint8_t* const* dev_frames,
+                                         const int* src_h, const int* src_w, const int64_t* host_pitch,
+                                         const int64_t* dev_pitch, int batch, const b200va_letterbox* geom,
                                          int64_t* bytes_copied, void* stream) {
   if (!h) return B200VA_ERR_INVALID;
   std::lock_guard<std::recursive_mutex> lock(h->mu);
   DeviceGuard guard(h->cfg.device);
-  cudaStream_t st = (cudaStream_t)stream;
+  REQUIRE(h, geom || batch == 0, "NULL geometry");
+  std::vector<int> new_h;
+  const int rc = upload_heights(h, src_h, src_w, batch, 0, 0, 1, geom, &new_h);
+  if (rc) return rc;
+  return upload_bgr(h, host_frames, dev_frames, src_h, src_w, host_pitch, dev_pitch, batch, new_h, bytes_copied,
+                    (cudaStream_t)stream);
+}
+
+// new_h as in upload_bgr; a needed luma row brings the chroma row it uses.
+static int upload_nv12(b200va_handle h, const b200va_nv12_frame* host, const b200va_nv12_frame* dev, const int* src_h,
+                       const int* src_w, int batch, const std::vector<int>& new_h, int64_t* bytes_copied, cudaStream_t st) {
   REQUIRE(h, host && dev && src_h && src_w, "NULL argument");
   REQUIRE(h, batch >= 0, "negative batch");
-  REQUIRE(h, rows_mode == 0 || rows_mode == 1, "unknown rows_mode %d", rows_mode);
   for (int b = 0; b < batch; ++b) {
     REQUIRE(h, host[b].y && host[b].uv && dev[b].y && dev[b].uv, "frame %d: NULL plane", b);
     REQUIRE(h, src_h[b] > 0 && src_w[b] > 0 && src_h[b] % 2 == 0 && src_w[b] % 2 == 0, "frame %d: NV12 needs an even size, got %dx%d",
@@ -1470,18 +1536,11 @@ extern "C" int b200va_upload_frames_nv12(b200va_handle h, const b200va_nv12_fram
   for (int b = 0; b < batch; ++b) {
     const int H = src_h[b], W = src_w[b];
     std::vector<char> need_y, need_uv;
-    if (rows_mode == 1) {
-      b200va_letterbox m;
-      REQUIRE(h, b200va_letterbox_meta(H, W, dst_h, dst_w, &m) == B200VA_OK && m.new_h > 0, "frame %d: bad letterbox geometry", b);
-      need_y.assign((size_t)H, 0);
+    if (!new_h.empty()) {
+      need_y = tapped_rows(H, new_h[b]);
       need_uv.assign((size_t)H / 2, 0);
-      for (int d = 0; d < m.new_h; ++d) {
-        int y0, y1;
-        short b0, b1;
-        linear_tap(H, m.new_h, d, false, &y0, &y1, &b0, &b1);
-        if (b0) need_y[y0] = need_uv[y0 >> 1] = 1;
-        if (b1) need_y[y1] = need_uv[y1 >> 1] = 1;
-      }
+      for (int y = 0; y < H; ++y)
+        if (need_y[y]) need_uv[y >> 1] = 1;
     }
     int rc = copy_plane_rows(h, const_cast<uint8_t*>(dev[b].y), dev[b].y_pitch, host[b].y, host[b].y_pitch, W, H, need_y, st, &total);
     if (rc) return rc;
@@ -1491,4 +1550,30 @@ extern "C" int b200va_upload_frames_nv12(b200va_handle h, const b200va_nv12_fram
   }
   if (bytes_copied) *bytes_copied = total;
   return B200VA_OK;
+}
+
+extern "C" int b200va_upload_frames_nv12(b200va_handle h, const b200va_nv12_frame* host, const b200va_nv12_frame* dev,
+                                         const int* src_h, const int* src_w, int batch, int dst_h, int dst_w, int rows_mode,
+                                         int64_t* bytes_copied, void* stream) {
+  if (!h) return B200VA_ERR_INVALID;
+  std::lock_guard<std::recursive_mutex> lock(h->mu);
+  DeviceGuard guard(h->cfg.device);
+  REQUIRE(h, rows_mode == 0 || rows_mode == 1, "unknown rows_mode %d", rows_mode);
+  std::vector<int> new_h;
+  const int rc = upload_heights(h, src_h, src_w, batch, dst_h, dst_w, rows_mode, nullptr, &new_h);
+  if (rc) return rc;
+  return upload_nv12(h, host, dev, src_h, src_w, batch, new_h, bytes_copied, (cudaStream_t)stream);
+}
+
+extern "C" int b200va_upload_frames_nv12_geom(b200va_handle h, const b200va_nv12_frame* host, const b200va_nv12_frame* dev,
+                                              const int* src_h, const int* src_w, int batch, const b200va_letterbox* geom,
+                                              int64_t* bytes_copied, void* stream) {
+  if (!h) return B200VA_ERR_INVALID;
+  std::lock_guard<std::recursive_mutex> lock(h->mu);
+  DeviceGuard guard(h->cfg.device);
+  REQUIRE(h, geom || batch == 0, "NULL geometry");
+  std::vector<int> new_h;
+  const int rc = upload_heights(h, src_h, src_w, batch, 0, 0, 1, geom, &new_h);
+  if (rc) return rc;
+  return upload_nv12(h, host, dev, src_h, src_w, batch, new_h, bytes_copied, (cudaStream_t)stream);
 }

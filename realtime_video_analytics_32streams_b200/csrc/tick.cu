@@ -2,13 +2,21 @@
 // the last head tensor as two branches of one call (fork / join on events, capturable in a graph).
 #include "common.cuh"
 
-int postprocess_then_track(b200va_handle h, const b200va_tick_args* a, void* stream, bool* fused, bool* tail_on_side,
-                           bool defer);                                // postprocess.cu
+int postprocess_then_track(b200va_handle h, const b200va_tick_args* a, const UltraOpts* ultra, void* stream, bool* fused,
+                           bool* tail_on_side, bool defer);            // postprocess.cu
 int postprocess_run_pending(b200va_handle h, void* stream);            // postprocess.cu
 bool postprocess_has_pending(b200va_handle h);                         // postprocess.cu
 
-// The letterbox of one tick: BGR frames (a->frames) or, when `nv12` is given, NV12 frames.
-static int tick_letterbox(b200va_handle h, const b200va_tick_args* a, const b200va_nv12_frame* nv12, cudaStream_t st) {
+// The letterbox of one tick: BGR frames (a->frames) or, when `nv12` is given, NV12 frames; with the caller's geometry
+// when `geom` is given (b200va_tick_ultralytics).
+static int tick_letterbox(b200va_handle h, const b200va_tick_args* a, const b200va_nv12_frame* nv12,
+                          const b200va_letterbox* geom, cudaStream_t st) {
+  if (geom && nv12)
+    return b200va_preprocess_geom_nv12(h, nv12, a->src_h, a->src_w, a->batch, a->roi_masks, geom, a->net_out, a->dst_h,
+                                       a->dst_w, a->out_format, st);
+  if (geom)
+    return b200va_preprocess_geom(h, a->frames, a->src_h, a->src_w, a->src_pitch, a->batch, a->roi_masks, geom, a->net_out,
+                                  a->dst_h, a->dst_w, a->out_format, st);
   if (nv12)
     return b200va_preprocess_nv12(h, nv12, a->src_h, a->src_w, a->batch, a->roi_masks, a->net_out, a->dst_h, a->dst_w,
                                   a->out_format, a->meta_out, st);
@@ -16,7 +24,9 @@ static int tick_letterbox(b200va_handle h, const b200va_tick_args* a, const b200
                            a->dst_w, a->out_format, a->meta_out, st);
 }
 
-static int tick_impl(b200va_handle h, const b200va_tick_args* a, const b200va_nv12_frame* nv12, void* stream) {
+// ultra / geom: b200va_tick_ultralytics (NULL for b200va_tick*).
+static int tick_impl(b200va_handle h, const b200va_tick_args* a, const b200va_nv12_frame* nv12, const UltraOpts* ultra,
+                     const b200va_letterbox* geom, void* stream) {
   std::lock_guard<std::recursive_mutex> lock(h->mu);
   DeviceGuard guard(h->cfg.device);
   REQUIRE(h, a->schedule >= 0 && a->schedule <= 6, "unknown schedule %d", a->schedule);
@@ -62,13 +72,13 @@ static int tick_impl(b200va_handle h, const b200va_tick_args* a, const b200va_nv
     }
     if (side) note(cudaEventRecord(h->ev_join, h->side_stream), "cudaEventRecord(join)");
     bool tracked = false, tail = false;
-    if (rc == B200VA_OK && has_post) rc = postprocess_then_track(h, a, main_st, &tracked, &tail, true);
+    if (rc == B200VA_OK && has_post) rc = postprocess_then_track(h, a, ultra, main_st, &tracked, &tail, true);
     if (rc == B200VA_OK && has_trk && !has_post)
       rc = b200va_tracker_update(h, a->stream_slots, a->trk_batch, a->dets, a->max_dets, a->det_scale, a->skip, a->trk_cfg,
                                  a->id_base, a->tracks, a->new_counts, main_st);
     if (rc == B200VA_OK && has_pre) {
       if (a->ev_pre_begin) note(cudaEventRecord((cudaEvent_t)a->ev_pre_begin, main_st), "cudaEventRecord(pre_begin)");
-      if (rc == B200VA_OK) rc = tick_letterbox(h, a, nv12, main_st);
+      if (rc == B200VA_OK) rc = tick_letterbox(h, a, nv12, geom, main_st);
       if (rc == B200VA_OK && a->ev_pre_end) note(cudaEventRecord((cudaEvent_t)a->ev_pre_end, main_st), "cudaEventRecord(pre_end)");
     }
     if (side) note(cudaStreamWaitEvent(main_st, h->ev_join, 0), "cudaStreamWaitEvent(join)");
@@ -97,7 +107,7 @@ static int tick_impl(b200va_handle h, const b200va_tick_args* a, const b200va_nv
     h->hook_recorded = false;
     h->post_tail_stream = sched3 ? h->side_stream : nullptr;
     // sparse scenes: NMS and the tracker update of the same rows run as ONE kernel (k_post_track)
-    rc = postprocess_then_track(h, a, post_st, &tracked, &tail_on_side, false);
+    rc = postprocess_then_track(h, a, ultra, post_st, &tracked, &tail_on_side, false);
     h->hook_after_decode = nullptr;
     h->post_tail_stream = nullptr;
     // the post-process reports whether it recorded the hook (it does not for empty or malformed heads)
@@ -113,7 +123,7 @@ static int tick_impl(b200va_handle h, const b200va_tick_args* a, const b200va_nv
   h->pdl_preprocess_wait = schedule == 5;
   if (rc == B200VA_OK && has_pre) {
     if (a->ev_pre_begin) note(cudaEventRecord((cudaEvent_t)a->ev_pre_begin, main_st), "cudaEventRecord(pre_begin)");
-    if (rc == B200VA_OK) rc = tick_letterbox(h, a, nv12, main_st);
+    if (rc == B200VA_OK) rc = tick_letterbox(h, a, nv12, geom, main_st);
     if (rc == B200VA_OK && a->ev_pre_end) note(cudaEventRecord((cudaEvent_t)a->ev_pre_end, main_st), "cudaEventRecord(pre_end)");
   }
   h->pdl_preprocess = false;
@@ -124,7 +134,7 @@ static int tick_impl(b200va_handle h, const b200va_tick_args* a, const b200va_nv
 
 extern "C" int b200va_tick(b200va_handle h, const b200va_tick_args* a, void* stream) {
   if (!h || !a) return B200VA_ERR_INVALID;
-  return tick_impl(h, a, nullptr, stream);
+  return tick_impl(h, a, nullptr, nullptr, nullptr, stream);
 }
 
 extern "C" int b200va_tick_nv12(b200va_handle h, const b200va_tick_args* a, const b200va_nv12_frame* frames, void* stream) {
@@ -133,5 +143,16 @@ extern "C" int b200va_tick_nv12(b200va_handle h, const b200va_tick_args* a, cons
     std::lock_guard<std::recursive_mutex> lock(h->mu);
     return set_error(h, B200VA_ERR_INVALID, "b200va_tick_nv12: NULL frames for a batch of %d", a->batch);
   }
-  return tick_impl(h, a, frames, stream);
+  return tick_impl(h, a, frames, nullptr, nullptr, stream);
+}
+
+extern "C" int b200va_tick_ultralytics(b200va_handle h, const b200va_tick_args* a, const b200va_tick_ultra* u,
+                                       const b200va_nv12_frame* frames, void* stream) {
+  if (!h || !a || !u) return B200VA_ERR_INVALID;
+  if (a->batch > 0 && (!u->geom || (!frames && !a->frames))) {
+    std::lock_guard<std::recursive_mutex> lock(h->mu);
+    return set_error(h, B200VA_ERR_INVALID, "b200va_tick_ultralytics: NULL frames or geometry for a batch of %d", a->batch);
+  }
+  const UltraOpts ultra{u->src_h, u->src_w, u->in_h, u->in_w, u->agnostic ? 1 : 0, u->max_det};
+  return tick_impl(h, a, frames, &ultra, u->geom, stream);
 }

@@ -139,11 +139,13 @@ class B200Detector:
             raise ValueError(f"infer returned {tuple(head.shape)} for a batch of {len(frames)}")
         return self._run_post(head, metas, dets_out), metas
 
-    def _run_post(self, head, metas, dets_out=None):
+    def _run_post(self, head, metas, dets_out=None, fold_filter=None):
+        """``fold_filter`` overrides the detector's own setting for this call (a batched engine always folds)."""
         cfg = self.config
         thr = float(cfg.confidence_threshold)
+        fold = self.fold_filter if fold_filter is None else fold_filter
         return self.h.postprocess(head, metas, thr, float(cfg.iou_threshold), getattr(cfg, "classes", None) or None,
-                                  filter_conf=thr if self.fold_filter else None, out=dets_out)
+                                  filter_conf=thr if fold else None, out=dets_out)
 
     def _to_detections(self, dets, packets) -> List[List[Detection]]:
         """Device SoA -> ``Detection`` objects: one pinned device->host copy of the flat table (and the capacity
@@ -190,13 +192,18 @@ class B200UltralyticsDetector(B200Detector):
         super().__init__(config, input_hw=input_hw, infer=infer, handle=handle, fold_filter=fold_filter)
         self.auto, self.stride, self.max_det, self.agnostic = bool(auto), int(stride), int(max_det), bool(agnostic)
 
+    def frame_geometry(self, h: int, w: int):
+        """(Letterbox, (out_h, out_w)) of one frame alone: the rect shape ``predict`` gives a single image."""
+        m, oh, ow = _native.letterbox_meta_ultralytics(int(h), int(w), self.input_hw[0], self.input_hw[1], self.auto,
+                                                       self.stride)
+        return m, (oh, ow)
+
     def _geometry(self, shapes):
         geoms, outs = [], set()
         for h, w in shapes:
-            m, oh, ow = _native.letterbox_meta_ultralytics(int(h), int(w), self.input_hw[0], self.input_hw[1], self.auto,
-                                                           self.stride)
+            m, out_hw = self.frame_geometry(h, w)
             geoms.append(m)
-            outs.add((oh, ow))
+            outs.add(out_hw)
         if len(outs) != 1:
             # LetterBox(auto=...) is only rect when every image of the batch has the same shape (same_shapes)
             geoms = [_native.letterbox_meta_ultralytics(int(h), int(w), self.input_hw[0], self.input_hw[1], False,
@@ -205,10 +212,12 @@ class B200UltralyticsDetector(B200Detector):
         return geoms, next(iter(outs))
 
     def _preprocess(self, frame, roi_mask=None):
-        dev = self._stager.upload([frame])  # every row: the sparse upload pattern is the reference letterbox's
-        geoms, in_hw = self._geometry([dev[0].shape[:2]])
+        """A host frame (BGR or NV12) crosses PCIe as just the rows this frame's LetterBox reads."""
+        shape = _native.frame_hw(frame)
+        geoms, in_hw = self._geometry([shape])
+        dev = self._stager.upload([frame], geoms=geoms)
         tensor = self.h.preprocess_geom(dev, geoms, in_hw, self._fmt, [roi_mask] if roi_mask is not None else None)
-        return tensor, {"orig_shape": tuple(int(v) for v in dev[0].shape[:2]), "in_shape": in_hw}
+        return tensor, {"orig_shape": shape, "in_shape": in_hw}
 
     def _postprocess(self, predictions, packet: FramePacket, meta: dict) -> List[Detection]:
         head = self._as_head(predictions)
@@ -218,18 +227,44 @@ class B200UltralyticsDetector(B200Detector):
         return self._to_detections(dets, [packet])[0]
 
     def predict_batch_device(self, frames, roi_masks=None, dets_out=None):
-        dev = self._stager.upload(frames)
-        shapes = [tuple(int(v) for v in d.shape[:2]) for d in dev]
+        shapes = [_native.frame_hw(f) for f in frames]
         geoms, in_hw = self._geometry(shapes)
-        tensor = self.h.preprocess_geom(dev, geoms, in_hw, self._fmt, roi_masks)
+        dev = self._stager.upload(frames, geoms=geoms)
+        tensor = self.letterbox(dev, geoms, in_hw, roi_masks)
         head = self._as_head(self._infer(tensor))
         if head.dim() != 3 or head.shape[0] != len(frames):
             raise ValueError(f"infer returned {tuple(head.shape)} for a batch of {len(frames)}")
         return self._run_post_ultra(head, shapes, in_hw, dets_out), geoms
 
-    def _run_post_ultra(self, head, shapes, in_hw, dets_out=None):
+    def letterbox(self, frames, geoms, in_hw, roi_masks=None, fmt=None, out=None, on_run=None):
+        """``preprocess_geom`` of device frames that may mix BGR and NV12: one call per run of consecutive frames of one
+        kind, into the rows of ``out`` at their positions.  ``on_run(b, e)`` is called before the call for frames
+        ``[b, e)`` of a batch of several runs (e.g. to point the device skip mask at their entries)."""
+        fmt = self._fmt if fmt is None else fmt
+        kinds = [_native.is_nv12(f) for f in frames]
+        masks = list(roi_masks) if roi_masks is not None else [None] * len(frames)
+        b = 0
+        while b < len(frames):
+            e = b + 1
+            while e < len(frames) and kinds[e] == kinds[b]:
+                e += 1
+            if (b, e) == (0, len(frames)):
+                return self.h.preprocess_geom(frames, geoms, in_hw, fmt, roi_masks, out=out)
+            if on_run is not None:
+                on_run(b, e)
+            if out is None:
+                t = self.h.torch
+                dtype = {_native.OUT_F32_RGB_NCHW: t.float32, _native.OUT_F16_RGB_NCHW: t.float16}.get(fmt & 0xff, t.uint8)
+                shape = (len(frames), *in_hw, 3) if (fmt & 0xff) == _native.OUT_U8_BGR_NHWC else (len(frames), 3, *in_hw)
+                out = t.empty(shape, dtype=dtype, device=self.h.device)
+            self.h.preprocess_geom(frames[b:e], geoms[b:e], in_hw, fmt, masks[b:e], out=out[b:e])
+            b = e
+        return out
+
+    def _run_post_ultra(self, head, shapes, in_hw, dets_out=None, fold_filter=None):
         cfg = self.config
         thr = float(cfg.confidence_threshold)
+        fold = self.fold_filter if fold_filter is None else fold_filter
         return self.h.postprocess_ultralytics(head, shapes, in_hw, thr, float(cfg.iou_threshold),
                                               getattr(cfg, "classes", None) or None, self.agnostic, self.max_det,
-                                              filter_conf=thr if self.fold_filter else None, out=dets_out)
+                                              filter_conf=thr if fold else None, out=dets_out)

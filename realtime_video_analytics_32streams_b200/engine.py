@@ -25,7 +25,7 @@ from typing import Callable, Dict, List, Optional, Sequence
 import numpy as np
 
 from . import _native
-from .detector import B200Detector
+from .detector import B200Detector, B200UltralyticsDetector
 from .frame_filter import MotionFilter, roi_mask
 from .runtime import FrameStager, get_handle
 from .tracker import B200IouTracker
@@ -173,8 +173,13 @@ class HotPathEngine:
 
     def __init__(self, streams: Sequence, detector_config, tracker_config, infer: Callable,
                  handle: Optional[_native.Handle] = None, input_hw=None, depth: int = 2, static_pads: bool = True,
-                 on_overflow: str = "raise", profile: bool = False, device_gates: bool = False):
-        """``device_gates``: take the motion and adaptive-FPS decisions on the device (``b200va_gates_decide`` /
+                 on_overflow: str = "raise", profile: bool = False, device_gates: bool = False, detector=None):
+        """``detector``: the detector whose semantics the tick runs (its config, forward, input size and handle; then
+        ``detector_config``, ``infer``, ``input_hw`` and ``handle`` are not used).  By default a ``B200Detector`` (the
+        reference's numpy-path semantics).  A ``B200UltralyticsDetector`` gives what that detector's ``predict`` gives
+        frame by frame: every frame is letterboxed to its own rect shape (``LetterBox(auto=True)`` of one image), and
+        frames of equal network-input shape share one letterbox, forward and post-process call.
+        ``device_gates``: take the motion and adaptive-FPS decisions on the device (``b200va_gates_decide`` /
         ``b200va_gates_commit``): no host round trip inside a tick, every live frame keeps its batch position (``infer``
         sees all of them; rows of gated-off frames hold stale pixels and their heads are ignored), and ticks may be
         pipelined (``submit`` before ``collect``) even for streams with motion_filter / adaptive_fps.  Results are
@@ -185,11 +190,18 @@ class HotPathEngine:
         if on_overflow not in ("raise", "warn"):
             raise ValueError("on_overflow must be 'raise' or 'warn'")
         self.on_overflow, self.profile = on_overflow, bool(profile)
+        if detector is not None:
+            handle = detector.h
         self.h = handle if handle is not None else get_handle()
         if self.profile:
             self.h.set_profiling(True)
         self.streams = list(streams)
-        self.detector = B200Detector(detector_config, input_hw=input_hw, infer=infer, handle=self.h, fold_filter=True)
+        if detector is None:
+            detector = B200Detector(detector_config, input_hw=input_hw, infer=infer, handle=self.h, fold_filter=True)
+        self.detector = detector
+        self.ultralytics = isinstance(detector, B200UltralyticsDetector)
+        self._ultra_geoms: Dict[tuple, tuple] = {}  # frame (h, w) -> (Letterbox, network-input (h, w))
+        self._scratch = None  # detection rows of one shape group, before they are copied to their stream positions
         self.tracker = B200IouTracker(tracker_config, handle=self.h)
         self.state: Dict[str, _StreamState] = {s.name: _StreamState(s) for s in self.streams}
         self.stager = FrameStager(self.h)
@@ -201,8 +213,7 @@ class HotPathEngine:
         self._batches: Dict[tuple, _native.FrameBatch] = {}
         self._persistent = set()  # ids of the engine's own persistent device tensors (downsample outputs)
         self._small: Dict[tuple, object] = {}
-        self._net = None
-        self._net_shapes = []
+        self._nets: Dict[tuple, tuple] = {}  # network-input (h, w) -> (persistent buffer, source (h, w) of each position)
         # the network-input buffer is persistent: pad rows are written once per geometry (B200VA_OUT_FLAG_PADS_VALID).
         # Needs an `infer` that does not write into its input; pass static_pads=False otherwise.
         self.static_pads = bool(static_pads)
@@ -254,13 +265,16 @@ class HotPathEngine:
             b = e
         return out, metas
 
-    def _net_in(self, n: int):
+    def _net_in(self, n: int, hw=None):
+        """The persistent network-input buffer of one input shape (default: the detector's input size)."""
         t = self.h.torch
+        hw = tuple(hw or self.detector.input_hw)
         dtype = t.float16 if self.detector._fmt == _native.OUT_F16_RGB_NCHW else t.float32
-        if self._net is None or self._net.shape[0] < n or self._net.dtype != dtype:
-            self._net = t.empty((max(n, len(self.streams)), 3, *self.detector.input_hw), dtype=dtype, device=self.h.device)
-            self._net_shapes = [None] * self._net.shape[0]  # source (h, w) whose pad rows each position holds
-        return self._net[:n]
+        net, _ = self._nets.get(hw, (None, None))
+        if net is None or net.shape[0] < n or net.dtype != dtype:
+            net = t.empty((max(n, len(self.streams)), 3, *hw), dtype=dtype, device=self.h.device)
+            self._nets[hw] = (net, [None] * net.shape[0])  # source (h, w) whose pad rows each position holds
+        return net[:n]
 
     def _bgr_buffer(self, pos: int, hw, full: bool = False):
         """One persistent BGR buffer per (stream position, size, purpose): stable addresses, no per-tick allocation."""
@@ -271,14 +285,65 @@ class HotPathEngine:
             self._persistent.add(id(buf))
         return buf
 
-    def _pads_flag(self, frames) -> int:
-        """B200VA_OUT_FLAG_PADS_VALID when every batch position was last written from a frame of the same size
-        (same letterbox geometry, same format): its pad rows are already in the persistent buffer."""
+    def _pads_flag(self, frames, hw=None) -> int:
+        """B200VA_OUT_FLAG_PADS_VALID when every batch position of the ``hw`` buffer was last written from a frame of
+        the same size (same letterbox geometry, same format): its pad rows are already in the persistent buffer."""
+        held = self._nets[tuple(hw or self.detector.input_hw)][1]
         shapes = [_native.frame_hw(f) for f in frames]
-        valid = all(self._net_shapes[k] == sh for k, sh in enumerate(shapes))
+        valid = all(held[k] == sh for k, sh in enumerate(shapes))
         for k, sh in enumerate(shapes):
-            self._net_shapes[k] = sh
+            held[k] = sh
         return _native.OUT_FLAG_PADS_VALID if (valid and self.static_pads) else 0
+
+    def _ultra_geom(self, hw):
+        """(Letterbox, network-input (h, w)) the Ultralytics detector's batch-1 ``predict`` gives a frame of size ``hw``."""
+        g = self._ultra_geoms.get(hw)
+        if g is None:
+            g = self._ultra_geoms[hw] = self.detector.frame_geometry(*hw)
+        return g
+
+    def _predict_ultralytics(self, frames, masks, streams, dets, infer_ctx, skip=None):
+        """Letterbox -> forward -> ``postprocess_ultralytics`` of ``frames`` (stream indices ``streams``) into the rows
+        of ``dets`` at their positions.  Frames are grouped by network-input shape (padding them to a common canvas
+        would change the model's output); each group runs its own letterbox, forward and post-process, and when the
+        groups interleave, its detection rows are copied to their positions on the device.  ``skip`` (device gates):
+        one flag per position, gathered per group for the group's kernels."""
+        det, h, t = self.detector, self.h, self.h.torch
+        geoms, groups = [], {}
+        for j, f in enumerate(frames):
+            g, in_hw = self._ultra_geom(_native.frame_hw(f))
+            geoms.append(g)
+            groups.setdefault(in_hw, []).append(j)
+        whole = len(groups) == 1  # one group holds every position in order: no gather, no copy
+        for in_hw, idx in groups.items():
+            n = len(idx)
+            pos = None if whole else t.tensor(idx, dtype=t.int64, device=h.device)
+            g_frames = [frames[j] for j in idx]
+            g_skip = None if skip is None else (skip if whole else skip.index_select(0, pos))
+            net = self._net_in(n, in_hw)
+            pads = self._pads_flag(g_frames, in_hw)
+            if skip is not None:
+                # a batch position whose pad rows were never written must be letterboxed whatever its gate says
+                h.set_skip_mask(g_skip if pads else None)
+            tensor = det.letterbox(g_frames, [geoms[j] for j in idx], in_hw, [masks[j] for j in idx], det._fmt | pads, net,
+                                   on_run=(lambda b, e: h.set_skip_mask(g_skip[b:e])) if skip is not None and pads else None)
+            if skip is not None:
+                h.set_skip_mask(g_skip)
+            self.active_streams = [streams[j] for j in idx]
+            head = det._infer(tensor) if infer_ctx is None else det._infer_fn(tensor, infer_ctx)
+            head = det._as_head(head)
+            if head.dim() != 3 or head.shape[0] != n:
+                raise ValueError(f"infer returned {tuple(head.shape)} for a batch of {n}")
+            if whole:
+                out = dets
+            else:
+                if self._scratch is None:
+                    self._scratch = h.alloc_dets(max(len(self.streams), 1))
+                out = {k: v[:n] for k, v in self._scratch.items() if not k.startswith("_")}
+            det._run_post_ultra(head, [_native.frame_hw(f) for f in g_frames], in_hw, out, fold_filter=True)
+            if not whole:
+                for k in ("bbox_xyxy", "conf", "cls", "count"):
+                    dets[k].index_copy_(0, pos, out[k])
 
     # --------------------------------------------------------------------------------------
     def tick(self, frames: Sequence, frame_ids: Optional[Sequence[int]] = None, infer_ctx=None) -> List[FrameResult]:
@@ -306,7 +371,11 @@ class HotPathEngine:
         for i, st in zip(live, states):
             sparse_ok[i] = (not getattr(st.cfg, "motion_filter", False)
                             and float(getattr(st.cfg, "downsample_ratio", 1.0)) >= 0.999)
-        staged = self.stager.upload(list(frames), sparse_for=self.detector.input_hw, sparse_ok=sparse_ok)
+        if self.ultralytics:  # each frame's own LetterBox geometry decides which rows it reads
+            geoms = [self._ultra_geom(_native.frame_hw(f))[0] if f is not None else None for f in frames]
+            staged = self.stager.upload(list(frames), sparse_ok=sparse_ok, geoms=geoms)
+        else:
+            staged = self.stager.upload(list(frames), sparse_for=self.detector.input_hw, sparse_ok=sparse_ok)
         ctx.keep = self.stager.take_sources()
         ctx.gen += 1
         dev_frames = [staged[i] for i in live]
@@ -379,7 +448,10 @@ class HotPathEngine:
         n_act = len(active)
         nb = len(order)
         dets = {k_: v[:nb] for k_, v in ctx.dets.items() if not k_.startswith("_")}
-        if n_act:
+        if n_act and self.ultralytics:
+            self._predict_ultralytics([work[k] for k in active], [work_masks[k] for k in active], [live[k] for k in active],
+                                      {k_: v[:n_act] for k_, v in dets.items()}, infer_ctx)
+        elif n_act:
             net = self._net_in(n_act)
             act_frames = [work[k] for k in active]
             tensor, metas = self._letterbox(act_frames, [work_masks[k] for k in active],
@@ -391,7 +463,7 @@ class HotPathEngine:
             head = self.detector._as_head(head)
             if head.dim() != 3 or head.shape[0] != n_act:
                 raise ValueError(f"infer returned {tuple(head.shape)} for a batch of {n_act}")
-            self.detector._run_post(head, metas, {k_: v[:n_act] for k_, v in dets.items()})
+            self.detector._run_post(head, metas, {k_: v[:n_act] for k_, v in dets.items()}, fold_filter=True)
         scale = [1.0 / max(ratios[k], 1e-6) if ratios[k] < 0.999 else 1.0 for k in order]
         out = {k_: v[:nb] for k_, v in ctx.tracks.items() if not k_.startswith("_")}
         self.tracker.update_batch([names[k] for k in order], dets,
@@ -444,18 +516,22 @@ class HotPathEngine:
         dets = {k_: v[:nb] for k_, v in ctx.dets.items() if not k_.startswith("_")}
         out = {k_: v[:nb] for k_, v in ctx.tracks.items() if not k_.startswith("_")}
         try:
-            net = self._net_in(nb)
-            pads = self._pads_flag(work)
-            # a batch position whose pad rows were never written must be letterboxed whatever its gate says
-            h.set_skip_mask(skip if pads else None)
-            tensor, metas = self._letterbox(work, work_masks, self.detector._fmt | pads, net, skip if pads else None)
-            h.set_skip_mask(skip)
-            self.active_streams = list(live)
-            head = self.detector._infer(tensor) if infer_ctx is None else self.detector._infer_fn(tensor, infer_ctx)
-            head = self.detector._as_head(head)
-            if head.dim() != 3 or head.shape[0] != nb:
-                raise ValueError(f"infer returned {tuple(head.shape)} for a batch of {nb}")
-            self.detector._run_post(head, metas, dets)
+            if self.ultralytics:
+                self._predict_ultralytics(work, work_masks, list(live), dets, infer_ctx, skip)
+                h.set_skip_mask(skip)
+            else:
+                net = self._net_in(nb)
+                pads = self._pads_flag(work)
+                # a batch position whose pad rows were never written must be letterboxed whatever its gate says
+                h.set_skip_mask(skip if pads else None)
+                tensor, metas = self._letterbox(work, work_masks, self.detector._fmt | pads, net, skip if pads else None)
+                h.set_skip_mask(skip)
+                self.active_streams = list(live)
+                head = self.detector._infer(tensor) if infer_ctx is None else self.detector._infer_fn(tensor, infer_ctx)
+                head = self.detector._as_head(head)
+                if head.dim() != 3 or head.shape[0] != nb:
+                    raise ValueError(f"infer returned {tuple(head.shape)} for a batch of {nb}")
+                self.detector._run_post(head, metas, dets, fold_filter=True)
             scale = [1.0 / max(r, 1e-6) if r < 0.999 else 1.0 for r in ratios]
             self.tracker.update_batch(names, dets, det_scale=scale if any(s != 1.0 for s in scale) else None, out=out)
             h.gates_commit(gates, dets["count"], out["count"], skip, ctx.gate_state[:nb])

@@ -107,14 +107,17 @@ class FrameStager:
             self._ids.add(id(buf))
         return buf
 
-    def upload(self, frames: Sequence, sparse_for=None, sparse_ok: Optional[Sequence[bool]] = None) -> List:
+    def upload(self, frames: Sequence, sparse_for=None, sparse_ok: Optional[Sequence[bool]] = None,
+               geoms: Optional[Sequence] = None) -> List:
         """Return CUDA uint8 [H,W,3] tensors for ``frames``; CUDA tensors pass through untouched.  Host NV12 frames
         (uint8 ``[3H/2, W]`` NumPy arrays or CPU tensors, OpenCV's layout) land in CUDA ``[3H/2, W]`` tensors, half the
-        bytes of BGR, sparsely under the same ``sparse_ok`` rule; ``(y, uv)`` pairs of CUDA planes pass through."""
+        bytes of BGR, sparsely under the same ``sparse_ok`` rule; ``(y, uv)`` pairs of CUDA planes pass through.
+        ``geoms`` is the per-frame form of ``sparse_for``: ``geoms[k]`` (a ``Letterbox``, or None for every row) is the
+        geometry ``preprocess_geom`` will letterbox frame k with, and only the rows it reads are uploaded."""
         t = self.h.torch
         out: List = [None] * len(frames)
-        groups = {False: ([], []), True: ([], [])}
-        nv12 = {False: ([], []), True: ([], [])}
+        groups = {False: ([], [], []), True: ([], [], [])}
+        nv12 = {False: ([], [], []), True: ([], [], [])}
         keep = []
         for k, f in enumerate(frames):
             if f is None:
@@ -122,7 +125,8 @@ class FrameStager:
             if (t.is_tensor(f) and f.is_cuda) or isinstance(f, (tuple, list)):
                 out[k] = f
                 continue
-            sparse = bool(sparse_for) and (sparse_ok is None or bool(sparse_ok[k]))
+            geom = geoms[k] if geoms is not None else None
+            sparse = (geom is not None if geoms is not None else bool(sparse_for)) and (sparse_ok is None or bool(sparse_ok[k]))
             if _native.is_nv12(f):
                 a = f if t.is_tensor(f) else np.asarray(f)
                 if t.is_tensor(a):
@@ -144,6 +148,7 @@ class FrameStager:
                 out[k] = dev
                 nv12[sparse][0].append(_native.Nv12Frame(ptr, ptr + h * pitch, pitch, pitch))
                 nv12[sparse][1].append(dev)
+                nv12[sparse][2].append(geom)
                 continue
             if t.is_tensor(f):
                 if f.dtype != t.uint8 or f.dim() != 3 or f.shape[2] != 3 or f.stride(2) != 1 or f.stride(1) != 3:
@@ -162,11 +167,15 @@ class FrameStager:
             out[k] = dev
             groups[sparse][0].append((ptr, pitch))
             groups[sparse][1].append(dev)
-        for sparse, (ptrs, devs) in groups.items():
+            groups[sparse][2].append(geom)
+        by_geom = geoms is not None
+        for sparse, (ptrs, devs, gs) in groups.items():
             if devs:
-                self.bytes_moved += self.h.upload_frames(ptrs, devs, sparse_for if sparse else None)
-        for sparse, (hosts, devs) in nv12.items():
+                self.bytes_moved += self.h.upload_frames(ptrs, devs, sparse_for if sparse and not by_geom else None,
+                                                         geoms=gs if sparse and by_geom else None)
+        for sparse, (hosts, devs, gs) in nv12.items():
             if devs:
-                self.bytes_moved += self.h.upload_frames_nv12(hosts, devs, sparse_for if sparse else None)
+                self.bytes_moved += self.h.upload_frames_nv12(hosts, devs, sparse_for if sparse and not by_geom else None,
+                                                              geoms=gs if sparse and by_geom else None)
         self._keep = keep  # sources stay alive until the caller synchronises (end of the tick)
         return out
