@@ -363,6 +363,8 @@ B200VA_API int b200va_dfl_decode(b200va_handle h, const float* raw, int batch, i
  * (:111-126), _iou (:129-147) for a batch of streams; state lives in the handle per slot.
  * stream_slots HOST [batch] slot ids in [0, max_streams), distinct within a call
  * dets         detections per frame ([batch, max_dets] SoA as produced by b200va_postprocess);
+ *              max_dets in [1, 32768] (a track row remembers its detection in 16 bits), else
+ *              B200VA_ERR_INVALID;
  *              det_scale HOST double [batch] or NULL: pipeline.py:224-240 rescale (1/ratio), applied
  *              in float64 to the boxes before matching
  * skip         HOST uint8 [batch] or NULL: 1 = tracker.update(stream, []) (pipeline.py:214-215)
@@ -371,7 +373,10 @@ B200VA_API int b200va_dfl_decode(b200va_handle h, const float* raw, int batch, i
  *              which reproduces one shared itertools.count(1) updated stream by stream
  *              (tracker.py:47, pipeline.py:452)
  * out          all surviving tracks per stream in insertion order (tracker.py:95), may be NULL
- * new_counts   DEVICE int32 [batch] number of tracks created by this call, may be NULL */
+ * new_counts   DEVICE int32 [batch] number of tracks created by this call, may be NULL
+ * The IoU is tracker.py's float64 arithmetic with Python's builtin min / max, track first: a NaN
+ * coordinate of a detection is replaced by the track's in the intersection (so such a detection can
+ * match, with an IoU above 1 even), a NaN coordinate of a track makes its IoU 0. */
 B200VA_API int b200va_tracker_update(b200va_handle h, const int* stream_slots, int batch, const b200va_dets* dets,
                           int max_dets, const double* det_scale, const uint8_t* skip,
                           const b200va_tracker_cfg* cfg, const int64_t* id_base, const b200va_tracks* out,

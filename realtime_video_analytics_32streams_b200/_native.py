@@ -16,6 +16,7 @@ PKG_DIR = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("B200VA_LIB") or os.path.join(PKG_DIR, "lib", "libb200va.so")
 
 OK, ERR_INVALID, ERR_CUDA, ERR_CAPACITY, ERR_STATE = 0, -1, -2, -3, -4
+TRACKER_MAX_DETS = 32768  # most detection rows per stream b200va_tracker_update[_f64] take (max_dets)
 OUT_F32_RGB_NCHW, OUT_F16_RGB_NCHW, OUT_U8_BGR_NCHW, OUT_U8_BGR_NHWC = 0, 1, 2, 3
 OUT_FLAG_PADS_VALID = 0x100  # OR into the format: the pad rows of `out` are still valid from an earlier call
 HEAD_CHANNEL_MAJOR, HEAD_ANCHOR_MAJOR = 0, 1

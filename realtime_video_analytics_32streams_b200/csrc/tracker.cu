@@ -197,7 +197,7 @@ extern "C" int b200va_tracker_update(b200va_handle h, const int* stream_slots, i
   std::lock_guard<std::recursive_mutex> lock(h->mu);
   DeviceGuard guard(h->cfg.device);
   REQUIRE(h, dets && dets->bbox_xyxy && dets->conf && dets->cls && dets->count, "NULL detections");
-  REQUIRE(h, max_dets > 0, "max_dets must be positive");
+  REQUIRE(h, max_dets > 0 && max_dets <= kTrkMaxDets, "max_dets %d outside [1, %d]", max_dets, kTrkMaxDets);
   TrkParams p;
   memset(&p, 0, sizeof(p));
   p.f_box = dets->bbox_xyxy;
@@ -216,7 +216,7 @@ extern "C" int b200va_tracker_update_f64(b200va_handle h, const int* stream_slot
   std::lock_guard<std::recursive_mutex> lock(h->mu);
   DeviceGuard guard(h->cfg.device);
   REQUIRE(h, dets && dets->bbox_xyxy && dets->conf && dets->cls && dets->count, "NULL detections");
-  REQUIRE(h, max_dets > 0, "max_dets must be positive");
+  REQUIRE(h, max_dets > 0 && max_dets <= kTrkMaxDets, "max_dets %d outside [1, %d]", max_dets, kTrkMaxDets);
   TrkParams p;
   memset(&p, 0, sizeof(p));
   p.d_box = dets->bbox_xyxy;

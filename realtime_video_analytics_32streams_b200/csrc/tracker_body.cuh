@@ -67,14 +67,22 @@ struct TrkParams {
 namespace {
 
 
-// tracker.py:129-147, IEEE double, no contraction.
+// Python's builtin min / max on two floats: the first argument unless the second compares strictly below / above it.
+// So a NaN second argument gives the first, a NaN first argument gives NaN (fmin / fmax return the non-NaN operand
+// either way).  The tracker calls them with the track's coordinate first (tracker.py:129-147): a NaN coordinate of the
+// detection is replaced by the track's in the intersection, a NaN coordinate of the track makes the intersection 0.
+__device__ __forceinline__ double py_min(double a, double b) { return b < a ? b : a; }
+__device__ __forceinline__ double py_max(double a, double b) { return b > a ? b : a; }
+__device__ __forceinline__ double py_relu(double x) { return x > 0.0 ? x : 0.0; }  // max(0.0, x)
+
+// tracker.py:129-147, IEEE double, no contraction; a = the track, b = the detection.
 __device__ __forceinline__ double iou64(double ax1, double ay1, double ax2, double ay2, double bx1, double by1,
                                         double bx2, double by2) {
-  const double iw = fmax(0.0, __dsub_rn(fmin(ax2, bx2), fmax(ax1, bx1)));
-  const double ih = fmax(0.0, __dsub_rn(fmin(ay2, by2), fmax(ay1, by1)));
+  const double iw = py_relu(__dsub_rn(py_min(ax2, bx2), py_max(ax1, bx1)));
+  const double ih = py_relu(__dsub_rn(py_min(ay2, by2), py_max(ay1, by1)));
   const double inter = __dmul_rn(iw, ih);
-  const double area_a = __dmul_rn(fmax(0.0, __dsub_rn(ax2, ax1)), fmax(0.0, __dsub_rn(ay2, ay1)));
-  const double area_b = __dmul_rn(fmax(0.0, __dsub_rn(bx2, bx1)), fmax(0.0, __dsub_rn(by2, by1)));
+  const double area_a = __dmul_rn(py_relu(__dsub_rn(ax2, ax1)), py_relu(__dsub_rn(ay2, ay1)));
+  const double area_b = __dmul_rn(py_relu(__dsub_rn(bx2, bx1)), py_relu(__dsub_rn(by2, by1)));
   const double uni = __dsub_rn(__dadd_rn(area_a, area_b), inter);
   if (uni <= 0.0) return 0.0;
   return __ddiv_rn(inter, uni);
@@ -119,32 +127,53 @@ __device__ __forceinline__ void stage_detection(DetStage& sd, int i, float4 f4, 
 // Boxes whose intersection is empty have IoU 0, which can never beat best_iou = 0.0 (tracker.py:100-106).
 // A cheap superset of overlaps(): the same eight comparisons on order-preserving integer keys of the doubles' HIGH
 // words (x > y implies key(x) >= key(y), whatever the signs), as `>=`.  It may pass pairs that do not overlap (their
-// IoU then comes out as 0 and is discarded like before) but never rejects one that does; NaN coordinates pass or fail
-// arbitrarily, which is harmless for the same reason.  Integer compares instead of a chain of eight dependent float64
-// compares: the pre-filter runs once per (detection, track) pair on the latency-bound path.
+// IoU then comes out as 0 and is discarded like before) but never rejects one that does.  Non-finite coordinates:
+// a NaN of the DETECTION does not empty the intersection (iou64 puts the track's coordinate in its place), so the
+// detection's keys (det_keys) give a NaN or infinite lower coordinate (x1, y1) key 0 and an upper one (x2, y2) key
+// 0xFFFFFFFF, which pass every comparison.  A NaN of the TRACK makes the IoU 0 whatever the detection is, so the
+// track's keys (box_keys) are the plain hi_key and may reject such a pair arbitrarily.  Integer compares instead of a
+// chain of eight dependent float64 compares: the pre-filter runs once per (detection, track) pair on the
+// latency-bound path.
 __device__ __forceinline__ uint32_t hi_key(double v) {
   const int hi = __double2hiint(v);
   return (uint32_t)hi ^ ((uint32_t)(hi >> 31) | 0x80000000u);
 }
+__device__ __forceinline__ uint32_t nonfinite_mask(double v) {
+  return ((uint32_t)__double2hiint(v) & 0x7ff00000u) == 0x7ff00000u ? 0xffffffffu : 0u;
+}
+__device__ __forceinline__ uint32_t lower_key(double v) { return hi_key(v) & ~nonfinite_mask(v); }
+__device__ __forceinline__ uint32_t upper_key(double v) { return hi_key(v) | nonfinite_mask(v); }
 __device__ __forceinline__ bool may_overlap(const double4 a, const double4 b) {
   const uint32_t ax = hi_key(a.x), ay = hi_key(a.y), az = hi_key(a.z), aw = hi_key(a.w);
-  const uint32_t bx = hi_key(b.x), by = hi_key(b.y), bz = hi_key(b.z), bw = hi_key(b.w);
+  const uint32_t bx = lower_key(b.x), by = lower_key(b.y), bz = upper_key(b.z), bw = upper_key(b.w);
   return (az >= bx) & (bz >= ax) & (az >= ax) & (bz >= bx) & (aw >= by) & (bw >= ay) & (aw >= ay) & (bw >= by);
 }
 
 // Row bytes of a stream's working table: box 32, class 4, hits 4, claims 4, last detection 2, overlap keys 16.
 constexpr int kTrkRowBytes = 62;
-// The overlap keys of a row: hi_key of (x1, y1, x2, y2), 16 bytes.  Phase A of a dense stream tests every (detection,
-// track) pair; reading the track's four doubles for that costs 8 shared-memory wavefronts per warp step (32-byte lane
-// stride) and eight float64 compares, the keys cost 4 wavefronts and four integer compares -- and only a pair that
-// passes them (a superset of the overlapping ones, see may_overlap) looks at the doubles.
-__device__ __forceinline__ uint4 box_keys(const double4 b) { return make_uint4(hi_key(b.x), hi_key(b.y), hi_key(b.z), hi_key(b.w)); }
+// The last detection of a row is an int16_t index into the frame's detections, so a call takes at most this many
+// detection rows per stream (b200va_tracker_update[_f64] refuse more; the tick's rows are max_dets <= 8192).
+constexpr int kTrkMaxDets = 32768;
+// The overlap keys of a row: hi_key of (x1, y1, x2, y2), 16 bytes (det_keys for the chunk's detections).  Phase A of
+// a dense stream tests every (detection, track) pair; reading the track's four doubles for that costs 8 shared-memory
+// wavefronts per warp step (32-byte lane stride) and eight float64 compares, the keys cost 4 wavefronts and four
+// integer compares -- and only a pair that passes them (a superset of the overlapping ones, see may_overlap) looks at
+// the doubles.
+__device__ __forceinline__ uint4 box_keys(const double4 b) {
+  return make_uint4(hi_key(b.x), hi_key(b.y), hi_key(b.z), hi_key(b.w));
+}
+__device__ __forceinline__ uint4 det_keys(const double4 b) {
+  return make_uint4(lower_key(b.x), lower_key(b.y), upper_key(b.z), upper_key(b.w));
+}
 __device__ __forceinline__ uint4* trk_key_table(uint8_t* tab, int cap) {
   return reinterpret_cast<uint4*>(tab + (((size_t)cap * 46 + kDetChunk * 4 + 15) & ~(size_t)15));
 }
 
+// The intersection of track (or earlier detection) `a` and detection `b` is not empty.  The terms with a coordinate of
+// `b` are negated comparisons, so a NaN there passes them (see iou64); a NaN of `a` fails `a.z > a.x` or `a.w > a.y`.
 __device__ __forceinline__ bool overlaps(const double4 a, const double4 b) {
-  return (a.z > b.x) & (b.z > a.x) & (a.z > a.x) & (b.z > b.x) & (a.w > b.y) & (b.w > a.y) & (a.w > a.y) & (b.w > b.y);
+  return !(b.x >= a.z) & !(a.x >= b.z) & (a.z > a.x) & !(b.x >= b.z) & !(b.y >= a.w) & !(a.y >= b.w) & (a.w > a.y) &
+         !(b.y >= b.w);
 }
 
 // Best track for one detection among tracks t = first, first + stride, ... (tracker.py:97-109).
@@ -204,7 +233,7 @@ struct TrkShared {
   int s_T, s_new, s_is_last, s_fallback, s_nconf;
   int n_plist;      // phase A, few pairs: number of listed (overlapping, same class) pairs
   uint32_t plist[kTrkPairs];  // idx | detection << 16 | (vs track) << 31
-  uint4 dkey[kDetChunk];      // phase A, many pairs: overlap keys of the chunk's detections (box_keys)
+  uint4 dkey[kDetChunk];      // phase A, many pairs: overlap keys of the chunk's detections (det_keys)
   int s_prestaged;  // fused kernel: detections of this frame (count) whose first chunk the NMS half left in `sd`; -1 = none
   int wsum[kTrkThreadsMax / 32];
   int warp_cnt[kTrkThreadsMax / 32];
@@ -399,7 +428,7 @@ __device__ __forceinline__ void tracker_stream_impl(const TrkParams& p, const in
     // ---- phase A: every IoU the chunk can need.  Warp w takes detections w, w+8, ..; lanes take tracks ----
     const int Tc = s_T;
     for (int t = tid; t < Tc + kDetChunk; t += kTrkThreads) aux[t] = 0;  // claims per track
-    if (!SMALL && tid < nd) sh.dkey[tid] = box_keys(sd.box[tid]);
+    if (!SMALL && tid < nd) sh.dkey[tid] = det_keys(sd.box[tid]);
     __syncthreads();
     const int pairs_t = nd * Tc, pairs = pairs_t + nd * nd;
     static_assert(kTrkPairs >= 8 * kTrkThreadsMin, "the pair list must hold every pair of the small path");
@@ -520,7 +549,8 @@ __device__ __forceinline__ void tracker_stream_impl(const TrkParams& p, const in
         const bool vs_track = blk < nblk_t;
         const int r0 = (vs_track ? blk * 64 : 0) + lane, r1 = r0 + 32;
         const int rows = vs_track ? Tc : nd;
-        // (a row past the end gets keys no box can meet)
+        // (a row past the end gets keys that no finite box meets; a detection with non-finite coordinates can meet
+        // them, since det_keys widens those, so the `r0 >= rows` masks below are what drops such rows)
         uint4 k0 = make_uint4(0xffffffffu, 0xffffffffu, 0u, 0u), k1 = k0;
         int c0 = 0, c1 = 0;
         if (r0 < rows) {

@@ -121,10 +121,15 @@ class B200IouTracker:
     # ---- reference API ---------------------------------------------------------------------
     def update(self, stream_name: str, detections: Iterable) -> List[Track]:
         """tracker.py:50-95.  One pinned flat upload (boxes, confidences, classes, count), one launch, one flat
-        read-back (track table + capacity flags)."""
+        read-back (track table + capacity flags).  Takes at most ``TRACKER_MAX_DETS`` (32768) detections per call and
+        raises ``B200VAError`` with ``ERR_INVALID`` for more, leaving the tracker as it was (the reference takes any
+        number)."""
         h, t = self.h, self.h.torch
         dets = detections if isinstance(detections, (list, tuple)) else list(detections)
         n = len(dets)
+        if n > _native.TRACKER_MAX_DETS:  # checked before the staging grows: its row count is the call's max_dets
+            raise _native.B200VAError(_native.ERR_INVALID, f"{n} detections in one update (at most "
+                                                           f"{_native.TRACKER_MAX_DETS})")
         if self._in is None or self._in.cap < n:
             self._in = _HostDets(h, max(64, 1 << max(n - 1, 0).bit_length()))
         if self._out is None:
